@@ -13,7 +13,7 @@ ARCH      := -gencode arch=compute_100a,code=sm_100a
 NVFLAGS   := $(ARCH) -O3 -std=c++17 -lineinfo -fmad=false -prec-div=true -prec-sqrt=true \
              -Xcompiler -fPIC,-ffp-contract=off,-fno-fast-math,-Wall -Xptxas -v
 LIBSRC    := $(CSRC)/rt_kernels.cu $(CSRC)/rt_tile.cu $(CSRC)/rt_phased.cu $(CSRC)/rt_api.cpp $(CSRC)/rt_scene.cpp
-LIBHDR    := $(CSRC)/rt_device.cuh $(CSRC)/rt_cull.cuh $(CSRC)/rt_kernels.h $(CSRC)/rt_scene.h include/rtrace.h
+LIBHDR    := $(CSRC)/rt_device.cuh $(CSRC)/rt_cull.cuh $(CSRC)/rt_pack.cuh $(CSRC)/rt_kernels.h $(CSRC)/rt_scene.h include/rtrace.h
 
 all: rtrace
 

@@ -19,6 +19,11 @@ Frame 0 is BASELINE configs[2] ("c3").  The same invocation also measures, as su
             NVLink, end to end every rank copies its blocks into one shared pinned host frame over its own
             PCIe link; a cross-rank barrier closes every frame (frame latency, not throughput)
 `--workload X` measures one workload alone (c1/c2/c3/c3l10/c4/c5), `--mode bands` its row-band split.
+`--steps K` is the number of timed steps of every measurement (kernel-only and end to end, sub-records included).
+`--dump-outputs DIR` writes, after the timed steps, the frame the kernel-only path computed in its last step as
+DIR/<workload>.npy (float32 RGBA values; rank 0's frame; a fixed seeded sample of a frame too large for the run's
+DUMP_BYTES), so that two builds can be compared output for output: the scenes and cameras of a run depend on its
+arguments only.
 
 metric  = Mrays/s (primary + shadow rays, counted as the reference's work is counted)
 value   = whole-job rays / device time of the K steps (CUDA events on the launch stream, max over ranks),
@@ -58,6 +63,8 @@ ORBIT_FRAMES = 120               # c5: eye and camera basis rotated about the fl
 # from the oracle's counters (tests/golden/oracle_derived.json); used when the fixture lacks the config.
 FLOP_PER_RAY_FALLBACK = 645.0
 METRIC = "Mrays/s (primary+shadow)"
+DUMP_BYTES = 64 * 10 ** 6        # --dump-outputs: all files of one run together, .npy headers included
+DUMP_SEED = 20261020
 KERNEL_SOURCES = ("rt_phased.cu", "rt_cull.cuh", "rt_pack.cuh", "rt_device.cuh", "rt_kernels.cu", "rt_tile.cu")
 
 
@@ -91,6 +98,45 @@ def workload_name(name, level, width, height, spp):
 
 def log(*a):
     print(*a, file=sys.stderr, flush=True)
+
+
+def dump_names(args, world):
+    """The files a run with these arguments writes under --dump-outputs, one per measurement; rank 0 writes them all."""
+    workload = args.workload or DEFAULT_WORKLOAD
+    if args.impl == "reference":
+        return [workload]
+    names = [workload + "_bands" if args.mode == "bands" and world > 1 else workload]
+    if args.workload is None and not args.no_also:
+        names += ["c2", "c4"] + (["c4_bands"] if world > 1 else [])
+    return names
+
+
+def dump_pixels(n_files):
+    """Pixels kept per frame when a run writes n_files frames: DUMP_BYTES split evenly, 16 bytes a pixel (float32
+    RGBA), 4 KiB per file left for the .npy header."""
+    return (DUMP_BYTES // n_files - 4096) // 16
+
+
+def sample_pixels(frame, pixels):
+    """An (h, w, 4) RGBA8 frame as float32 (n, 4), pixels in row-major order: the whole frame if it has at most
+    `pixels` pixels, else the same seeded sample of `pixels` of them in every run."""
+    import numpy as np
+    px = np.asarray(frame).reshape(-1, 4)
+    if len(px) > pixels:
+        px = px[np.sort(np.random.default_rng(DUMP_SEED).choice(len(px), pixels, replace=False))]
+    return px.astype(np.float32)
+
+
+def dump_frame(args, world, name, frame):
+    """--dump-outputs: the frame as <DIR>/<name>.npy, sampled so that the run's files stay within DUMP_BYTES."""
+    import numpy as np
+    names = dump_names(args, world)
+    if name not in names:
+        raise RuntimeError("bench.py: %s is not among the files this run writes (%s)" % (name, names))
+    os.makedirs(args.dump_outputs, exist_ok=True)
+    path = os.path.join(args.dump_outputs, name + ".npy")
+    np.save(path, sample_pixels(frame, dump_pixels(len(names))))
+    log("bench.py: wrote", path)
 
 
 def oracle_case(width, height, spp, level):
@@ -220,19 +266,19 @@ def pin_to_gpu_cpus(local_rank):
 # CPU legs (the oracle: test infrastructure, allowed here as the reported baseline only)
 # ---------------------------------------------------------------------------------------------------
 def cpu_frames(workload, width, height, spp, level, frames, threads):
-    """Whole frames of the workload on `threads` host threads -> (rays, seconds, flop/ray of the last frame)."""
+    """Whole frames of the workload on `threads` host threads -> (rays, seconds, flop/ray of the last frame, last frame)."""
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     import _oracle as o   # bench.py's cpu_baseline / reference legs are allowed to run the oracle
     s = o.Scene(level=level)
     rays = secs = 0.0
-    ctr = None
+    ctr = img = None
     for f in frames:
         cam = o.make_camera(*orbit_basis(f % ORBIT_FRAMES)) if workload == "c5" else None   # f: an orbit frame index
         t0 = time.perf_counter()
-        _, ctr = s.render_rows(width, height, spp, 0, 1, height, threads=threads, camera=cam)
+        img, ctr = s.render_rows(width, height, spp, 0, 1, height, threads=threads, camera=cam)
         secs += time.perf_counter() - t0
         rays += ctr.primary_rays + ctr.shadow_rays
-    return rays, secs, (ctr.flop_per_ray() if ctr else None)
+    return rays, secs, (ctr.flop_per_ray() if ctr else None), img
 
 
 def cpu_leg(workload, width, height, spp, level, budget_s=12.0):
@@ -242,7 +288,7 @@ def cpu_leg(workload, width, height, spp, level, budget_s=12.0):
     rays = secs = 0.0
     n, fpr = 0, None
     while n == 0 or (secs < budget_s and secs / n * (n + 1) < 2.5 * budget_s):
-        r, s, fpr = cpu_frames(workload, width, height, spp, level, [(n * 47) % ORBIT_FRAMES], cores)   # 0, 47, 94, 21, ..: spread
+        r, s, fpr, _ = cpu_frames(workload, width, height, spp, level, [(n * 47) % ORBIT_FRAMES], cores)   # 0, 47, 94, 21, ..: spread
         rays, secs, n = rays + r, secs + s, n + 1
     what = "orbit frame(s) %s" % [(k * 47) % ORBIT_FRAMES for k in range(n)] if workload == "c5" else "%d repeat(s) of the frame" % n
     return {"value": rays / secs / 1e6, "unit": "Mrays/s", "cores": cores, "kind": "port",
@@ -268,10 +314,16 @@ def run_reference(args, workload):
     rays = secs = 0.0
     done = 0
     for i in range(args.steps):
-        r, s, _ = cpu_frames(workload, width, height, spp, level, [orbit_frame(i, args.steps)], cores)   # the native arm's mix
+        r, s, _, img = cpu_frames(workload, width, height, spp, level, [orbit_frame(i, args.steps)], cores)   # the native arm's mix
         rays, secs, done = rays + r, secs + s, done + 1
         if time.perf_counter() - t_all > 200.0:   # keep the whole run within a few minutes on any host
             break
+    if args.dump_outputs:   # the last frame rendered; only c5's frame changes from step to step
+        if done < args.steps and workload == "c5":
+            log("bench.py: the reference arm stopped after %d of %d steps; %s.npy holds orbit frame %d, the native arm's "
+                "holds orbit frame %d" % (done, args.steps, workload, orbit_frame(done - 1, args.steps),
+                                          orbit_frame(args.steps - 1, args.steps)))
+        dump_frame(args, 1, workload, img)
     v = rays / secs / 1e6
     sample = "each step = one whole %dx%d spp %d level %d frame%s on %d host threads; %d of %d steps timed" % (
         width, height, spp, level, " (orbit frame i)" if workload == "c5" else "", cores, done, args.steps)
@@ -448,7 +500,7 @@ def measure_frames(job, workload, steps, warmup, cpu_baseline=False):
     fb = torch.zeros((height, width, 4), dtype=torch.uint8, device="cuda")
     _, st0 = rt.Renderer.render_rows(opts, scene, out_ptr=fb.data_ptr(), stream=job.stream.cuda_stream, want_stats=True)
     launches_per_step, variant_used = int(st0.kernel_launches), int(st0.variant_used)
-    e2e_steps = max(5, min(steps, 100))
+    e2e_steps = steps
     # rays of this rank's steps, counted on the device the way the reference's work is counted
     if sweep:
         table = {f: scene.count_rays(width, height, spp, camera=cams[f]) for f in sorted({frame_of(i) for i in range(steps)})}
@@ -465,6 +517,8 @@ def measure_frames(job, workload, steps, warmup, cpu_baseline=False):
         step(i)
     job.barrier()
     dev_ms, wall_ms = job.timed(steps, step)
+    if job.args.dump_outputs and rank == 0:   # fb holds the frame of the last timed step (job.timed synchronises)
+        dump_frame(job.args, world, workload, fb.cpu().numpy())
 
     # ---- e2e: the C-ABI call a user makes, every frame delivered to HOST memory ----
     # All ranks PULL frames from one queue (a counter in shared memory, rt_render_sweep_pull): the job is
@@ -679,7 +733,11 @@ def measure_bands(job, workload, steps, warmup, gather="peer"):
         got = rt.PinnedBuffer(height * row_bytes)
         rt.memcpy(got.ptr, frame_base, got.nbytes)
         verified = (hashlib.sha256(got.array.tobytes()).hexdigest() == case["rgba_sha256"]) if case else None
+        if job.args.dump_outputs:
+            dump_frame(job.args, world, workload + "_bands", got.array)
         got.close()
+    elif rank == 0 and job.args.dump_outputs:
+        dump_frame(job.args, world, workload + "_bands", partition.deinterleave(gathered, height).cpu().numpy())
     job.barrier()
 
     # ---- e2e: one shared pinned host frame (RGB8, the body of the P6 file), every rank copies its own blocks into it ----
@@ -723,7 +781,7 @@ def measure_bands(job, workload, steps, warmup, gather="peer"):
             dist.barrier()     # nobody overwrites the frame before the sink is done with it
     for i in range(3):
         e2e_step(i)
-    e2e_steps = max(5, min(steps, 50))
+    e2e_steps = steps
     job.barrier()
     t_begin = time.time()
     e0 = time.perf_counter()
@@ -778,7 +836,7 @@ def measure_bands(job, workload, steps, warmup, gather="peer"):
     }
 
 
-def main():
+def parse_args(argv=None):
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=50)
@@ -798,7 +856,16 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-l2-flush", action="store_true")
     ap.add_argument("--no-also", action="store_true", help="default run without the sub-records")
-    args = ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the frame of each measurement's last timed step to DIR/<workload>.npy (float32)")
+    args = ap.parse_args(argv)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+def main():
+    args = parse_args()
     workload = args.workload or DEFAULT_WORKLOAD
 
     if args.impl == "reference":
@@ -824,9 +891,9 @@ def main():
                 also[name] = rec
         sub("c2", measure_frames(job, "c2", args.steps, args.warmup))
         # 8K frames: whole frames per rank from one queue at every N ("8K multi-frame"), and at N > 1 ONE frame split
-        sub("c4", measure_frames(job, "c4", max(3, min(args.steps, 20)), args.warmup))
+        sub("c4", measure_frames(job, "c4", args.steps, args.warmup))
         if world > 1:
-            sub("c4_bands", measure_bands(job, "c4", max(3, min(args.steps, 20)), args.warmup))
+            sub("c4_bands", measure_bands(job, "c4", args.steps, args.warmup))
     clocks = job.sampler.stop(job.windows) if job.sampler else None
     if rank == 0:
         out["also"] = also or None

@@ -1,12 +1,13 @@
 """Regenerates the golden fixtures under tests/golden/.
 
-Run in the build container (needs /root/reference and PIL):
-    python tests/golden/make_golden.py
+Needs a checkout of the reference (Byron/rust-tracer) and PIL:
+    python tests/golden/make_golden.py <reference checkout>
 
 1. rtrace_output_1024x768.json -- derived from the REFERENCE's own artefact
    src/img/rtrace-output.png (the README hero image = exact output of `make image`,
    SURVEY F2): payload sha256, per-row CRC32s, spot pixels, background count.
-   This is what pins the oracle.
+   This is what pins the oracle.  rtrace_output_1024x768_rows.npz holds the same
+   image's pixels, every 4th row, so that a mismatch can be located without the reference.
 2. oracle_derived.json -- outputs of the (pinned) oracle for configurations the
    reference ships no image for: frame hashes and ray counts.  These pin the
    oracle against accidental edits; they are NOT independent evidence.
@@ -21,17 +22,17 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(HERE))
-REF_PNG = "/root/reference/src/img/rtrace-output.png"
+STORED_ROW_STEP = 4
 
 
-def from_reference_png():
+def from_reference_png(ref_png):
     from PIL import Image
-    rgb = np.array(Image.open(REF_PNG).convert("RGB"))
+    rgb = np.array(Image.open(ref_png).convert("RGB"))
     h, w, _ = rgb.shape
     spots = [(0, 0), (384, 512), (600, 400), (700, 512), (200, 300), (300, 512), (767, 1023), (100, 512), (500, 100)]
     out = {
         "source": "reference src/img/rtrace-output.png (make image: 1024x768, spp 4, level 8)",
-        "png_sha256": hashlib.sha256(open(REF_PNG, "rb").read()).hexdigest(),
+        "png_sha256": hashlib.sha256(open(ref_png, "rb").read()).hexdigest(),
         "width": w, "height": h, "spp": 4, "level": 8,
         "rgb_sha256": hashlib.sha256(rgb.tobytes()).hexdigest(),
         "ppm_sha256": hashlib.sha256(b"P6\n%d %d\n255\n" % (w, h) + rgb.tobytes()).hexdigest(),
@@ -42,6 +43,8 @@ def from_reference_png():
         "unique_colours": int(len(np.unique(rgb.reshape(-1, 3), axis=0))),
     }
     json.dump(out, open(os.path.join(HERE, "rtrace_output_1024x768.json"), "w"), indent=1)
+    rows = np.arange(0, h, STORED_ROW_STEP, dtype=np.uint16)
+    np.savez_compressed(os.path.join(HERE, "rtrace_output_1024x768_rows.npz"), rows=rows, rgb=rgb[rows])
     print("reference golden:", out["rgb_sha256"])
 
 
@@ -102,5 +105,7 @@ if __name__ == "__main__":
         d["c5_cases"] = c5_frames()
         json.dump(d, open(path, "w"), indent=1)
     else:
-        from_reference_png()
+        if len(sys.argv) < 2:
+            raise SystemExit("usage: make_golden.py <reference checkout> | --only-c5")
+        from_reference_png(os.path.join(sys.argv[1], "src", "img", "rtrace-output.png"))
         from_oracle()

@@ -31,6 +31,93 @@ def test_reference_arm_prints_one_json_line_with_the_contract_keys():
     assert "1024x768" in d["config"]["workload"]
 
 
+def _dumped_rgb_sha256(path):
+    import hashlib
+    import numpy as np
+    px = np.load(path)
+    assert px.dtype == np.float32 and px.shape == (1024 * 768, 4)
+    assert (px == np.round(px)).all() and px.min() >= 0 and px.max() <= 255
+    return hashlib.sha256(np.ascontiguousarray(px[:, :3].astype(np.uint8)).tobytes()).hexdigest()
+
+
+def test_reference_arm_dumps_the_frame_it_rendered(tmp_path):
+    """--dump-outputs: c1 (`make image`) is small enough to be written whole; its pixels are the reference's image."""
+    r = run_bench("--impl", "reference", "--workload", "c1", "--steps", "1", "--warmup", "0",
+                  "--dump-outputs", str(tmp_path / "out"))
+    assert r.returncode == 0, r.stderr
+    gold = json.load(open(os.path.join(ROOT, "tests", "golden", "rtrace_output_1024x768.json")))
+    assert os.listdir(tmp_path / "out") == ["c1.npy"]
+    assert _dumped_rgb_sha256(tmp_path / "out" / "c1.npy") == gold["rgb_sha256"]
+
+
+def test_dump_of_a_large_frame_is_a_fixed_sample():
+    """A frame larger than the run's share of the dump budget is sampled: the same pixels in every run, row-major."""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    h, w = 2160, 3840
+    frame = np.full((h, w, 4), 7, np.uint8)
+    idx = np.arange(h * w, dtype=np.int64)   # every pixel's index, spelled in base 251 over R, G, B
+    frame[:, :, 0] = (idx % 251).reshape(h, w)
+    frame[:, :, 1] = (idx // 251 % 251).reshape(h, w)
+    frame[:, :, 2] = (idx // 251 ** 2 % 251).reshape(h, w)
+    n = bench.dump_pixels(3)
+    a, b = bench.sample_pixels(frame, n), bench.sample_pixels(frame.copy(), n)
+    assert a.dtype == np.float32 and a.shape == (n, 4) and n < h * w and np.array_equal(a, b)
+    where = a[:, 0].astype(np.int64) + 251 * a[:, 1].astype(np.int64) + 251 ** 2 * a[:, 2].astype(np.int64)
+    assert (np.diff(where) > 0).all() and where[-1] < h * w
+    assert np.array_equal(a, frame.reshape(-1, 4)[where].astype(np.float32))
+
+
+@pytest.mark.parametrize("argv", [[], ["--no-also"], ["--workload", "c4"], ["--workload", "c4", "--mode", "bands"],
+                                  ["--impl", "reference"]], ids=lambda a: " ".join(a) or "default")
+def test_dumps_of_a_run_stay_within_64_mb_at_any_gpu_count(tmp_path, argv):
+    """--dump-outputs writes one file per measurement, from rank 0 only, and sizes the samples so that all files of a
+    run together stay within 64 MB whatever the number of ranks; a file outside that plan is refused."""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    frames = {}
+    for world in (1, 2, 8):
+        out = tmp_path / str(world)
+        args = bench.parse_args(argv + ["--gpus", str(world), "--dump-outputs", str(out)])
+        names = bench.dump_names(args, world)
+        for name in names:
+            w, h = bench.WORKLOADS[name.replace("_bands", "")][:2]
+            if (w, h) not in frames:
+                frames[w, h] = np.zeros((h, w, 4), np.uint8)
+            bench.dump_frame(args, world, name, frames[w, h])
+        assert sorted(os.listdir(out)) == sorted(n + ".npy" for n in names)
+        assert sum(os.path.getsize(out / f) for f in os.listdir(out)) <= 64 * 10 ** 6, (argv, world)
+        with pytest.raises(RuntimeError):
+            bench.dump_frame(args, world, "c3", frames[next(iter(frames))])
+    if not argv:   # the default run: c5 + c2 + c4 on one rank, + the 8K band split on more
+        assert bench.dump_names(bench.parse_args([]), 1) == ["c5", "c2", "c4"]
+        assert bench.dump_names(bench.parse_args([]), 8) == ["c5", "c2", "c4", "c4_bands"]
+
+
+@pytest.mark.gpu
+def test_native_arm_dumps_its_last_frames_and_times_every_step(tmp_path, oracle):
+    """A default run at --steps 2: every measurement (c5 and the c2 / c4 sub-records, kernel-only and end to end) times
+    exactly 2 steps, and the dumped c2 sample is the oracle's frame at the same pixels."""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    r = run_bench("--steps", "2", "--warmup", "3", "--no-cpu-baseline", "--dump-outputs", str(tmp_path / "out"))
+    assert r.returncode == 0, r.stderr
+    d = json.loads(r.stdout)
+    assert d["steps"] == 2 and d["e2e"]["steps"] == 2
+    for sub in ("c2", "c4"):
+        assert d["also"][sub]["steps"] == 2 and d["also"][sub]["e2e"]["steps"] == 2, sub
+    files = sorted(os.listdir(tmp_path / "out"))
+    assert files == ["c2.npy", "c4.npy", "c5.npy"]
+    assert sum(os.path.getsize(tmp_path / "out" / f) for f in files) <= 64 * 10 ** 6
+    got = np.load(tmp_path / "out" / "c2.npy")
+    w, h, spp, level = bench.WORKLOADS["c2"]
+    ref, _ = oracle.Scene(level=level).render(w, h, spp)
+    assert np.array_equal(got, bench.sample_pixels(ref, len(got)))
+
+
 def test_reference_arm_runs_on_rank_zero_only():
     r = run_bench("--impl", "reference", "--workload", "c1", "--steps", "1", "--gpus", "2",
                   env={"RANK": "1", "WORLD_SIZE": "2", "LOCAL_RANK": "1"})
