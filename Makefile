@@ -12,8 +12,8 @@ ARCH      := -gencode arch=compute_100a,code=sm_100a
 # -fmad=false + *_rn intrinsics: no FMA contraction on the parity-critical path (SURVEY F3).
 NVFLAGS   := $(ARCH) -O3 -std=c++17 -lineinfo -fmad=false -prec-div=true -prec-sqrt=true \
              -Xcompiler -fPIC,-ffp-contract=off,-fno-fast-math,-Wall -Xptxas -v
-LIBSRC    := $(CSRC)/rt_kernels.cu $(CSRC)/rt_tile.cu $(CSRC)/rt_phased.cu $(CSRC)/rt_api.cpp $(CSRC)/rt_scene.cpp
-LIBHDR    := $(CSRC)/rt_device.cuh $(CSRC)/rt_cull.cuh $(CSRC)/rt_pack.cuh $(CSRC)/rt_kernels.h $(CSRC)/rt_scene.h include/rtrace.h
+LIBSRC    := $(CSRC)/rt_kernels.cu $(CSRC)/rt_tile.cu $(CSRC)/rt_phased.cu $(CSRC)/rt_png.cu $(CSRC)/rt_api.cpp $(CSRC)/rt_scene.cpp
+LIBHDR    := $(CSRC)/rt_device.cuh $(CSRC)/rt_cull.cuh $(CSRC)/rt_pack.cuh $(CSRC)/rt_kernels.h $(CSRC)/rt_png.h $(CSRC)/rt_scene.h include/rtrace.h
 
 all: rtrace
 

@@ -226,6 +226,25 @@ int rt_render_sweep_multi(rt_scene *const *scenes, int ngpu, const rt_camera *ca
                           uint32_t width, uint32_t height, uint32_t spp, int rgb,
                           rt_frame_callback cb, void *user, rt_stats *stats);
 
+/* ---- PNG output, encoded on the GPU ------------------------------------------------------------------------
+ * One fixed layout, so there is exactly one file per image (DESIGN.md "PNG output"): 8-bit RGB (alpha dropped, as
+ * the P6 sink does), one IDAT chunk per band of 16 rows, every row one byte-aligned fixed-Huffman deflate block of
+ * literals and distance-3 matches.  Any PNG decoder reads it. */
+/* Worst-case size of rt_encode_png's output for a width x height frame (1..65535 each). */
+int rt_png_bound(uint32_t width, uint32_t height, size_t *bytes);
+/* PNG file (layout above) of a width x height RGBA8 frame in device memory of the current device
+ * (pitch 0 = width*4; alpha is dropped).  png_out: host or device memory.  Waits for `stream` and
+ * returns the file length in *len_out; RT_ERR_BUFFER (with *len_out = the needed size) if cap is short;
+ * RT_ERR_INVALID for a host rgba pointer or a zero size. */
+int rt_encode_png(const uint8_t *rgba, uint32_t width, uint32_t height, size_t pitch_bytes,
+                  uint8_t *png_out, size_t cap, size_t *len_out, void *stream);
+/* rt_render_sweep_multi delivering each frame as a complete PNG file (len = file size), in frame order,
+ * on the calling thread; ngpu == 1 is the single-GPU pipelined sweep.  Each frame is encoded on its GPU behind
+ * its render launches and only the file's bytes cross the host link. */
+int rt_render_sweep_png(rt_scene *const *scenes, int ngpu, const rt_camera *cameras, uint32_t n_frames,
+                        uint32_t width, uint32_t height, uint32_t spp,
+                        rt_frame_callback cb, void *user, rt_stats *stats);
+
 /* Count rays the way the reference's work is counted (SURVEY 8d): primary =
  * rows*width*spp^2, shadow = samples with a hit facing the light. */
 int rt_count_rays(const rt_scene *s, const rt_camera *camera,

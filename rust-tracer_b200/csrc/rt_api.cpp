@@ -15,6 +15,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <map>
+#include <memory>
 #include <mutex>
 #include <new>
 #include <thread>
@@ -22,6 +23,7 @@
 
 #include "rt_device.cuh"
 #include "rt_kernels.h"
+#include "rt_png.h"
 #include "rt_scene.h"
 
 // ---------------------------------------------------------------------------
@@ -64,8 +66,16 @@ struct rt_scene {
     int sweep_nb = 0;  // buffers of the ring that are allocated
     cudaStream_t copy_stream = nullptr, render2 = nullptr;
     cudaEvent_t sweep_rendered[SWEEP_RING] = {nullptr, nullptr, nullptr}, sweep_copied[SWEEP_RING] = {nullptr, nullptr, nullptr};
+    size_t sweep_host_bytes = 0;  // size of each sweep_host buffer
     std::map<cudaStream_t, Phased> phased;
     std::mutex mu_phased;  // guards the map only (mu may already be held by the caller)
+    // rt_render_sweep_png: the encoded file of each ring buffer (its length word after it), the lengths read back to
+    // the host, and the encoder's scratch, one per render stream
+    uint8_t *sweep_png[SWEEP_RING] = {nullptr, nullptr, nullptr};
+    size_t sweep_png_cap[SWEEP_RING] = {0, 0, 0};
+    unsigned long long *sweep_len_host = nullptr;
+    cudaEvent_t sweep_len_ready[SWEEP_RING] = {nullptr, nullptr, nullptr};
+    std::map<cudaStream_t, std::pair<uint8_t *, size_t>> png_scratch;
 };
 
 namespace {
@@ -80,6 +90,9 @@ struct RowLayout {
     uint32_t block_shift = 0;
     bool out_abs = false;
 };
+
+// What a sweep hands to its frame callback: the RGBA8 frame, its RGB8 bytes (the P6 body), or a PNG file.
+enum class OutKind { RGBA, RGB, PNG };
 
 int fail(int code, const char *fmt, ...) {
     va_list ap;
@@ -345,6 +358,13 @@ int launch(rt_scene *s, rt::RenderParams &p, bool diag, cudaStream_t stream) {
     return RT_OK;
 }
 
+// rt_encode_png's device buffers for one (device, stream); `mu` serialises the calls that share them.
+struct PngEncodeScratch {
+    std::mutex mu;
+    uint8_t *scratch = nullptr, *out = nullptr;  // out: the file, then its length word
+    size_t scratch_cap = 0, out_cap = 0;
+};
+
 int launches_per_frame(const rt::RenderParams &p) { return kernel_variant(p) == RT_KERNEL_PHASED ? 4 : 1; }
 // RT_KERNEL_* and RT_VARIANT_* share their numbering (rt_kernels.h, rtrace.h)
 uint32_t variant_used(const rt::RenderParams &p) { return (uint32_t)kernel_variant(p); }
@@ -449,7 +469,12 @@ void rt_scene_destroy(rt_scene *s) {
             if (s->sweep_host[k]) cudaFreeHost(s->sweep_host[k]);
             if (s->sweep_rendered[k]) cudaEventDestroy(s->sweep_rendered[k]);
             if (s->sweep_copied[k]) cudaEventDestroy(s->sweep_copied[k]);
+            if (s->sweep_png[k]) cudaFree(s->sweep_png[k]);
+            if (s->sweep_len_ready[k]) cudaEventDestroy(s->sweep_len_ready[k]);
         }
+        if (s->sweep_len_host) cudaFreeHost(s->sweep_len_host);
+        for (auto &kv : s->png_scratch)
+            if (kv.second.first) cudaFree(kv.second.first);
         if (s->copy_stream) cudaStreamDestroy(s->copy_stream);
         if (s->render2) cudaStreamDestroy(s->render2);
         for (auto &kv : s->phased) {
@@ -748,10 +773,19 @@ struct CallbackSource : FrameSource {
 };
 
 static int sweep_locked(rt_scene *s, FrameSource &src, uint32_t width, uint32_t height, uint32_t spp, rt_frame_callback cb,
-                        void *user, rt_stats *stats, bool rgb);
+                        void *user, rt_stats *stats, OutKind kind);
+
+// The PNG encoder's scratch for this render stream (allocated on first use, grown on demand): two frames in flight
+// on two streams encode at the same time.
+static int png_scratch_for(rt_scene *s, cudaStream_t stream, uint32_t width, uint32_t height, uint8_t **out) {
+    std::pair<uint8_t *, size_t> &sc = s->png_scratch[stream];
+    int rc = ensure(&sc.first, &sc.second, rt_png_scratch_bytes(width, height));
+    *out = sc.first;
+    return rc;
+}
 
 static int sweep_impl(const rt_scene *cs, FrameSource &src, uint32_t width, uint32_t height, uint32_t spp,
-                      rt_frame_callback cb, void *user, rt_stats *stats, bool rgb) {
+                      rt_frame_callback cb, void *user, rt_stats *stats, OutKind kind) {
     rt_scene *s = const_cast<rt_scene *>(cs);
     int rc = check_frame_args(s, width, height, spp, 0, 1, height);
     if (rc != RT_OK) return rc;
@@ -759,7 +793,7 @@ static int sweep_impl(const rt_scene *cs, FrameSource &src, uint32_t width, uint
     DeviceGuard guard(s->device);
     if (!guard.ok) return fail(RT_ERR_CUDA, "cannot select device %d", s->device);
     std::lock_guard<std::mutex> lock(s->mu);
-    rc = sweep_locked(s, src, width, height, spp, cb, user, stats, rgb);
+    rc = sweep_locked(s, src, width, height, spp, cb, user, stats, kind);
     if (rc != RT_OK) {  // leave no render or copy in flight on the ring buffers (keeps the first error text)
         if (s->own_stream) cudaStreamSynchronize(s->own_stream);
         if (s->render2) cudaStreamSynchronize(s->render2);
@@ -770,11 +804,14 @@ static int sweep_impl(const rt_scene *cs, FrameSource &src, uint32_t width, uint
 }
 
 static int sweep_locked(rt_scene *s, FrameSource &src, uint32_t width, uint32_t height, uint32_t spp, rt_frame_callback cb,
-                        void *user, rt_stats *stats, bool rgb) {
+                        void *user, rt_stats *stats, OutKind kind) {
     int rc = RT_OK;
     const double t0 = now_ms();
+    const bool rgb = kind == OutKind::RGB, png = kind == OutKind::PNG;
     const size_t row_bytes = (size_t)width * 4, frame_bytes = row_bytes * height;
     const size_t out_bytes = rgb ? (size_t)width * height * 3 : frame_bytes;
+    const size_t png_bytes = png ? rt_png_bound_bytes(width, height) : 0, png_len_at = (png_bytes + 7) / 8 * 8;
+    const size_t host_bytes = std::max(frame_bytes, png_bytes);
     // `depth` frames render at a time, each on its own stream (depth 2: the launch tails of frame f are filled
     // by the first launches of frame f+1), while an earlier frame is copied out: depth + 1 device frames and
     // pinned host frames.  Measured on B200 (C5, 4K 4x4 level 9): 1.395 ms per delivered frame with one render
@@ -785,23 +822,32 @@ static int sweep_locked(rt_scene *s, FrameSource &src, uint32_t width, uint32_t 
         if (*e == '1') depth = 1;
     }
     const int nb = depth + 1;
-    if (s->sweep_bytes < frame_bytes || s->sweep_nb < nb) {
+    if (s->sweep_bytes < frame_bytes || s->sweep_host_bytes < host_bytes || s->sweep_nb < nb) {
         for (int k = 0; k < rt_scene::SWEEP_RING; k++) {
             if (s->sweep_dev[k]) cudaFree(s->sweep_dev[k]);
             if (s->sweep_host[k]) cudaFreeHost(s->sweep_host[k]);
             s->sweep_dev[k] = s->sweep_host[k] = nullptr;
         }
         s->sweep_bytes = 0;
+        s->sweep_host_bytes = 0;
         s->sweep_nb = 0;
         for (int k = 0; k < nb; k++) {
             if (s->sweep_rgb[k]) cudaFree(s->sweep_rgb[k]);
             s->sweep_rgb[k] = nullptr;
             CUDA_TRY(cudaMalloc(&s->sweep_dev[k], frame_bytes));
             CUDA_TRY(cudaMalloc(&s->sweep_rgb[k], frame_bytes / 4 * 3 + 16));
-            CUDA_TRY(cudaHostAlloc((void **)&s->sweep_host[k], frame_bytes, cudaHostAllocPortable));
+            CUDA_TRY(cudaHostAlloc((void **)&s->sweep_host[k], host_bytes, cudaHostAllocPortable));
         }
         s->sweep_bytes = frame_bytes;
+        s->sweep_host_bytes = host_bytes;
         s->sweep_nb = nb;
+    }
+    if (png) {
+        for (int k = 0; k < nb; k++) {
+            rc = ensure(&s->sweep_png[k], &s->sweep_png_cap[k], png_len_at + sizeof(unsigned long long));
+            if (rc != RT_OK) return rc;
+        }
+        if (!s->sweep_len_host) CUDA_TRY(cudaHostAlloc((void **)&s->sweep_len_host, sizeof(unsigned long long) * rt_scene::SWEEP_RING, cudaHostAllocPortable));
     }
     if (depth == 2 && !s->render2) CUDA_TRY(cudaStreamCreateWithFlags(&s->render2, cudaStreamNonBlocking));
     if (!s->copy_stream) {
@@ -809,6 +855,7 @@ static int sweep_locked(rt_scene *s, FrameSource &src, uint32_t width, uint32_t 
         for (int k = 0; k < rt_scene::SWEEP_RING; k++) {
             CUDA_TRY(cudaEventCreateWithFlags(&s->sweep_rendered[k], cudaEventDisableTiming));
             CUDA_TRY(cudaEventCreateWithFlags(&s->sweep_copied[k], cudaEventDisableTiming));
+            CUDA_TRY(cudaEventCreateWithFlags(&s->sweep_len_ready[k], cudaEventDisableTiming));
         }
     }
     uint32_t launches = 0, used = 0;
@@ -839,18 +886,39 @@ static int sweep_locked(rt_scene *s, FrameSource &src, uint32_t width, uint32_t 
                     CUDA_TRY(rt_launch_pack_rgb(s->sweep_dev[k], s->sweep_rgb[k], (size_t)width * height, rs));
                     launches += 1;
                 }
-                CUDA_TRY(cudaEventRecord(s->sweep_rendered[k], rs));
-                CUDA_TRY(cudaStreamWaitEvent(s->copy_stream, s->sweep_rendered[k], 0));
-                CUDA_TRY(cudaMemcpyAsync(s->sweep_host[k], rgb ? s->sweep_rgb[k] : s->sweep_dev[k], out_bytes, cudaMemcpyDeviceToHost, s->copy_stream));
-                CUDA_TRY(cudaEventRecord(s->sweep_copied[k], s->copy_stream));
+                if (png) {
+                    // encode behind the frame's launches; only the length word comes back now (on the render
+                    // stream, so that the copy stream never waits for a later frame); the file is copied at hand-over
+                    uint8_t *scratch = nullptr;
+                    rc = png_scratch_for(s, rs, width, height, &scratch);
+                    if (rc != RT_OK) return rc;
+                    unsigned long long *len_word = reinterpret_cast<unsigned long long *>(s->sweep_png[k] + png_len_at);
+                    CUDA_TRY(rt_launch_png_encode(s->sweep_dev[k], row_bytes, width, height, scratch, s->sweep_png[k], len_word, rs));
+                    CUDA_TRY(cudaMemcpyAsync(&s->sweep_len_host[k], len_word, sizeof(unsigned long long), cudaMemcpyDeviceToHost, rs));
+                    CUDA_TRY(cudaEventRecord(s->sweep_len_ready[k], rs));
+                    launches += 2;
+                } else {
+                    CUDA_TRY(cudaEventRecord(s->sweep_rendered[k], rs));
+                    CUDA_TRY(cudaStreamWaitEvent(s->copy_stream, s->sweep_rendered[k], 0));
+                    CUDA_TRY(cudaMemcpyAsync(s->sweep_host[k], rgb ? s->sweep_rgb[k] : s->sweep_dev[k], out_bytes, cudaMemcpyDeviceToHost, s->copy_stream));
+                    CUDA_TRY(cudaEventRecord(s->sweep_copied[k], s->copy_stream));
+                }
                 issued++;
             }
         }
         if (issued - delivered > (uint64_t)depth || (!more && delivered < issued)) {
             // hand the oldest frame to the caller while the later ones render
             const int k = (int)(delivered % (uint64_t)nb);
+            size_t len = out_bytes;
+            if (png) {  // the file's length first, then just that many bytes
+                CUDA_TRY(cudaEventSynchronize(s->sweep_len_ready[k]));
+                len = (size_t)s->sweep_len_host[k];
+                if (len > png_bytes) return fail(RT_ERR_CUDA, "PNG encoder returned %zu bytes, more than the bound %zu", len, png_bytes);
+                CUDA_TRY(cudaMemcpyAsync(s->sweep_host[k], s->sweep_png[k], len, cudaMemcpyDeviceToHost, s->copy_stream));
+                CUDA_TRY(cudaEventRecord(s->sweep_copied[k], s->copy_stream));
+            }
             CUDA_TRY(cudaEventSynchronize(s->sweep_copied[k]));
-            if (cb) cb(user, (uint32_t)ids[k], s->sweep_host[k], out_bytes);
+            if (cb) cb(user, (uint32_t)ids[k], s->sweep_host[k], len);
             delivered++;
         }
     }
@@ -867,20 +935,20 @@ static int sweep_locked(rt_scene *s, FrameSource &src, uint32_t width, uint32_t 
 int rt_render_sweep(const rt_scene *s, const rt_camera *cameras, uint32_t n_frames, uint32_t width, uint32_t height,
                     uint32_t spp, rt_frame_callback cb, void *user, rt_stats *stats) {
     ListSource src(cameras, n_frames);
-    return sweep_impl(s, src, width, height, spp, cb, user, stats, false);
+    return sweep_impl(s, src, width, height, spp, cb, user, stats, OutKind::RGBA);
 }
 
 int rt_render_sweep_rgb(const rt_scene *s, const rt_camera *cameras, uint32_t n_frames, uint32_t width, uint32_t height,
                         uint32_t spp, rt_frame_callback cb, void *user, rt_stats *stats) {
     ListSource src(cameras, n_frames);
-    return sweep_impl(s, src, width, height, spp, cb, user, stats, true);
+    return sweep_impl(s, src, width, height, spp, cb, user, stats, OutKind::RGB);
 }
 
 int rt_render_sweep_pull(const rt_scene *s, rt_next_frame_callback next, void *next_user, uint32_t width, uint32_t height,
                          uint32_t spp, int rgb, rt_frame_callback cb, void *user, rt_stats *stats) {
     if (!next) return fail(RT_ERR_INVALID, "next-frame callback is NULL");
     CallbackSource src(next, next_user);
-    return sweep_impl(s, src, width, height, spp, cb, user, stats, rgb != 0);
+    return sweep_impl(s, src, width, height, spp, cb, user, stats, rgb ? OutKind::RGB : OutKind::RGBA);
 }
 
 // Body of rt_render_frame_multi once every scene's scratch is locked.  `launched` records the GPUs that have
@@ -1089,12 +1157,8 @@ void board_offer(void *user, uint32_t frame, const uint8_t *data, size_t len) {
     b.cv.wait(lock, [&] { return b.abort || b.next_deliver != frame; });
 }
 
-}  // namespace
-
-extern "C" {
-
-int rt_render_sweep_multi(rt_scene *const *scenes, int ngpu, const rt_camera *cameras, uint32_t n_frames, uint32_t width,
-                          uint32_t height, uint32_t spp, int rgb, rt_frame_callback cb, void *user, rt_stats *stats) {
+static int sweep_multi_impl(rt_scene *const *scenes, int ngpu, const rt_camera *cameras, uint32_t n_frames, uint32_t width,
+                            uint32_t height, uint32_t spp, OutKind kind, rt_frame_callback cb, void *user, rt_stats *stats) {
     if (!scenes || ngpu < 1) return fail(RT_ERR_INVALID, "need at least one scene");
     for (int g = 0; g < ngpu; g++) {
         int rc = check_frame_args(scenes[g], width, height, spp, 0, 1, height);
@@ -1104,7 +1168,7 @@ int rt_render_sweep_multi(rt_scene *const *scenes, int ngpu, const rt_camera *ca
     if (n_frames == 0) return RT_OK;
     if (ngpu == 1) {
         ListSource src(cameras, n_frames);
-        return sweep_impl(scenes[0], src, width, height, spp, cb, user, stats, rgb != 0);
+        return sweep_impl(scenes[0], src, width, height, spp, cb, user, stats, kind);
     }
     {   // distinct scenes (each worker locks its own)
         std::vector<rt_scene *> order(scenes, scenes + ngpu);
@@ -1125,7 +1189,7 @@ int rt_render_sweep_multi(rt_scene *const *scenes, int ngpu, const rt_camera *ca
         workers.emplace_back([&, g, variant]() {
             g_variant = variant;
             BoardSource src(board);
-            const int rc = sweep_impl(scenes[g], src, width, height, spp, board_offer, &board, &wstats[(size_t)g], rgb != 0);
+            const int rc = sweep_impl(scenes[g], src, width, height, spp, board_offer, &board, &wstats[(size_t)g], kind);
             std::lock_guard<std::mutex> lock(board.mu);
             if (rc != RT_OK && board.rc == RT_OK) {
                 board.rc = rc;
@@ -1169,6 +1233,21 @@ int rt_render_sweep_multi(rt_scene *const *scenes, int ngpu, const rt_camera *ca
         stats->variant_used = wstats[0].variant_used;
     }
     return RT_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int rt_render_sweep_multi(rt_scene *const *scenes, int ngpu, const rt_camera *cameras, uint32_t n_frames, uint32_t width,
+                          uint32_t height, uint32_t spp, int rgb, rt_frame_callback cb, void *user, rt_stats *stats) {
+    return sweep_multi_impl(scenes, ngpu, cameras, n_frames, width, height, spp, rgb ? OutKind::RGB : OutKind::RGBA, cb,
+                            user, stats);
+}
+
+int rt_render_sweep_png(rt_scene *const *scenes, int ngpu, const rt_camera *cameras, uint32_t n_frames, uint32_t width,
+                        uint32_t height, uint32_t spp, rt_frame_callback cb, void *user, rt_stats *stats) {
+    return sweep_multi_impl(scenes, ngpu, cameras, n_frames, width, height, spp, OutKind::PNG, cb, user, stats);
 }
 
 uint64_t rt_atomic_fetch_add_u64(void *addr, uint64_t value) {
@@ -1351,6 +1430,57 @@ int rt_pack_rgb_rows(const uint8_t *rgba_frame, uint8_t *rgb_frame, uint32_t wid
         return fail(RT_ERR_INVALID, "row blocks must start at multiples of 4 pixels (row_start %u, row_stride %u, width %u)", row_start, row_stride, width);
     if ((((uintptr_t)rgba_frame) & 15) || (((uintptr_t)rgb_frame) & 3)) return fail(RT_ERR_INVALID, "buffers must be 16- / 4-byte aligned");
     CUDA_TRY(rt_launch_pack_rgb_blocks(rgba_frame, rgb_frame, width, height, row_start, row_stride, row_block, (cudaStream_t)stream));
+    return RT_OK;
+}
+
+int rt_png_bound(uint32_t width, uint32_t height, size_t *bytes) {
+    if (!bytes) return fail(RT_ERR_INVALID, "NULL argument");
+    if (width == 0 || height == 0 || width > 65535u || height > 65535u)
+        return fail(RT_ERR_INVALID, "width/height must be in 1..65535 (got %u x %u)", width, height);
+    *bytes = rt_png_bound_bytes(width, height);
+    return RT_OK;
+}
+
+int rt_encode_png(const uint8_t *rgba, uint32_t width, uint32_t height, size_t pitch_bytes, uint8_t *png_out, size_t cap,
+                  size_t *len_out, void *stream_) {
+    if (!rgba || !len_out || (!png_out && cap)) return fail(RT_ERR_INVALID, "NULL argument");
+    *len_out = 0;
+    size_t bound = 0;
+    int rc = rt_png_bound(width, height, &bound);
+    if (rc != RT_OK) return rc;
+    const size_t row_bytes = (size_t)width * 4;
+    if (pitch_bytes == 0) pitch_bytes = row_bytes;
+    if (pitch_bytes < row_bytes) return fail(RT_ERR_INVALID, "pitch %zu is smaller than a row (%zu bytes)", pitch_bytes, row_bytes);
+    int dev = -1, cur = -1;
+    if (!is_device_ptr(rgba, &dev)) return fail(RT_ERR_INVALID, "rgba must be device memory");
+    CUDA_TRY(cudaGetDevice(&cur));
+    if (dev != cur) return fail(RT_ERR_INVALID, "rgba lives on device %d, the current device is %d", dev, cur);
+    cudaStream_t stream = (cudaStream_t)stream_;
+    // scratch per (device, stream), kept for the life of the process: no allocation per call once it has grown
+    static std::mutex g_mu;
+    static std::map<std::pair<int, cudaStream_t>, std::unique_ptr<PngEncodeScratch>> g_scratch;
+    PngEncodeScratch *sc;
+    {
+        std::lock_guard<std::mutex> lock(g_mu);
+        std::unique_ptr<PngEncodeScratch> &slot = g_scratch[std::make_pair(cur, stream)];
+        if (!slot) slot.reset(new (std::nothrow) PngEncodeScratch());
+        if (!slot) return fail(RT_ERR_NOMEM, "out of host memory");
+        sc = slot.get();
+    }
+    std::lock_guard<std::mutex> lock(sc->mu);
+    const size_t len_at = (bound + 7) / 8 * 8;
+    rc = ensure(&sc->scratch, &sc->scratch_cap, rt_png_scratch_bytes(width, height));
+    if (rc == RT_OK) rc = ensure(&sc->out, &sc->out_cap, len_at + sizeof(unsigned long long));
+    if (rc != RT_OK) return rc;
+    unsigned long long *len_word = reinterpret_cast<unsigned long long *>(sc->out + len_at), len = 0;
+    CUDA_TRY(rt_launch_png_encode(rgba, pitch_bytes, width, height, sc->scratch, sc->out, len_word, stream));
+    CUDA_TRY(cudaMemcpyAsync(&len, len_word, sizeof(len), cudaMemcpyDeviceToHost, stream));
+    CUDA_TRY(cudaStreamSynchronize(stream));
+    if (len == 0 || len > bound) return fail(RT_ERR_CUDA, "PNG encoder returned %llu bytes (bound %zu)", len, bound);
+    *len_out = (size_t)len;
+    if (len > cap) return fail(RT_ERR_BUFFER, "png_out holds %zu bytes, the file needs %llu", cap, len);
+    CUDA_TRY(cudaMemcpyAsync(png_out, sc->out, (size_t)len, cudaMemcpyDefault, stream));
+    CUDA_TRY(cudaStreamSynchronize(stream));
     return RT_OK;
 }
 

@@ -12,7 +12,8 @@
 // Additive flags: --level=L (scene depth, default 8 as at render.rs:147),
 // --gpus=N / RTRACE_GPUS (default 1: one frame = interleaved row blocks over the GPUs; a sweep = the GPUs draw
 // frames from one queue), --frames=K (orbit sweep; frame f goes to <stem>.f.tga, frame 0 is the reference camera), --stats (summary on stderr), --buckets (the reference's 64x64 bucket
-// schedule through Renderer::render_region instead of one launch per frame).
+// schedule through Renderer::render_region instead of one launch per frame), --format=tga|png (a real TGA, or a PNG
+// encoded on the GPU: the output is then named *.png and sweep frames <stem>.f.png).
 #include <cerrno>
 #include <chrono>
 #include <cmath>
@@ -53,14 +54,15 @@ const char *USAGE =
     "        --gpus <N>                         GPUs to render on: a frame is split into interleaved row blocks,\n"
     "                                           a sweep (--frames) into whole frames [default: 1 or RTRACE_GPUS]\n"
     "        --frames <K>                       Render a K-frame orbit of the camera [default: 1]\n"
-    "        --format <ppm|tga>                 File contents: the reference's binary PPM, or a real TGA [default: ppm]\n"
+    "        --format <ppm|tga|png>             File contents: the reference's binary PPM, a real TGA, or a PNG encoded\n"
+    "                                           on the GPU (the output is then named *.png) [default: ppm]\n"
     "        --preview <N>                      Undersampled preview: trace one pixel per NxN block (1 sample) [default: off]\n"
     "        --stats                            Print a timing summary to stderr\n"
     "        --buckets                          Render 64x64 buckets one by one in the reference's order (sizes must\n"
     "                                           be multiples of 64, as in the reference); default is whole frames\n"
     "\n"
     "ARGS:\n"
-    "    <output>    Either a file with .tga extension, or - to write file to stdout\n";
+    "    <output>    Either a file with .tga extension (.png with --format png), or - to write file to stdout\n";
 
 [[noreturn]] void usage_error(const std::string &msg) {
     // clap 2: message + usage hint on stderr, exit status 1
@@ -219,9 +221,11 @@ int main(int argc, char **argv) {
     const std::string &output_file = args.output;
     FileOrAnyWriter output;
     FILE *fp = nullptr;
+    const bool png = args.format == "png";
+    const std::string ext = png ? "png" : "tga";
     if (output_file != "-") {
-        if (extension_of(output_file) != "tga") {
-            printf("Output file '%s' must have the tga extension, e.g. %s\n", output_file.c_str(), with_extension(output_file, "tga").c_str());
+        if (extension_of(output_file) != ext) {
+            printf("Output file '%s' must have the %s extension, e.g. %s\n", output_file.c_str(), ext.c_str(), with_extension(output_file, ext).c_str());
             return 0;
         }
     }
@@ -237,8 +241,10 @@ int main(int argc, char **argv) {
     unsigned frames = (unsigned)parse_or_panic(args.frames.empty() ? "1" : args.frames, 100000, "frames");
     if (gpus < 1) gpus = 1;
     if (frames < 1) frames = 1;
-    if (!args.format.empty() && args.format != "ppm" && args.format != "tga")
-        usage_error("'" + args.format + "' isn't a valid value for '--format <ppm|tga>'");
+    if (!args.format.empty() && args.format != "ppm" && args.format != "tga" && !png)
+        usage_error("'" + args.format + "' isn't a valid value for '--format <ppm|tga|png>'");
+    // the bucket schedule exists to drive the host writer seam; a PNG is encoded on the GPU from a whole frame
+    if (png && args.buckets) usage_error("The argument '--buckets' cannot be used with '--format png'");
     const bool real_tga = args.format == "tga";
     const unsigned preview = args.preview.empty() ? 0u : (unsigned)parse_or_panic(args.preview, 1024, "preview");
     if (options.width == 0 || options.height == 0) {
@@ -255,7 +261,7 @@ int main(int argc, char **argv) {
         auto frame_path = [&](unsigned f) {
             if (frames == 1 || output_file == "-") return output_file;
             char suffix[32];
-            snprintf(suffix, sizeof(suffix), "%04u.tga", f);
+            snprintf(suffix, sizeof(suffix), "%04u.%s", f, ext.c_str());
             return with_extension(output_file, suffix);
         };
         auto open_output = [&](unsigned f) {
@@ -271,18 +277,27 @@ int main(int argc, char **argv) {
             for (unsigned f = 0; f < frames; f++) cams.push_back(orbit_camera(f, frames));
             rt_stats st;
             auto r0 = clk::now();
-            // frames arrive as RGB8: exactly the body PPMStdoutRGBABufferWriter would write (render.rs:377-397)
-            Renderer::render_sweep(options, scene, cams, [&](uint32_t f, const uint8_t *rgb, size_t len) {
-                output = open_output(f);
-                if (real_tga) {
-                    write_tga(output.f, options.width, options.height, rgb, (size_t)options.width * 3, 3);
-                } else {
-                    fprintf(output.f, "P6\n%u %u\n255\n", (unsigned)options.width, (unsigned)options.height);
-                    if (fwrite(rgb, 1, len, output.f) != len) throw Panic("write_all failed");
+            if (png) {  // frames arrive as complete PNG files
+                Renderer::render_sweep_png(options, scene, cams, [&](uint32_t f, const uint8_t *file, size_t len) {
+                    output = open_output(f);
+                    if (fwrite(file, 1, len, output.f) != len) throw Panic("write_all failed");
                     fflush(output.f);
-                }
-                if (fp) fclose(fp), fp = nullptr;
-            }, &st, true);
+                    if (fp) fclose(fp), fp = nullptr;
+                }, &st);
+            } else {
+                // frames arrive as RGB8: exactly the body PPMStdoutRGBABufferWriter would write (render.rs:377-397)
+                Renderer::render_sweep(options, scene, cams, [&](uint32_t f, const uint8_t *rgb, size_t len) {
+                    output = open_output(f);
+                    if (real_tga) {
+                        write_tga(output.f, options.width, options.height, rgb, (size_t)options.width * 3, 3);
+                    } else {
+                        fprintf(output.f, "P6\n%u %u\n255\n", (unsigned)options.width, (unsigned)options.height);
+                        if (fwrite(rgb, 1, len, output.f) != len) throw Panic("write_all failed");
+                        fflush(output.f);
+                    }
+                    if (fp) fclose(fp), fp = nullptr;
+                }, &st, true);
+            }
             render_ms += std::chrono::duration<double, std::milli>(clk::now() - r0).count();
             kernel_ms = 0.0;
         } else {
@@ -290,7 +305,12 @@ int main(int argc, char **argv) {
                 output = open_output(f);
                 rt_camera cam = orbit_camera(f, frames);
                 rt_stats st;
-                {
+                if (png) {
+                    auto r0 = clk::now();
+                    Renderer::render_png(options, scene, output.f, frames > 1 ? &cam : nullptr, preview, &st);
+                    render_ms += std::chrono::duration<double, std::milli>(clk::now() - r0).count();
+                    kernel_ms += preview ? 0.0 : st.kernel_ms;
+                } else {
                     std::unique_ptr<RGBABufferWriter> sink;
                     if (real_tga) sink.reset(new TGARGBABufferWriter(&output));
                     else sink.reset(new PPMStdoutRGBABufferWriter(true, &output));

@@ -349,29 +349,80 @@ struct Renderer {
     // own frames (copy-out of one frame overlapping the render of the next two), and `sink(f, bytes, len)` is
     // called once per frame, in frame order, on the calling thread -- the role of the reference's main thread
     // draining the channel into the writer (render.rs:301-307).  With rgb = true the frames arrive as RGB8
-    // (the body of the P6 file, alpha already dropped).  An exception thrown by the sink does not cross the C
-    // boundary: it is caught in the trampoline, the remaining frames are skipped, and it is rethrown here once
-    // the sweep has returned (no render or copy is left in flight on the library's buffers).
+    // (the body of the P6 file, alpha already dropped).  An exception thrown by the sink is rethrown here once the
+    // sweep has returned (sweep_through).
     template <class Sink>
     static void render_sweep(const RenderOptions &o, const Scene &scene, const std::vector<rt_camera> &cameras,
                              Sink &&sink, rt_stats *stats = nullptr, bool rgb = false) {
+        sweep_through(sink, "Renderer::render_sweep", [&](rt_frame_callback cb, void *user) {
+            return rt_render_sweep_multi(scene.replicas(), scene.gpus(), cameras.data(), (uint32_t)cameras.size(), o.width,
+                                         o.height, o.samples_per_pixel, rgb ? 1 : 0, cb, user, stats);
+        });
+    }
+
+    // The same sweep delivering every frame as a PNG file encoded on its GPU (extension): `sink(f, file, len)`.
+    template <class Sink>
+    static void render_sweep_png(const RenderOptions &o, const Scene &scene, const std::vector<rt_camera> &cameras,
+                                 Sink &&sink, rt_stats *stats = nullptr) {
+        sweep_through(sink, "Renderer::render_sweep_png", [&](rt_frame_callback cb, void *user) {
+            return rt_render_sweep_png(scene.replicas(), scene.gpus(), cameras.data(), (uint32_t)cameras.size(), o.width,
+                                       o.height, o.samples_per_pixel, cb, user, stats);
+        });
+    }
+
+    // One frame (or an undersampled preview when preview_step > 0) as a PNG file on `f` (extension): rendered into
+    // device memory of the first GPU (with several GPUs their kernels store their rows there) and encoded there,
+    // so only the file crosses the host link.
+    static void render_png(const RenderOptions &o, const Scene &scene, FILE *f, const rt_camera *camera = nullptr,
+                           uint32_t preview_step = 0, rt_stats *stats = nullptr) {
+        struct Buffers {
+            void *frame = nullptr, *file = nullptr;
+            ~Buffers() {
+                rt_device_free(frame);
+                rt_host_free(file);
+            }
+        } b;
+        const size_t frame_bytes = (size_t)o.width * o.height * 4;
+        size_t bound = 0, len = 0;
+        rt_check(rt_png_bound(o.width, o.height, &bound), "Renderer::render_png");
+        rt_check(rt_device_alloc(frame_bytes, &b.frame), "Renderer::render_png");
+        rt_check(rt_host_alloc(bound, &b.file), "Renderer::render_png");
+        uint8_t *frame = static_cast<uint8_t *>(b.frame);
+        if (preview_step)
+            rt_check(rt_render_preview(scene.replicas()[0], camera, o.width, o.height, preview_step, frame, frame_bytes, nullptr),
+                     "Renderer::render_preview");
+        else
+            rt_check(rt_render_frame_multi(scene.replicas(), scene.gpus(), camera, o.width, o.height, o.samples_per_pixel,
+                                           frame, frame_bytes, stats),
+                     "Renderer::render");
+        rt_check(rt_encode_png(frame, o.width, o.height, 0, static_cast<uint8_t *>(b.file), bound, &len, nullptr),
+                 "Renderer::render_png");
+        if (fwrite(b.file, 1, len, f) != len) throw Panic("write_all failed");
+        fflush(f);
+    }
+
+  private:
+    // `call(cb, user)` runs a sweep that hands each frame to `sink`.  An exception thrown by the sink does not cross
+    // the C boundary: it is caught in the trampoline, the remaining frames are skipped, and it is rethrown here once
+    // the sweep has returned (no render or copy is left in flight on the library's buffers).
+    template <class Sink, class Call>
+    static void sweep_through(Sink &sink, const char *what, Call &&call) {
         struct Ctx {
-            typename std::remove_reference<Sink>::type *sink;
+            Sink *sink;
             std::exception_ptr error;
         } ctx{&sink, nullptr};
-        auto trampoline = [](void *user, uint32_t frame, const uint8_t *rgba, size_t len) {
+        auto trampoline = [](void *user, uint32_t frame, const uint8_t *data, size_t len) {
             Ctx *c = static_cast<Ctx *>(user);
             if (c->error) return;  // a previous frame's sink failed: drain quietly
             try {
-                (*c->sink)(frame, rgba, len);
+                (*c->sink)(frame, data, len);
             } catch (...) {
                 c->error = std::current_exception();
             }
         };
-        const int rc = rt_render_sweep_multi(scene.replicas(), scene.gpus(), cameras.data(), (uint32_t)cameras.size(), o.width,
-                                             o.height, o.samples_per_pixel, rgb ? 1 : 0, trampoline, &ctx, stats);
+        const int rc = call(trampoline, &ctx);
         if (ctx.error) std::rethrow_exception(ctx.error);
-        rt_check(rc, "Renderer::render_sweep");
+        rt_check(rc, what);
     }
 };
 

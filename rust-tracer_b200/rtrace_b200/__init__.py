@@ -25,6 +25,7 @@ ABI_SYMBOLS = [
     "rt_scene_device", "rt_render_region", "rt_render_preview", "rt_render_rows", "rt_render_row_blocks", "rt_render_frame", "rt_render_sweep", "rt_render_sweep_rgb",
     "rt_render_frame_multi", "rt_render_sweep_multi", "rt_render_sweep_pull", "rt_atomic_fetch_add_u64",
     "rt_count_rays", "rt_trace_rays", "rt_measure_fp32_peak", "rt_microbench_fp32", "rt_selftest_math", "rt_debug_phased_tiles", "rt_host_alloc", "rt_host_free", "rt_host_register", "rt_host_unregister", "rt_microbench_d2h", "rt_device_alloc", "rt_device_free", "rt_ipc_export", "rt_ipc_open", "rt_ipc_close", "rt_memcpy", "rt_memcpy2d_async", "rt_pack_rgb_rows",
+    "rt_png_bound", "rt_encode_png", "rt_render_sweep_png",
 ]
 
 
@@ -123,6 +124,10 @@ def lib():
     L.rt_host_register.argtypes = [vp, C.c_size_t]
     L.rt_host_unregister.argtypes = [vp]
     L.rt_microbench_d2h.argtypes = [C.c_size_t, C.c_int, C.c_int, C.POINTER(C.c_double)]
+    L.rt_png_bound.argtypes = [u32, u32, C.POINTER(C.c_size_t)]
+    L.rt_encode_png.argtypes = [vp, u32, u32, C.c_size_t, vp, C.c_size_t, C.POINTER(C.c_size_t), vp]
+    L.rt_render_sweep_png.argtypes = [C.POINTER(vp), C.c_int, C.POINTER(Camera), u32, u32, u32, u32, FRAME_CALLBACK, vp,
+                                      C.POINTER(Stats)]
     if os.environ.get("RTRACE_B200_LIB"):
         L = real
     _lib = L
@@ -414,6 +419,23 @@ class Renderer:
         return st
 
     @staticmethod
+    def render_sweep_png(options, scenes, n_frames, cameras=None, on_frame=None):
+        """The frame-sharded sweep (render_sweep_multi) delivering every frame as a PNG file encoded on its GPU:
+        on_frame(f, bytes) in frame order on the calling thread; one scene is the single-GPU sweep."""
+        w, h, spp = options.width, options.height, options.samples_per_pixel
+        cams = (Camera * n_frames)(*cameras) if cameras is not None else None
+
+        def _cb(user, frame, ptr, nbytes):
+            if on_frame is not None:
+                on_frame(int(frame), C.string_at(ptr, nbytes))
+
+        cb = FRAME_CALLBACK(_cb)
+        st = Stats()
+        arr = (C.c_void_p * len(scenes))(*[s.handle for s in scenes])
+        _check(lib().rt_render_sweep_png(arr, len(scenes), cams, n_frames, w, h, spp, cb, None, C.byref(st)))
+        return st
+
+    @staticmethod
     def render_multi(options, scenes, camera=None, want_stats=False):
         """Whole frame on len(scenes) GPUs of this process, rows interleaved, gathered on GPU 0."""
         w, h, spp = options.width, options.height, options.samples_per_pixel
@@ -506,6 +528,23 @@ def pack_rgb_rows(rgba_ptr, rgb_ptr, width, height, row_start, row_stride, row_b
 
 def memcpy2d_async(dst, dpitch, src, spitch, width_bytes, rows, stream=None):
     _check(lib().rt_memcpy2d_async(C.c_void_p(dst), dpitch, C.c_void_p(src), spitch, width_bytes, rows, stream))
+
+
+def png_bound(width, height):
+    """Worst-case size of encode_png's file for a width x height frame (pure arithmetic, no device needed)."""
+    n = C.c_size_t()
+    _check(lib().rt_png_bound(width, height, C.byref(n)))
+    return n.value
+
+
+def encode_png(device_ptr, width, height, pitch=0, stream=None):
+    """PNG file (bytes) of a width x height RGBA8 frame in device memory of the current device (alpha dropped),
+    encoded on the GPU (rt_encode_png); waits for `stream`."""
+    cap = png_bound(width, height)
+    out = C.create_string_buffer(cap)
+    n = C.c_size_t()
+    _check(lib().rt_encode_png(C.c_void_p(device_ptr), width, height, pitch, out, cap, C.byref(n), stream))
+    return out.raw[:n.value]
 
 
 def ipc_close(ptr):

@@ -64,6 +64,12 @@ extern "C" {
                                 stats: *mut RtStats) -> c_int;
     pub fn rt_host_alloc(bytes: usize, out: *mut *mut c_void) -> c_int;
     pub fn rt_host_free(p: *mut c_void);
+    pub fn rt_png_bound(width: u32, height: u32, bytes: *mut usize) -> c_int;
+    pub fn rt_encode_png(rgba: *const u8, width: u32, height: u32, pitch_bytes: usize, png_out: *mut u8, cap: usize,
+                         len_out: *mut usize, stream: *mut c_void) -> c_int;
+    pub fn rt_render_sweep_png(scenes: *const *mut RtScene, ngpu: c_int, cameras: *const RtCamera, n_frames: u32,
+                               width: u32, height: u32, spp: u32, cb: RtFrameCallback, user: *mut c_void,
+                               stats: *mut RtStats) -> c_int;
 }
 
 pub fn last_error() -> String {
