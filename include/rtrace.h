@@ -245,6 +245,27 @@ int rt_render_sweep_png(rt_scene *const *scenes, int ngpu, const rt_camera *came
                         uint32_t width, uint32_t height, uint32_t spp,
                         rt_frame_callback cb, void *user, rt_stats *stats);
 
+/* ---- Animated PNG (APNG) of a sweep, encoded on the GPU ------------------------------------------------------
+ * One file per animation, written as one payload per frame (DESIGN.md "Animated PNG"): the file is the payloads of
+ * frames 0 .. n_frames-1 back to back.  Each frame's zlib stream is exactly that of its rt_encode_png file.  Frame 0
+ * carries the signature, IHDR, acTL (n_frames, loop for ever), its fcTL and its IDAT chunks, so a viewer without
+ * APNG support shows frame 0.  Every later frame is an fcTL and the same chunks as fdAT.  The last frame also carries
+ * IEND.  Every frame is full size and shows for delay_num / delay_den seconds. */
+/* Worst-case payload of one frame of a width x height, n_frames animation (pure arithmetic, no device).
+ * RT_ERR_INVALID for a size outside 1..65535, n_frames == 0, or sequence numbers beyond 2^31 - 1. */
+int rt_apng_bound(uint32_t width, uint32_t height, uint32_t n_frames, size_t *frame_bytes);
+/* Payload of frame `frame` of an n_frames animation from a width x height RGBA8 frame in device memory of the
+ * current device.  Errors as rt_encode_png, plus RT_ERR_INVALID when frame >= n_frames.  Uses rt_encode_png's
+ * scratch of this (device, stream). */
+int rt_encode_apng_frame(const uint8_t *rgba, uint32_t width, uint32_t height, size_t pitch_bytes, uint32_t frame,
+                         uint32_t n_frames, uint16_t delay_num, uint16_t delay_den, uint8_t *out, size_t cap,
+                         size_t *len_out, void *stream);
+/* rt_render_sweep_png delivering each frame's payload instead of a PNG file: the bytes handed to `cb`, concatenated
+ * in frame order, are the animation.  Each frame is encoded on the GPU that rendered it. */
+int rt_render_sweep_apng(rt_scene *const *scenes, int ngpu, const rt_camera *cameras, uint32_t n_frames,
+                         uint32_t width, uint32_t height, uint32_t spp, uint16_t delay_num, uint16_t delay_den,
+                         rt_frame_callback cb, void *user, rt_stats *stats);
+
 /* Count rays the way the reference's work is counted (SURVEY 8d): primary =
  * rows*width*spp^2, shadow = samples with a hit facing the light. */
 int rt_count_rays(const rt_scene *s, const rt_camera *camera,

@@ -91,8 +91,15 @@ struct RowLayout {
     bool out_abs = false;
 };
 
-// What a sweep hands to its frame callback: the RGBA8 frame, its RGB8 bytes (the P6 body), or a PNG file.
-enum class OutKind { RGBA, RGB, PNG };
+// What a sweep hands to its frame callback: the RGBA8 frame, its RGB8 bytes (the P6 body), a PNG file, or the
+// frame's payload of an animated PNG.
+enum class OutKind { RGBA, RGB, PNG, APNG };
+
+// The animation an APNG frame belongs to: its frame count and how long each frame shows (delay_num / delay_den s).
+struct Animation {
+    uint32_t n_frames = 0;
+    uint16_t delay_num = 0, delay_den = 0;
+};
 
 int fail(int code, const char *fmt, ...) {
     va_list ap;
@@ -773,7 +780,7 @@ struct CallbackSource : FrameSource {
 };
 
 static int sweep_locked(rt_scene *s, FrameSource &src, uint32_t width, uint32_t height, uint32_t spp, rt_frame_callback cb,
-                        void *user, rt_stats *stats, OutKind kind);
+                        void *user, rt_stats *stats, OutKind kind, const Animation &anim);
 
 // The PNG encoder's scratch for this render stream (allocated on first use, grown on demand): two frames in flight
 // on two streams encode at the same time.
@@ -785,7 +792,7 @@ static int png_scratch_for(rt_scene *s, cudaStream_t stream, uint32_t width, uin
 }
 
 static int sweep_impl(const rt_scene *cs, FrameSource &src, uint32_t width, uint32_t height, uint32_t spp,
-                      rt_frame_callback cb, void *user, rt_stats *stats, OutKind kind) {
+                      rt_frame_callback cb, void *user, rt_stats *stats, OutKind kind, const Animation &anim = Animation()) {
     rt_scene *s = const_cast<rt_scene *>(cs);
     int rc = check_frame_args(s, width, height, spp, 0, 1, height);
     if (rc != RT_OK) return rc;
@@ -793,7 +800,7 @@ static int sweep_impl(const rt_scene *cs, FrameSource &src, uint32_t width, uint
     DeviceGuard guard(s->device);
     if (!guard.ok) return fail(RT_ERR_CUDA, "cannot select device %d", s->device);
     std::lock_guard<std::mutex> lock(s->mu);
-    rc = sweep_locked(s, src, width, height, spp, cb, user, stats, kind);
+    rc = sweep_locked(s, src, width, height, spp, cb, user, stats, kind, anim);
     if (rc != RT_OK) {  // leave no render or copy in flight on the ring buffers (keeps the first error text)
         if (s->own_stream) cudaStreamSynchronize(s->own_stream);
         if (s->render2) cudaStreamSynchronize(s->render2);
@@ -804,13 +811,15 @@ static int sweep_impl(const rt_scene *cs, FrameSource &src, uint32_t width, uint
 }
 
 static int sweep_locked(rt_scene *s, FrameSource &src, uint32_t width, uint32_t height, uint32_t spp, rt_frame_callback cb,
-                        void *user, rt_stats *stats, OutKind kind) {
+                        void *user, rt_stats *stats, OutKind kind, const Animation &anim) {
     int rc = RT_OK;
     const double t0 = now_ms();
-    const bool rgb = kind == OutKind::RGB, png = kind == OutKind::PNG;
+    // an APNG frame takes the PNG path with another bound and another encode launch
+    const bool rgb = kind == OutKind::RGB, apng = kind == OutKind::APNG, png = kind == OutKind::PNG || apng;
     const size_t row_bytes = (size_t)width * 4, frame_bytes = row_bytes * height;
     const size_t out_bytes = rgb ? (size_t)width * height * 3 : frame_bytes;
-    const size_t png_bytes = png ? rt_png_bound_bytes(width, height) : 0, png_len_at = (png_bytes + 7) / 8 * 8;
+    const size_t png_bytes = apng ? rt_apng_bound_bytes(width, height) : png ? rt_png_bound_bytes(width, height) : 0;
+    const size_t png_len_at = (png_bytes + 7) / 8 * 8;
     const size_t host_bytes = std::max(frame_bytes, png_bytes);
     // `depth` frames render at a time, each on its own stream (depth 2: the launch tails of frame f are filled
     // by the first launches of frame f+1), while an earlier frame is copied out: depth + 1 device frames and
@@ -893,7 +902,11 @@ static int sweep_locked(rt_scene *s, FrameSource &src, uint32_t width, uint32_t 
                     rc = png_scratch_for(s, rs, width, height, &scratch);
                     if (rc != RT_OK) return rc;
                     unsigned long long *len_word = reinterpret_cast<unsigned long long *>(s->sweep_png[k] + png_len_at);
-                    CUDA_TRY(rt_launch_png_encode(s->sweep_dev[k], row_bytes, width, height, scratch, s->sweep_png[k], len_word, rs));
+                    if (apng)
+                        CUDA_TRY(rt_launch_apng_encode(s->sweep_dev[k], row_bytes, width, height, (uint32_t)id, anim.n_frames,
+                                                       anim.delay_num, anim.delay_den, scratch, s->sweep_png[k], len_word, rs));
+                    else
+                        CUDA_TRY(rt_launch_png_encode(s->sweep_dev[k], row_bytes, width, height, scratch, s->sweep_png[k], len_word, rs));
                     CUDA_TRY(cudaMemcpyAsync(&s->sweep_len_host[k], len_word, sizeof(unsigned long long), cudaMemcpyDeviceToHost, rs));
                     CUDA_TRY(cudaEventRecord(s->sweep_len_ready[k], rs));
                     launches += 2;
@@ -1158,7 +1171,8 @@ void board_offer(void *user, uint32_t frame, const uint8_t *data, size_t len) {
 }
 
 static int sweep_multi_impl(rt_scene *const *scenes, int ngpu, const rt_camera *cameras, uint32_t n_frames, uint32_t width,
-                            uint32_t height, uint32_t spp, OutKind kind, rt_frame_callback cb, void *user, rt_stats *stats) {
+                            uint32_t height, uint32_t spp, OutKind kind, rt_frame_callback cb, void *user, rt_stats *stats,
+                            const Animation &anim = Animation()) {
     if (!scenes || ngpu < 1) return fail(RT_ERR_INVALID, "need at least one scene");
     for (int g = 0; g < ngpu; g++) {
         int rc = check_frame_args(scenes[g], width, height, spp, 0, 1, height);
@@ -1168,7 +1182,7 @@ static int sweep_multi_impl(rt_scene *const *scenes, int ngpu, const rt_camera *
     if (n_frames == 0) return RT_OK;
     if (ngpu == 1) {
         ListSource src(cameras, n_frames);
-        return sweep_impl(scenes[0], src, width, height, spp, cb, user, stats, kind);
+        return sweep_impl(scenes[0], src, width, height, spp, cb, user, stats, kind, anim);
     }
     {   // distinct scenes (each worker locks its own)
         std::vector<rt_scene *> order(scenes, scenes + ngpu);
@@ -1189,7 +1203,7 @@ static int sweep_multi_impl(rt_scene *const *scenes, int ngpu, const rt_camera *
         workers.emplace_back([&, g, variant]() {
             g_variant = variant;
             BoardSource src(board);
-            const int rc = sweep_impl(scenes[g], src, width, height, spp, board_offer, &board, &wstats[(size_t)g], kind);
+            const int rc = sweep_impl(scenes[g], src, width, height, spp, board_offer, &board, &wstats[(size_t)g], kind, anim);
             std::lock_guard<std::mutex> lock(board.mu);
             if (rc != RT_OK && board.rc == RT_OK) {
                 board.rc = rc;
@@ -1248,6 +1262,17 @@ int rt_render_sweep_multi(rt_scene *const *scenes, int ngpu, const rt_camera *ca
 int rt_render_sweep_png(rt_scene *const *scenes, int ngpu, const rt_camera *cameras, uint32_t n_frames, uint32_t width,
                         uint32_t height, uint32_t spp, rt_frame_callback cb, void *user, rt_stats *stats) {
     return sweep_multi_impl(scenes, ngpu, cameras, n_frames, width, height, spp, OutKind::PNG, cb, user, stats);
+}
+
+int rt_render_sweep_apng(rt_scene *const *scenes, int ngpu, const rt_camera *cameras, uint32_t n_frames, uint32_t width,
+                         uint32_t height, uint32_t spp, uint16_t delay_num, uint16_t delay_den, rt_frame_callback cb,
+                         void *user, rt_stats *stats) {
+    size_t bound = 0;
+    const int rc = rt_apng_bound(width, height, n_frames, &bound);
+    if (rc != RT_OK) return rc;
+    Animation anim;
+    anim.n_frames = n_frames, anim.delay_num = delay_num, anim.delay_den = delay_den;
+    return sweep_multi_impl(scenes, ngpu, cameras, n_frames, width, height, spp, OutKind::APNG, cb, user, stats, anim);
 }
 
 uint64_t rt_atomic_fetch_add_u64(void *addr, uint64_t value) {
@@ -1441,13 +1466,29 @@ int rt_png_bound(uint32_t width, uint32_t height, size_t *bytes) {
     return RT_OK;
 }
 
-int rt_encode_png(const uint8_t *rgba, uint32_t width, uint32_t height, size_t pitch_bytes, uint8_t *png_out, size_t cap,
-                  size_t *len_out, void *stream_) {
-    if (!rgba || !len_out || (!png_out && cap)) return fail(RT_ERR_INVALID, "NULL argument");
+int rt_apng_bound(uint32_t width, uint32_t height, uint32_t n_frames, size_t *frame_bytes) {
+    if (!frame_bytes) return fail(RT_ERR_INVALID, "NULL argument");
+    size_t png = 0;
+    const int rc = rt_png_bound(width, height, &png);
+    if (rc != RT_OK) return rc;
+    if (n_frames == 0) return fail(RT_ERR_INVALID, "an animation needs at least one frame");
+    // the last chunk's sequence number, (n - 1)(C + 1) with C = bands + 2 chunks of zlib data per frame
+    const uint64_t last_seq = (uint64_t)(n_frames - 1) * ((height + 15u) / 16u + 3u);
+    if (last_seq > 0x7fffffffu)
+        return fail(RT_ERR_INVALID, "%u frames of height %u need sequence numbers beyond 2^31 - 1", n_frames, height);
+    *frame_bytes = rt_apng_bound_bytes(width, height);
+    return RT_OK;
+}
+
+// rt_encode_png (anim == nullptr) and rt_encode_apng_frame (frame `frame` of *anim)
+static int encode_impl(const uint8_t *rgba, uint32_t width, uint32_t height, size_t pitch_bytes, uint8_t *file_out,
+                       size_t cap, size_t *len_out, void *stream_, const Animation *anim, uint32_t frame) {
+    if (!rgba || !len_out || (!file_out && cap)) return fail(RT_ERR_INVALID, "NULL argument");
     *len_out = 0;
     size_t bound = 0;
-    int rc = rt_png_bound(width, height, &bound);
+    int rc = anim ? rt_apng_bound(width, height, anim->n_frames, &bound) : rt_png_bound(width, height, &bound);
     if (rc != RT_OK) return rc;
+    if (anim && frame >= anim->n_frames) return fail(RT_ERR_INVALID, "frame %u of an animation of %u frames", frame, anim->n_frames);
     const size_t row_bytes = (size_t)width * 4;
     if (pitch_bytes == 0) pitch_bytes = row_bytes;
     if (pitch_bytes < row_bytes) return fail(RT_ERR_INVALID, "pitch %zu is smaller than a row (%zu bytes)", pitch_bytes, row_bytes);
@@ -1473,15 +1514,33 @@ int rt_encode_png(const uint8_t *rgba, uint32_t width, uint32_t height, size_t p
     if (rc == RT_OK) rc = ensure(&sc->out, &sc->out_cap, len_at + sizeof(unsigned long long));
     if (rc != RT_OK) return rc;
     unsigned long long *len_word = reinterpret_cast<unsigned long long *>(sc->out + len_at), len = 0;
-    CUDA_TRY(rt_launch_png_encode(rgba, pitch_bytes, width, height, sc->scratch, sc->out, len_word, stream));
+    if (anim)
+        CUDA_TRY(rt_launch_apng_encode(rgba, pitch_bytes, width, height, frame, anim->n_frames, anim->delay_num,
+                                       anim->delay_den, sc->scratch, sc->out, len_word, stream));
+    else
+        CUDA_TRY(rt_launch_png_encode(rgba, pitch_bytes, width, height, sc->scratch, sc->out, len_word, stream));
     CUDA_TRY(cudaMemcpyAsync(&len, len_word, sizeof(len), cudaMemcpyDeviceToHost, stream));
     CUDA_TRY(cudaStreamSynchronize(stream));
     if (len == 0 || len > bound) return fail(RT_ERR_CUDA, "PNG encoder returned %llu bytes (bound %zu)", len, bound);
     *len_out = (size_t)len;
-    if (len > cap) return fail(RT_ERR_BUFFER, "png_out holds %zu bytes, the file needs %llu", cap, len);
-    CUDA_TRY(cudaMemcpyAsync(png_out, sc->out, (size_t)len, cudaMemcpyDefault, stream));
+    if (len > cap) return fail(RT_ERR_BUFFER, "%s holds %zu bytes, the %s needs %llu", anim ? "out" : "png_out", cap,
+                               anim ? "frame" : "file", len);
+    CUDA_TRY(cudaMemcpyAsync(file_out, sc->out, (size_t)len, cudaMemcpyDefault, stream));
     CUDA_TRY(cudaStreamSynchronize(stream));
     return RT_OK;
+}
+
+int rt_encode_png(const uint8_t *rgba, uint32_t width, uint32_t height, size_t pitch_bytes, uint8_t *png_out, size_t cap,
+                  size_t *len_out, void *stream) {
+    return encode_impl(rgba, width, height, pitch_bytes, png_out, cap, len_out, stream, nullptr, 0);
+}
+
+int rt_encode_apng_frame(const uint8_t *rgba, uint32_t width, uint32_t height, size_t pitch_bytes, uint32_t frame,
+                         uint32_t n_frames, uint16_t delay_num, uint16_t delay_den, uint8_t *out, size_t cap,
+                         size_t *len_out, void *stream) {
+    Animation anim;
+    anim.n_frames = n_frames, anim.delay_num = delay_num, anim.delay_den = delay_den;
+    return encode_impl(rgba, width, height, pitch_bytes, out, cap, len_out, stream, &anim, frame);
 }
 
 int rt_host_register(void *p, size_t bytes) {

@@ -15,6 +15,8 @@
 // bits packed in shared memory and flushed to a global staging slot per row, the piece's CRC-32 and Adler-32
 // partials), then png_assemble (one CTA per band: the chunk's place from a scan of the band sizes, the copy of its
 // pieces into the file; CTA 0 writes the header, one more CTA the last IDAT, IEND and the file length).
+// apng_assemble (rt_encode_apng_frame, rt_render_sweep_apng) takes png_assemble's place for one frame of an animated
+// PNG: the same zlib stream, framed as that frame's piece of the animation (DESIGN.md "Animated PNG").
 #include "rt_png.h"
 
 namespace {
@@ -25,6 +27,7 @@ constexpr uint32_t ADLER_MOD = 65521u;
 constexpr uint32_t FULL = 0xffffffffu;
 constexpr uint32_t HEADER_BYTES = 8 + 25 + 14;  // signature, IHDR, IDAT(78 01)
 constexpr uint32_t TRAILER_BYTES = 18 + 12;     // IDAT(03 00 + Adler-32), IEND
+constexpr uint32_t ACTL_BYTES = 12 + 8, FCTL_BYTES = 12 + 26;
 
 __constant__ uint16_t c_len_base[29] = {3,  4,  5,  6,  7,  8,  9,  10, 11,  13,  15,  17,  19,  23, 27,
                                         31, 35, 43, 51, 59, 67, 83, 99, 115, 131, 163, 195, 227, 258};
@@ -304,6 +307,79 @@ __global__ void __launch_bounds__(WARPS * 32) png_encode_rows(const uint8_t *__r
     }
 }
 
+// ---- apng_assemble's steps.  They are png_assemble's with the chunk framing as a parameter; png_assemble keeps its
+// own copy so that the PNG path runs exactly the machine code measured in DESIGN.md "PNG output". ---------------
+// The offset of CTA b's chunk (`head` bytes, then every earlier band's chunk of `framing` +
+// data bytes), and in s_rowoff the offsets of its rows' pieces within the chunk's data.
+__device__ __forceinline__ unsigned long long chunk_offset(const Scratch &sc, uint32_t height, uint32_t b,
+                                                           uint32_t framing, uint32_t head, unsigned long long *s_red,
+                                                           uint32_t *s_rowoff) {
+    const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31u;
+    const uint32_t bands = (height + BAND - 1) / BAND;
+    unsigned long long acc = 0;
+    for (uint32_t i = threadIdx.x; i < b; i += blockDim.x) acc += framing + sc.bands[i].x;
+    for (uint32_t d = 16; d; d >>= 1) acc += __shfl_xor_sync(FULL, acc, d);
+    if (lane == 0) s_red[warp] = acc;
+    if (threadIdx.x == 0) {
+        const uint32_t rows = b < bands ? min(BAND, height - b * BAND) : 0u;
+        s_rowoff[0] = 0;
+        for (uint32_t w = 0; w < rows; w++) s_rowoff[w + 1] = s_rowoff[w] + piece_bytes(sc.rows[b * BAND + w].x);
+    }
+    __syncthreads();
+    unsigned long long off = head;
+    for (uint32_t w = 0; w < WARPS; w++) off += s_red[w];
+    return off;
+}
+
+// Band b's pieces, one row per warp, to `dst` (the chunk's data).
+__device__ __forceinline__ void copy_pieces(const Scratch &sc, uint32_t height, uint32_t b, uint8_t *dst,
+                                            const uint32_t *s_rowoff) {
+    const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31u;
+    const uint32_t r = b * BAND + warp;
+    if (r < height) {
+        const uint32_t bits = sc.rows[r].x, len = piece_bytes(bits);
+        const uint8_t *staged = reinterpret_cast<const uint8_t *>(sc.stage + (size_t)r * sc.slot_words);
+        uint8_t *d = dst + s_rowoff[warp];
+        for (uint32_t q = lane; q < len; q += 32u) d[q] = (uint8_t)piece_byte(staged, bits, len, q);
+    }
+}
+
+// The PNG signature and IHDR at `out` (33 bytes).
+__device__ __forceinline__ void write_signature_ihdr(uint8_t *out, uint32_t width, uint32_t height, const uint32_t *table) {
+    const uint8_t sig[8] = {0x89, 'P', 'N', 'G', '\r', '\n', 0x1a, '\n'};
+    for (int k = 0; k < 8; k++) out[k] = sig[k];
+    uint8_t *ihdr = out + 8;
+    put_be32(ihdr + 8, width);
+    put_be32(ihdr + 12, height);
+    ihdr[16] = 8, ihdr[17] = 2, ihdr[18] = 0, ihdr[19] = 0, ihdr[20] = 0;
+    write_chunk(ihdr, "IHDR", 13, table);
+}
+
+// The zlib stream's Adler-32 (returned to thread 0) from the per-row partials.  Row r of n
+// bytes starts at byte r*n of N = n*h, so b gains W_r + n*(h-1-r)*S_r, where S_r = sum of its bytes and
+// W_r = sum of (n - k) * byte k.
+__device__ __forceinline__ uint32_t adler_of_rows(const Scratch &sc, uint32_t width, uint32_t height,
+                                                  unsigned long long *s_red, unsigned long long *s_red2) {
+    const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31u;
+    const uint32_t n = 1u + 3u * width, nm = n % ADLER_MOD;
+    unsigned long long sa = 0, sb = 0;
+    for (uint32_t r = threadIdx.x; r < height; r += blockDim.x) {
+        const uint4 ri = sc.rows[r];
+        const unsigned long long wgt = (unsigned long long)nm * ((height - 1u - r) % ADLER_MOD) % ADLER_MOD;
+        sa += ri.z;
+        sb += (ri.w + wgt * ri.z) % ADLER_MOD;
+    }
+    for (uint32_t d = 16; d; d >>= 1) sa += __shfl_xor_sync(FULL, sa, d), sb += __shfl_xor_sync(FULL, sb, d);
+    __syncthreads();  // s_red is reused
+    if (lane == 0) s_red[warp] = sa, s_red2[warp] = sb;
+    __syncthreads();
+    if (threadIdx.x != 0) return 0;
+    unsigned long long a = 1, bb = (unsigned long long)n * height % ADLER_MOD;
+    for (uint32_t w = 0; w < WARPS; w++) a += s_red[w], bb += s_red2[w];
+    a %= ADLER_MOD, bb %= ADLER_MOD;
+    return (uint32_t)((bb << 16) | a);
+}
+
 // CTA b < bands: band b's chunk; CTA `bands`: the last IDAT, IEND and the file length.
 __global__ void __launch_bounds__(WARPS * 32) png_assemble(uint32_t width, uint32_t height, Scratch sc,
                                                              uint8_t *__restrict__ out, unsigned long long *len_word) {
@@ -382,12 +458,111 @@ __global__ void __launch_bounds__(WARPS * 32) png_assemble(uint32_t width, uint3
     }
 }
 
+// Frame `frame` of an n_frames animation (delay = delay_num << 16 | delay_den), same grid as png_assemble.  The
+// payload is frame 0: signature, IHDR, acTL, fcTL 0, then the frame's IDAT chunks exactly as png_assemble writes them;
+// frame f >= 1: fcTL s_f, then the same C = bands + 2 chunks as fdAT, chunk k carrying sequence number s_f + 1 + k
+// before its data, where s_f = 1 + (f - 1)(C + 1).  The last frame also ends with IEND.  The animation is the payloads
+// in frame order, so no frame depends on another.
+__global__ void __launch_bounds__(WARPS * 32) apng_assemble(uint32_t width, uint32_t height, Scratch sc,
+                                                              uint32_t frame, uint32_t n_frames, uint32_t delay,
+                                                              uint8_t *__restrict__ out, unsigned long long *len_word) {
+    __shared__ uint32_t s_table[256], s_x2n[32];
+    __shared__ unsigned long long s_red[WARPS], s_red2[WARPS];
+    __shared__ uint32_t s_rowoff[BAND + 1];
+    const uint32_t b = blockIdx.x;
+    const uint32_t bands = (height + BAND - 1) / BAND;
+    const bool first = frame == 0;
+    const uint32_t seq_bytes = first ? 0u : 4u;  // an fdAT's sequence number, before the data
+    const uint32_t fctl_seq = first ? 0u : 1u + (frame - 1u) * (bands + 3u);
+    init_crc_tables(s_table, s_x2n);
+    const uint32_t head = (first ? 8u + 25u + ACTL_BYTES : 0u) + FCTL_BYTES + 14u + seq_bytes;
+    const unsigned long long off = chunk_offset(sc, height, b, 12u + seq_bytes, head, s_red, s_rowoff);
+
+    if (b < bands) {
+        copy_pieces(sc, height, b, out + off + 8 + seq_bytes, s_rowoff);
+        if (threadIdx.x == 0) {
+            const uint2 band = sc.bands[b];
+            uint8_t *c = out + off;
+            put_be32(c, band.x + seq_bytes);
+            if (first) {
+                c[4] = 'I', c[5] = 'D', c[6] = 'A', c[7] = 'T';
+                put_be32(c + 8 + band.x, band.y);
+            } else {
+                // crc("fdAT" seq data) = crc("IDAT" data) ^ x^(8 |data|) (crc("IDAT") ^ crc("fdAT" seq)): the band's
+                // CRC is reused instead of reading the data again
+                c[4] = 'f', c[5] = 'd', c[6] = 'A', c[7] = 'T';
+                put_be32(c + 8, fctl_seq + 2u + b);
+                const uint8_t idat[4] = {'I', 'D', 'A', 'T'};
+                const uint32_t diff = ~crc_bytes(0xffffffffu, idat, 4, s_table) ^ ~crc_bytes(0xffffffffu, c + 4, 8, s_table);
+                put_be32(c + 12 + band.x, band.y ^ crc_combine(diff, 0u, band.x, s_x2n));
+            }
+        }
+        if (b == 0 && threadIdx.x == 0) {
+            uint8_t *p = out;
+            if (first) {
+                write_signature_ihdr(p, width, height, s_table);
+                put_be32(p + 33 + 8, n_frames);
+                put_be32(p + 33 + 12, 0u);  // num_plays 0: loop for ever
+                write_chunk(p + 33, "acTL", 8, s_table);
+                p += 33 + ACTL_BYTES;
+            }
+            put_be32(p + 8, fctl_seq);
+            put_be32(p + 12, width);
+            put_be32(p + 16, height);
+            put_be32(p + 20, 0u);  // x and y offsets: every frame is full size
+            put_be32(p + 24, 0u);
+            put_be32(p + 28, delay);
+            p[32] = 0, p[33] = 0;  // dispose_op NONE, blend_op SOURCE
+            write_chunk(p, "fcTL", 26, s_table);
+            p += FCTL_BYTES;
+            if (first) {
+                p[8] = 0x78, p[9] = 0x01;
+                write_chunk(p, "IDAT", 2, s_table);
+            } else {
+                put_be32(p + 8, fctl_seq + 1u);
+                p[12] = 0x78, p[13] = 0x01;
+                write_chunk(p, "fdAT", 6, s_table);
+            }
+        }
+        return;
+    }
+    const uint32_t adler = adler_of_rows(sc, width, height, s_red, s_red2);
+    if (threadIdx.x == 0) {
+        uint8_t *last = out + off, *d = last + 8 + seq_bytes;
+        if (!first) put_be32(last + 8, fctl_seq + bands + 2u);
+        d[0] = 0x03, d[1] = 0x00;
+        put_be32(d + 2, adler);
+        write_chunk(last, first ? "IDAT" : "fdAT", 6 + seq_bytes, s_table);
+        unsigned long long end = off + 18 + seq_bytes;
+        if (frame + 1u == n_frames) write_chunk(out + end, "IEND", 0, s_table), end += 12;
+        *len_word = end;
+    }
+}
+
+// The scratch block's pieces (rt_png_scratch_bytes) for a frame of layout `l`.
+Scratch scratch_at(const Layout &l, void *scratch) {
+    uint8_t *p = static_cast<uint8_t *>(scratch);
+    Scratch sc;
+    sc.stage = reinterpret_cast<uint32_t *>(p);
+    sc.masks = reinterpret_cast<uint32_t *>(p + l.stage_bytes);
+    sc.rows = reinterpret_cast<uint4 *>(p + l.stage_bytes + l.mask_bytes);
+    sc.bands = reinterpret_cast<uint2 *>(p + l.stage_bytes + l.mask_bytes + l.rows_bytes);
+    sc.slot_words = l.slot_words;
+    sc.mask_stride = l.mask_stride;
+    return sc;
+}
+
 }  // namespace
 
 size_t rt_png_bound_bytes(uint32_t width, uint32_t height) {
     const Layout l = layout_of(width, height);
     const size_t piece = (3 + 9ull * l.n + 10 + 7) / 8 + 4;
     return HEADER_BYTES + 12ull * l.bands + (size_t)height * piece + TRAILER_BYTES;
+}
+
+size_t rt_apng_bound_bytes(uint32_t width, uint32_t height) {
+    const Layout l = layout_of(width, height);
+    return rt_png_bound_bytes(width, height) + ACTL_BYTES + FCTL_BYTES + 4ull * (l.bands + 2);
 }
 
 size_t rt_png_scratch_bytes(uint32_t width, uint32_t height) {
@@ -399,15 +574,20 @@ cudaError_t rt_launch_png_encode(const uint8_t *rgba, size_t pitch, uint32_t wid
                                  uint8_t *out, unsigned long long *len_word, cudaStream_t stream) {
     if (width == 0 || height == 0) return cudaErrorInvalidValue;
     const Layout l = layout_of(width, height);
-    uint8_t *p = static_cast<uint8_t *>(scratch);
-    Scratch sc;
-    sc.stage = reinterpret_cast<uint32_t *>(p);
-    sc.masks = reinterpret_cast<uint32_t *>(p + l.stage_bytes);
-    sc.rows = reinterpret_cast<uint4 *>(p + l.stage_bytes + l.mask_bytes);
-    sc.bands = reinterpret_cast<uint2 *>(p + l.stage_bytes + l.mask_bytes + l.rows_bytes);
-    sc.slot_words = l.slot_words;
-    sc.mask_stride = l.mask_stride;
+    const Scratch sc = scratch_at(l, scratch);
     png_encode_rows<<<l.bands, WARPS * 32, 0, stream>>>(rgba, pitch, width, height, sc);
     png_assemble<<<l.bands + 1, WARPS * 32, 0, stream>>>(width, height, sc, out, len_word);
+    return cudaGetLastError();
+}
+
+cudaError_t rt_launch_apng_encode(const uint8_t *rgba, size_t pitch, uint32_t width, uint32_t height, uint32_t frame,
+                                  uint32_t n_frames, uint16_t delay_num, uint16_t delay_den, void *scratch, uint8_t *out,
+                                  unsigned long long *len_word, cudaStream_t stream) {
+    if (width == 0 || height == 0 || frame >= n_frames) return cudaErrorInvalidValue;
+    const Layout l = layout_of(width, height);
+    const Scratch sc = scratch_at(l, scratch);
+    png_encode_rows<<<l.bands, WARPS * 32, 0, stream>>>(rgba, pitch, width, height, sc);
+    apng_assemble<<<l.bands + 1, WARPS * 32, 0, stream>>>(width, height, sc, frame, n_frames,
+                                                          (uint32_t)delay_num << 16 | delay_den, out, len_word);
     return cudaGetLastError();
 }

@@ -12,8 +12,9 @@
 // Additive flags: --level=L (scene depth, default 8 as at render.rs:147),
 // --gpus=N / RTRACE_GPUS (default 1: one frame = interleaved row blocks over the GPUs; a sweep = the GPUs draw
 // frames from one queue), --frames=K (orbit sweep; frame f goes to <stem>.f.tga, frame 0 is the reference camera), --stats (summary on stderr), --buckets (the reference's 64x64 bucket
-// schedule through Renderer::render_region instead of one launch per frame), --format=tga|png (a real TGA, or a PNG
-// encoded on the GPU: the output is then named *.png and sweep frames <stem>.f.png).
+// schedule through Renderer::render_region instead of one launch per frame), --format=tga|png|apng (a real TGA, a PNG
+// encoded on the GPU: the output is then named *.png and sweep frames <stem>.f.png, or all frames in ONE animated PNG
+// named *.png), --fps=F (frame rate of --format apng).
 #include <cerrno>
 #include <chrono>
 #include <cmath>
@@ -56,13 +57,15 @@ const char *USAGE =
     "        --frames <K>                       Render a K-frame orbit of the camera [default: 1]\n"
     "        --format <ppm|tga|png>             File contents: the reference's binary PPM, a real TGA, or a PNG encoded\n"
     "                                           on the GPU (the output is then named *.png) [default: ppm]\n"
+    "        --format apng                      All frames in one animated PNG encoded on the GPU (named *.png)\n"
+    "        --fps <F>                          Frames per second of --format apng, 1..65535 [default: 24]\n"
     "        --preview <N>                      Undersampled preview: trace one pixel per NxN block (1 sample) [default: off]\n"
     "        --stats                            Print a timing summary to stderr\n"
     "        --buckets                          Render 64x64 buckets one by one in the reference's order (sizes must\n"
     "                                           be multiples of 64, as in the reference); default is whole frames\n"
     "\n"
     "ARGS:\n"
-    "    <output>    Either a file with .tga extension (.png with --format png), or - to write file to stdout\n";
+    "    <output>    Either a file with .tga extension (.png with --format png or apng), or - to write file to stdout\n";
 
 [[noreturn]] void usage_error(const std::string &msg) {
     // clap 2: message + usage hint on stderr, exit status 1
@@ -96,7 +99,7 @@ unsigned long long parse_or_panic(const std::string &s, unsigned long long max, 
 }
 
 struct Args {
-    std::string width, height, ssp, numcores, output, level, gpus, frames, format, preview;
+    std::string width, height, ssp, numcores, output, level, gpus, frames, format, preview, fps;
     bool has_output = false, stats = false, buckets = false;
 };
 
@@ -109,7 +112,7 @@ Args parse_args(int argc, char **argv) {
     const Opt opts[] = {{"--width", &Args::width},   {"--height", &Args::height}, {"--samples-per-pixel", &Args::ssp},
                         {"--num-cores", &Args::numcores}, {"--level", &Args::level},   {"--gpus", &Args::gpus},
                         {"--frames", &Args::frames}, {"--format", &Args::format},
-                        {"--preview", &Args::preview}};
+                        {"--preview", &Args::preview}, {"--fps", &Args::fps}};
     bool only_positional = false;
     for (int i = 1; i < argc; i++) {
         std::string arg = argv[i];
@@ -221,8 +224,13 @@ int main(int argc, char **argv) {
     const std::string &output_file = args.output;
     FileOrAnyWriter output;
     FILE *fp = nullptr;
-    const bool png = args.format == "png";
-    const std::string ext = png ? "png" : "tga";
+    const bool png = args.format == "png", apng = args.format == "apng";
+    const std::string ext = png || apng ? "png" : "tga";
+    // before the output's name is checked: a misused --fps is a usage error whatever the name
+    if (!args.fps.empty() && !apng) usage_error("The argument '--fps' can only be used with '--format apng'");
+    unsigned long long fps = 24;
+    if (!args.fps.empty() && (!parse_unsigned(args.fps, 65535, &fps) || fps == 0))
+        usage_error("Invalid value for '--fps <F>': '" + args.fps + "' is not a whole number in 1..65535");
     if (output_file != "-") {
         if (extension_of(output_file) != ext) {
             printf("Output file '%s' must have the %s extension, e.g. %s\n", output_file.c_str(), ext.c_str(), with_extension(output_file, ext).c_str());
@@ -241,10 +249,10 @@ int main(int argc, char **argv) {
     unsigned frames = (unsigned)parse_or_panic(args.frames.empty() ? "1" : args.frames, 100000, "frames");
     if (gpus < 1) gpus = 1;
     if (frames < 1) frames = 1;
-    if (!args.format.empty() && args.format != "ppm" && args.format != "tga" && !png)
-        usage_error("'" + args.format + "' isn't a valid value for '--format <ppm|tga|png>'");
+    if (!args.format.empty() && args.format != "ppm" && args.format != "tga" && !png && !apng)
+        usage_error("'" + args.format + "' isn't a valid value for '--format <ppm|tga|png|apng>'");
     // the bucket schedule exists to drive the host writer seam; a PNG is encoded on the GPU from a whole frame
-    if (png && args.buckets) usage_error("The argument '--buckets' cannot be used with '--format png'");
+    if ((png || apng) && args.buckets) usage_error("The argument '--buckets' cannot be used with '--format " + args.format + "'");
     const bool real_tga = args.format == "tga";
     const unsigned preview = args.preview.empty() ? 0u : (unsigned)parse_or_panic(args.preview, 1024, "preview");
     if (options.width == 0 || options.height == 0) {
@@ -259,7 +267,7 @@ int main(int argc, char **argv) {
         auto t1 = clk::now();
         double render_ms = 0.0, kernel_ms = 0.0;
         auto frame_path = [&](unsigned f) {
-            if (frames == 1 || output_file == "-") return output_file;
+            if (frames == 1 || output_file == "-" || apng) return output_file;
             char suffix[32];
             snprintf(suffix, sizeof(suffix), "%04u.%s", f, ext.c_str());
             return with_extension(output_file, suffix);
@@ -277,7 +285,14 @@ int main(int argc, char **argv) {
             for (unsigned f = 0; f < frames; f++) cams.push_back(orbit_camera(f, frames));
             rt_stats st;
             auto r0 = clk::now();
-            if (png) {  // frames arrive as complete PNG files
+            if (apng) {  // frames arrive as the animation's payloads, in order: one file
+                output = open_output(0);
+                Renderer::render_sweep_apng(options, scene, cams, 1, (uint16_t)fps, [&](uint32_t, const uint8_t *data, size_t len) {
+                    if (fwrite(data, 1, len, output.f) != len) throw Panic("write_all failed");
+                }, &st);
+                fflush(output.f);
+                if (fp) fclose(fp), fp = nullptr;
+            } else if (png) {  // frames arrive as complete PNG files
                 Renderer::render_sweep_png(options, scene, cams, [&](uint32_t f, const uint8_t *file, size_t len) {
                     output = open_output(f);
                     if (fwrite(file, 1, len, output.f) != len) throw Panic("write_all failed");
@@ -302,12 +317,13 @@ int main(int argc, char **argv) {
             kernel_ms = 0.0;
         } else {
             for (unsigned f = 0; f < frames; f++) {
-                output = open_output(f);
+                if (!apng || f == 0) output = open_output(f);  // an animation is one file
                 rt_camera cam = orbit_camera(f, frames);
                 rt_stats st;
-                if (png) {
+                if (png || apng) {
+                    const Renderer::ApngFrame af{f, frames, 1, (uint16_t)fps};
                     auto r0 = clk::now();
-                    Renderer::render_png(options, scene, output.f, frames > 1 ? &cam : nullptr, preview, &st);
+                    Renderer::render_png(options, scene, output.f, frames > 1 ? &cam : nullptr, preview, &st, apng ? &af : nullptr);
                     render_ms += std::chrono::duration<double, std::milli>(clk::now() - r0).count();
                     kernel_ms += preview ? 0.0 : st.kernel_ms;
                 } else {
@@ -322,7 +338,7 @@ int main(int argc, char **argv) {
                     render_ms += std::chrono::duration<double, std::milli>(clk::now() - r0).count();
                     kernel_ms += st.kernel_ms;
                 }  // final write on drop (render.rs:331-335)
-                if (fp) fclose(fp), fp = nullptr;
+                if (fp && (!apng || f + 1 == frames)) fclose(fp), fp = nullptr;
             }
         }
         if (args.stats) {

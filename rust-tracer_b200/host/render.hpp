@@ -370,11 +370,28 @@ struct Renderer {
         });
     }
 
+    // The same sweep as one animated PNG whose frames each show for delay_num / delay_den seconds (extension):
+    // `sink(f, payload, len)` in frame order, and the payloads written one after the other are the file.
+    template <class Sink>
+    static void render_sweep_apng(const RenderOptions &o, const Scene &scene, const std::vector<rt_camera> &cameras,
+                                  uint16_t delay_num, uint16_t delay_den, Sink &&sink, rt_stats *stats = nullptr) {
+        sweep_through(sink, "Renderer::render_sweep_apng", [&](rt_frame_callback cb, void *user) {
+            return rt_render_sweep_apng(scene.replicas(), scene.gpus(), cameras.data(), (uint32_t)cameras.size(), o.width,
+                                        o.height, o.samples_per_pixel, delay_num, delay_den, cb, user, stats);
+        });
+    }
+
+    // Which frame of an animated PNG render_png writes, and the animation's frame count and frame delay.
+    struct ApngFrame {
+        uint32_t frame, n_frames;
+        uint16_t delay_num, delay_den;
+    };
+
     // One frame (or an undersampled preview when preview_step > 0) as a PNG file on `f` (extension): rendered into
     // device memory of the first GPU (with several GPUs their kernels store their rows there) and encoded there,
-    // so only the file crosses the host link.
+    // so only the file crosses the host link.  With `apng` the frame's payload of that animation is written instead.
     static void render_png(const RenderOptions &o, const Scene &scene, FILE *f, const rt_camera *camera = nullptr,
-                           uint32_t preview_step = 0, rt_stats *stats = nullptr) {
+                           uint32_t preview_step = 0, rt_stats *stats = nullptr, const ApngFrame *apng = nullptr) {
         struct Buffers {
             void *frame = nullptr, *file = nullptr;
             ~Buffers() {
@@ -384,7 +401,8 @@ struct Renderer {
         } b;
         const size_t frame_bytes = (size_t)o.width * o.height * 4;
         size_t bound = 0, len = 0;
-        rt_check(rt_png_bound(o.width, o.height, &bound), "Renderer::render_png");
+        rt_check(apng ? rt_apng_bound(o.width, o.height, apng->n_frames, &bound) : rt_png_bound(o.width, o.height, &bound),
+                 "Renderer::render_png");
         rt_check(rt_device_alloc(frame_bytes, &b.frame), "Renderer::render_png");
         rt_check(rt_host_alloc(bound, &b.file), "Renderer::render_png");
         uint8_t *frame = static_cast<uint8_t *>(b.frame);
@@ -395,7 +413,10 @@ struct Renderer {
             rt_check(rt_render_frame_multi(scene.replicas(), scene.gpus(), camera, o.width, o.height, o.samples_per_pixel,
                                            frame, frame_bytes, stats),
                      "Renderer::render");
-        rt_check(rt_encode_png(frame, o.width, o.height, 0, static_cast<uint8_t *>(b.file), bound, &len, nullptr),
+        uint8_t *file = static_cast<uint8_t *>(b.file);
+        rt_check(apng ? rt_encode_apng_frame(frame, o.width, o.height, 0, apng->frame, apng->n_frames, apng->delay_num,
+                                             apng->delay_den, file, bound, &len, nullptr)
+                      : rt_encode_png(frame, o.width, o.height, 0, file, bound, &len, nullptr),
                  "Renderer::render_png");
         if (fwrite(b.file, 1, len, f) != len) throw Panic("write_all failed");
         fflush(f);

@@ -26,6 +26,7 @@ ABI_SYMBOLS = [
     "rt_render_frame_multi", "rt_render_sweep_multi", "rt_render_sweep_pull", "rt_atomic_fetch_add_u64",
     "rt_count_rays", "rt_trace_rays", "rt_measure_fp32_peak", "rt_microbench_fp32", "rt_selftest_math", "rt_debug_phased_tiles", "rt_host_alloc", "rt_host_free", "rt_host_register", "rt_host_unregister", "rt_microbench_d2h", "rt_device_alloc", "rt_device_free", "rt_ipc_export", "rt_ipc_open", "rt_ipc_close", "rt_memcpy", "rt_memcpy2d_async", "rt_pack_rgb_rows",
     "rt_png_bound", "rt_encode_png", "rt_render_sweep_png",
+    "rt_apng_bound", "rt_encode_apng_frame", "rt_render_sweep_apng",
 ]
 
 
@@ -128,6 +129,11 @@ def lib():
     L.rt_encode_png.argtypes = [vp, u32, u32, C.c_size_t, vp, C.c_size_t, C.POINTER(C.c_size_t), vp]
     L.rt_render_sweep_png.argtypes = [C.POINTER(vp), C.c_int, C.POINTER(Camera), u32, u32, u32, u32, FRAME_CALLBACK, vp,
                                       C.POINTER(Stats)]
+    L.rt_apng_bound.argtypes = [u32, u32, u32, C.POINTER(C.c_size_t)]
+    L.rt_encode_apng_frame.argtypes = [vp, u32, u32, C.c_size_t, u32, u32, u16, u16, vp, C.c_size_t,
+                                       C.POINTER(C.c_size_t), vp]
+    L.rt_render_sweep_apng.argtypes = [C.POINTER(vp), C.c_int, C.POINTER(Camera), u32, u32, u32, u32, u16, u16,
+                                       FRAME_CALLBACK, vp, C.POINTER(Stats)]
     if os.environ.get("RTRACE_B200_LIB"):
         L = real
     _lib = L
@@ -436,6 +442,24 @@ class Renderer:
         return st
 
     @staticmethod
+    def render_sweep_apng(options, scenes, n_frames, cameras=None, fps=24, on_frame=None):
+        """The frame-sharded sweep (render_sweep_multi) as one animated PNG showing `fps` frames a second:
+        on_frame(f, bytes) receives frame f's payload in frame order on the calling thread, and the payloads joined
+        in that order are the file.  One scene is the single-GPU sweep."""
+        w, h, spp = options.width, options.height, options.samples_per_pixel
+        cams = (Camera * n_frames)(*cameras) if cameras is not None else None
+
+        def _cb(user, frame, ptr, nbytes):
+            if on_frame is not None:
+                on_frame(int(frame), C.string_at(ptr, nbytes))
+
+        cb = FRAME_CALLBACK(_cb)
+        st = Stats()
+        arr = (C.c_void_p * len(scenes))(*[s.handle for s in scenes])
+        _check(lib().rt_render_sweep_apng(arr, len(scenes), cams, n_frames, w, h, spp, 1, fps, cb, None, C.byref(st)))
+        return st
+
+    @staticmethod
     def render_multi(options, scenes, camera=None, want_stats=False):
         """Whole frame on len(scenes) GPUs of this process, rows interleaved, gathered on GPU 0."""
         w, h, spp = options.width, options.height, options.samples_per_pixel
@@ -544,6 +568,25 @@ def encode_png(device_ptr, width, height, pitch=0, stream=None):
     out = C.create_string_buffer(cap)
     n = C.c_size_t()
     _check(lib().rt_encode_png(C.c_void_p(device_ptr), width, height, pitch, out, cap, C.byref(n), stream))
+    return out.raw[:n.value]
+
+
+def apng_bound(width, height, n_frames):
+    """Worst-case size of one frame's payload of encode_apng_frame (pure arithmetic, no device needed)."""
+    n = C.c_size_t()
+    _check(lib().rt_apng_bound(width, height, n_frames, C.byref(n)))
+    return n.value
+
+
+def encode_apng_frame(device_ptr, width, height, frame, n_frames, fps=24, pitch=0, stream=None):
+    """Payload (bytes) of frame `frame` of an n_frames animated PNG showing `fps` frames a second, from a
+    width x height RGBA8 frame in device memory of the current device, encoded on the GPU (rt_encode_apng_frame);
+    the payloads of frames 0 .. n_frames-1 joined in order are the file.  Waits for `stream`."""
+    cap = apng_bound(width, height, n_frames)
+    out = C.create_string_buffer(cap)
+    n = C.c_size_t()
+    _check(lib().rt_encode_apng_frame(C.c_void_p(device_ptr), width, height, pitch, frame, n_frames, 1, fps, out, cap,
+                                      C.byref(n), stream))
     return out.raw[:n.value]
 
 

@@ -70,6 +70,13 @@ extern "C" {
     pub fn rt_render_sweep_png(scenes: *const *mut RtScene, ngpu: c_int, cameras: *const RtCamera, n_frames: u32,
                                width: u32, height: u32, spp: u32, cb: RtFrameCallback, user: *mut c_void,
                                stats: *mut RtStats) -> c_int;
+    pub fn rt_apng_bound(width: u32, height: u32, n_frames: u32, frame_bytes: *mut usize) -> c_int;
+    pub fn rt_encode_apng_frame(rgba: *const u8, width: u32, height: u32, pitch_bytes: usize, frame: u32,
+                                n_frames: u32, delay_num: u16, delay_den: u16, out: *mut u8, cap: usize,
+                                len_out: *mut usize, stream: *mut c_void) -> c_int;
+    pub fn rt_render_sweep_apng(scenes: *const *mut RtScene, ngpu: c_int, cameras: *const RtCamera, n_frames: u32,
+                                width: u32, height: u32, spp: u32, delay_num: u16, delay_den: u16,
+                                cb: RtFrameCallback, user: *mut c_void, stats: *mut RtStats) -> c_int;
 }
 
 pub fn last_error() -> String {
