@@ -26,58 +26,6 @@
 #include "rt_png.h"
 #include "rt_scene.h"
 
-// ---------------------------------------------------------------------------
-// rt_scene
-// ---------------------------------------------------------------------------
-struct rt_scene {
-    int device = 0;
-    rt::FlatScene flat;
-    uint32_t n = 0;
-    float4 *d_sph = nullptr;
-    uint32_t *d_skip = nullptr;
-    // scratch, guarded by mu (a scene may be used from several host threads)
-    std::mutex mu;
-    uint8_t *d_fb = nullptr;
-    size_t d_fb_cap = 0;
-    uint8_t *d_kinds = nullptr;
-    size_t d_kinds_cap = 0;
-    uint8_t *d_frame = nullptr;  // gathered frame (multi-GPU root)
-    size_t d_frame_cap = 0;
-    unsigned long long *d_ctr = nullptr;
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    cudaStream_t own_stream = nullptr;
-    // PHASED variant scratch, one set per stream (launches on different streams may overlap)
-    struct Phased {
-        uint32_t *winner = nullptr;
-        size_t winner_cap = 0;
-        uint4 *hdr = nullptr;
-        size_t hdr_cap = 0;
-        uint4 *pool = nullptr;
-        uint32_t pool_units = 0;
-        uint32_t *pool_count = nullptr;
-    };
-    // rt_render_sweep: ring of frame buffers (frames rendering at a time + one being copied out), the copy
-    // stream and the second render stream
-    static constexpr int SWEEP_RING = 3;
-    uint8_t *sweep_dev[SWEEP_RING] = {nullptr, nullptr, nullptr};
-    uint8_t *sweep_host[SWEEP_RING] = {nullptr, nullptr, nullptr};
-    uint8_t *sweep_rgb[SWEEP_RING] = {nullptr, nullptr, nullptr};
-    size_t sweep_bytes = 0;
-    int sweep_nb = 0;  // buffers of the ring that are allocated
-    cudaStream_t copy_stream = nullptr, render2 = nullptr;
-    cudaEvent_t sweep_rendered[SWEEP_RING] = {nullptr, nullptr, nullptr}, sweep_copied[SWEEP_RING] = {nullptr, nullptr, nullptr};
-    size_t sweep_host_bytes = 0;  // size of each sweep_host buffer
-    std::map<cudaStream_t, Phased> phased;
-    std::mutex mu_phased;  // guards the map only (mu may already be held by the caller)
-    // rt_render_sweep_png: the encoded file of each ring buffer (its length word after it), the lengths read back to
-    // the host, and the encoder's scratch, one per render stream
-    uint8_t *sweep_png[SWEEP_RING] = {nullptr, nullptr, nullptr};
-    size_t sweep_png_cap[SWEEP_RING] = {0, 0, 0};
-    unsigned long long *sweep_len_host = nullptr;
-    cudaEvent_t sweep_len_ready[SWEEP_RING] = {nullptr, nullptr, nullptr};
-    std::map<cudaStream_t, std::pair<uint8_t *, size_t>> png_scratch;
-};
-
 namespace {
 
 thread_local char g_err[512] = "";
@@ -91,9 +39,9 @@ struct RowLayout {
     bool out_abs = false;
 };
 
-// What a sweep hands to its frame callback: the RGBA8 frame, its RGB8 bytes (the P6 body), a PNG file, or the
-// frame's payload of an animated PNG.
-enum class OutKind { RGBA, RGB, PNG, APNG };
+// What a sweep hands to its frame callback: the RGBA8 frame, its RGB8 bytes (the P6 body), or a PNG file (with an
+// Animation: the frame's payload of an animated PNG).
+enum class OutKind { RGBA, RGB, PNG };
 
 // The animation an APNG frame belongs to: its frame count and how long each frame shows (delay_num / delay_den s).
 struct Animation {
@@ -114,6 +62,120 @@ int fail(int code, const char *fmt, ...) {
         cudaError_t e_ = (expr);                                                             \
         if (e_ != cudaSuccess) return fail(RT_ERR_CUDA, "%s: %s", #expr, cudaGetErrorString(e_)); \
     } while (0)
+
+#define RT_TRY(expr)                        \
+    do {                                    \
+        const int rc_ = (expr);             \
+        if (rc_ != RT_OK) return rc_;       \
+    } while (0)
+
+// Owners of the CUDA resources a scene (or an encoder's scratch) keeps between calls.  Each releases what it holds
+// when it goes, on the current device.
+struct NonCopyable {
+    NonCopyable() = default;
+    NonCopyable(const NonCopyable &) = delete;
+    NonCopyable &operator=(const NonCopyable &) = delete;
+};
+
+// A grow-only buffer of device memory (Pinned = false) or of pinned, portable host memory (Pinned = true).
+template <bool Pinned>
+struct Buffer : NonCopyable {
+    uint8_t *ptr = nullptr;
+    size_t cap = 0;
+    ~Buffer() { release(); }
+    template <class T>
+    T *as() const { return reinterpret_cast<T *>(ptr); }
+    // at least `need` bytes; the contents are not kept when the buffer grows
+    int ensure(size_t need) {
+        if (cap >= need) return RT_OK;
+        release();
+        cudaError_t e = Pinned ? cudaHostAlloc((void **)&ptr, need, cudaHostAllocPortable) : cudaMalloc((void **)&ptr, need);
+        if (e != cudaSuccess) {
+            ptr = nullptr;
+            return fail(e == cudaErrorMemoryAllocation ? RT_ERR_NOMEM : RT_ERR_CUDA, "%s(%zu): %s",
+                        Pinned ? "cudaHostAlloc" : "cudaMalloc", need, cudaGetErrorString(e));
+        }
+        cap = need;
+        return RT_OK;
+    }
+    void release() {
+        if (ptr) Pinned ? cudaFreeHost(ptr) : cudaFree(ptr);
+        ptr = nullptr;
+        cap = 0;
+    }
+};
+using DeviceBuffer = Buffer<false>;
+using HostBuffer = Buffer<true>;
+
+struct Event : NonCopyable {
+    cudaEvent_t ev = nullptr;
+    ~Event() {
+        if (ev) cudaEventDestroy(ev);
+    }
+    operator cudaEvent_t() const { return ev; }
+    int create(unsigned flags) {  // once; later calls keep the event
+        if (!ev) CUDA_TRY(cudaEventCreateWithFlags(&ev, flags));
+        return RT_OK;
+    }
+};
+
+// a stream that does not synchronise with the legacy default stream
+struct Stream : NonCopyable {
+    cudaStream_t st = nullptr;
+    ~Stream() {
+        if (st) cudaStreamDestroy(st);
+    }
+    operator cudaStream_t() const { return st; }
+    int create() {  // once; later calls keep the stream
+        if (!st) CUDA_TRY(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
+        return RT_OK;
+    }
+};
+
+// Scratch of the launches on one stream (launches on different streams may overlap): the PHASED variant's buffers
+// and the PNG encoder's.
+struct StreamScratch {
+    DeviceBuffer winner, hdr, pool, pool_count, png;
+    uint32_t pool_units = 0;  // pool entries the kernels may use: a forced RTRACE_POOL_UNITS may leave it below pool.cap
+};
+
+// One buffer of the sweep's ring: a frame from its render to its hand-over.
+struct SweepSlot {
+    DeviceBuffer frame;  // RGBA8
+    DeviceBuffer rgb;    // its RGB8 pack (RGB sweeps)
+    DeviceBuffer png;    // its PNG file, then the file's length word (PNG sweeps)
+    HostBuffer host;     // what the frame callback receives
+    HostBuffer len;      // the PNG length word read back
+    Event rendered, copied, len_ready;
+};
+
+}  // namespace
+
+// ---------------------------------------------------------------------------
+// rt_scene
+// ---------------------------------------------------------------------------
+struct rt_scene {
+    int device = 0;
+    rt::FlatScene flat;
+    uint32_t n = 0;
+    DeviceBuffer d_sph, d_skip;  // float4 / uint32_t per node
+    // scratch, guarded by mu (a scene may be used from several host threads)
+    std::mutex mu;
+    DeviceBuffer d_fb, d_kinds;
+    DeviceBuffer d_frame;  // gathered frame (multi-GPU root)
+    DeviceBuffer d_ctr;    // 16 ray counters
+    Event ev0, ev1;
+    Stream own_stream;
+    // rt_render_sweep: ring of frame buffers (frames rendering at a time + one being copied out), the copy
+    // stream and the second render stream
+    static constexpr int SWEEP_RING = 3;
+    SweepSlot sweep[SWEEP_RING];
+    Stream copy_stream, render2;
+    std::map<cudaStream_t, StreamScratch> scratch;
+    std::mutex mu_scratch;  // guards the map only (mu may already be held by the caller)
+};
+
+namespace {
 
 struct DeviceGuard {
     int prev = -1;
@@ -149,33 +211,32 @@ bool is_device_ptr(const void *ptr, int *dev) {
 int upload(rt_scene *s) {
     s->n = (uint32_t)s->flat.skip.size();
     CUDA_TRY(cudaGetDevice(&s->device));
-    CUDA_TRY(cudaMalloc(&s->d_sph, sizeof(float4) * s->n));
-    CUDA_TRY(cudaMalloc(&s->d_skip, sizeof(uint32_t) * s->n));
-    CUDA_TRY(cudaMemcpy(s->d_sph, s->flat.sph.data(), sizeof(float4) * s->n, cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMemcpy(s->d_skip, s->flat.skip.data(), sizeof(uint32_t) * s->n, cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMalloc(&s->d_ctr, sizeof(unsigned long long) * 16));
-    CUDA_TRY(cudaEventCreate(&s->ev0));
-    CUDA_TRY(cudaEventCreate(&s->ev1));
-    CUDA_TRY(cudaStreamCreateWithFlags(&s->own_stream, cudaStreamNonBlocking));
-    return RT_OK;
+    RT_TRY(s->d_sph.ensure(sizeof(float4) * s->n));
+    RT_TRY(s->d_skip.ensure(sizeof(uint32_t) * s->n));
+    CUDA_TRY(cudaMemcpy(s->d_sph.ptr, s->flat.sph.data(), sizeof(float4) * s->n, cudaMemcpyHostToDevice));
+    CUDA_TRY(cudaMemcpy(s->d_skip.ptr, s->flat.skip.data(), sizeof(uint32_t) * s->n, cudaMemcpyHostToDevice));
+    RT_TRY(s->d_ctr.ensure(sizeof(unsigned long long) * 16));
+    RT_TRY(s->ev0.create(cudaEventDefault));
+    RT_TRY(s->ev1.create(cudaEventDefault));
+    return s->own_stream.create();
 }
 
-int ensure(uint8_t **buf, size_t *cap, size_t need) {
-    if (*cap >= need) return RT_OK;
-    if (*buf) cudaFree(*buf);
-    *buf = nullptr;
-    *cap = 0;
-    cudaError_t e = cudaMalloc(buf, need);
-    if (e != cudaSuccess) return fail(e == cudaErrorMemoryAllocation ? RT_ERR_NOMEM : RT_ERR_CUDA, "cudaMalloc(%zu): %s", need, cudaGetErrorString(e));
-    *cap = need;
+// The end of both scene constructors: upload the nodes and hand the scene out, or destroy it.
+int finish_scene(rt_scene *s, rt_scene **out) {
+    const int rc = upload(s);
+    if (rc != RT_OK) {
+        rt_scene_destroy(s);
+        return rc;
+    }
+    *out = s;
     return RT_OK;
 }
 
 void fill_params(const rt_scene *s, const rt_camera *cam, uint32_t w, uint32_t h, uint32_t spp, uint32_t row_start,
                  uint32_t row_stride, uint32_t row_count, rt::RenderParams &p, RowLayout layout = RowLayout()) {
     memset(&p, 0, sizeof(p));
-    p.sph = s->d_sph;
-    p.skip = s->d_skip;
+    p.sph = s->d_sph.as<float4>();
+    p.skip = s->d_skip.as<uint32_t>();
     p.n_nodes = s->n;
     p.one = 1.0f;
     p.level = s->flat.level;
@@ -306,58 +367,52 @@ int kernel_variant(const rt::RenderParams &p) {
     return (pixel_tiles < 8000 && tile_ok) ? RT_KERNEL_TILE : RT_KERNEL_PHASED;
 }
 
-int tile_shape() {
-    static const char *force = getenv("RTRACE_TILE_SHAPE");  // kernel experiments
-    return (force && *force) ? atoi(force) : 0;
-}
-
-template <class T>
-int ensure_typed(T **buf, size_t *cap, size_t need_bytes) {
-    uint8_t *b = reinterpret_cast<uint8_t *>(*buf);
-    int rc = ensure(&b, cap, need_bytes);
-    *buf = reinterpret_cast<T *>(b);
-    return rc;
+// RTRACE_TILE_SHAPE (kernel experiments): the tile shape forced on the TILE and PHASED variants, -1 when unset
+int forced_tile_shape() {
+    static const char *force = getenv("RTRACE_TILE_SHAPE");
+    return (force && *force) ? atoi(force) : -1;
 }
 
 // Scratch of the PHASED variant for this stream (allocated on first use, grown on demand).
-int prepare_phased(rt_scene *s, rt::RenderParams &p, cudaStream_t stream) {
+int prepare_phased(rt_scene *s, rt::RenderParams &p, cudaStream_t stream, int shape) {
     size_t wb = 0, hb = 0;
     uint32_t units = 0;
-    rt_phased_scratch(p.width, p.row_count, p.spp, tile_shape(), &wb, &hb, &units);
+    rt_phased_scratch(p.width, p.row_count, p.spp, shape, &wb, &hb, &units);
     const char *cap = getenv("RTRACE_POOL_UNITS");  // tests: a tiny pool exercises the overflow fallback
     const bool forced_pool = cap && *cap;
     if (forced_pool) units = (uint32_t)strtoul(cap, nullptr, 10);
-    std::lock_guard<std::mutex> lock(s->mu_phased);
-    rt_scene::Phased &ph = s->phased[stream];
-    int rc = ensure_typed(&ph.winner, &ph.winner_cap, wb);
-    if (rc == RT_OK) rc = ensure_typed(&ph.hdr, &ph.hdr_cap, hb);
-    if (rc == RT_OK && ph.pool_units != units && (ph.pool_units < units || forced_pool)) {
-        size_t cap = (size_t)ph.pool_units * sizeof(uint4);
-        rc = ensure_typed(&ph.pool, &cap, (size_t)units * sizeof(uint4));
-        if (rc == RT_OK) ph.pool_units = units;
+    std::lock_guard<std::mutex> lock(s->mu_scratch);
+    StreamScratch &sc = s->scratch[stream];
+    RT_TRY(sc.winner.ensure(wb));
+    RT_TRY(sc.hdr.ensure(hb));
+    if (units > sc.pool_units || forced_pool) {  // the pool grows with the frame; only a forced size shrinks it
+        sc.pool_units = 0;                          // until the pool holds `units` (a failed ensure frees it)
+        RT_TRY(sc.pool.ensure((size_t)units * sizeof(uint4)));
+        sc.pool_units = units;
     }
-    if (rc == RT_OK && !ph.pool_count) CUDA_TRY(cudaMalloc(&ph.pool_count, sizeof(uint32_t)));
-    if (rc != RT_OK) return rc;
-    p.winner = ph.winner;
-    p.tile_hdr = ph.hdr;
-    p.pool = ph.pool;
-    p.pool_cap = ph.pool_units;
-    p.pool_count = ph.pool_count;
+    RT_TRY(sc.pool_count.ensure(sizeof(uint32_t)));
+    p.winner = sc.winner.as<uint32_t>();
+    p.tile_hdr = sc.hdr.as<uint4>();
+    p.pool = sc.pool.as<uint4>();
+    p.pool_cap = sc.pool_units;
+    p.pool_count = sc.pool_count.as<uint32_t>();
     return RT_OK;
 }
 
-int launch(rt_scene *s, rt::RenderParams &p, bool diag, cudaStream_t stream) {
-    const int v = kernel_variant(p);
+// Launches the kernel(s) of one frame on `stream`; *variant receives the kernel that renders it (RT_KERNEL_*,
+// numbered like RT_VARIANT_*).
+int launch(rt_scene *s, rt::RenderParams &p, bool diag, cudaStream_t stream, int *variant) {
+    const int v = kernel_variant(p), shape = forced_tile_shape();
+    *variant = v;
     cudaError_t e;
     if (v == RT_KERNEL_PHASED) {
-        int rc = prepare_phased(s, p, stream);
-        if (rc != RT_OK) return rc;
-        e = rt_launch_render_phased(diag, p, stream, tile_shape());
+        const int phased_shape = std::max(shape, 0);
+        RT_TRY(prepare_phased(s, p, stream, phased_shape));
+        e = rt_launch_render_phased(diag, p, stream, phased_shape);
     } else if (v == RT_KERNEL_TILE) {
         // AUTO picks the fused kernel only for small frames, where one independent warp per tile
         // (shape 2) beats CTA-shared culls (warps waiting at barriers with too few CTAs to cover them)
-        static const char *force = getenv("RTRACE_TILE_SHAPE");
-        e = rt_launch_render_tile(diag, p, stream, (force && *force) ? atoi(force) : (g_variant == RT_VARIANT_AUTO ? 2 : 0));
+        e = rt_launch_render_tile(diag, p, stream, shape >= 0 ? shape : (g_variant == RT_VARIANT_AUTO ? 2 : 0));
     } else {
         e = rt_launch_render(v, diag, p, stream);
     }
@@ -365,16 +420,53 @@ int launch(rt_scene *s, rt::RenderParams &p, bool diag, cudaStream_t stream) {
     return RT_OK;
 }
 
+uint32_t launches_of(int variant) { return variant == RT_KERNEL_PHASED ? 4 : 1; }
+
+// Queues on `stream` the PNG encode of the RGBA8 frame `rgba` (anim != nullptr: frame `frame`'s payload of that
+// animated PNG) into `out` -- the file, then its length word -- and the copy of the length word to *len_host.
+// `bound` is the bound of that file (rt_png_bound_bytes / rt_apng_bound_bytes).
+int queue_encode(const uint8_t *rgba, size_t pitch, uint32_t width, uint32_t height, const Animation *anim,
+                 uint32_t frame, size_t bound, DeviceBuffer &scratch, DeviceBuffer &out, unsigned long long *len_host,
+                 cudaStream_t stream) {
+    const size_t len_at = (bound + 7) / 8 * 8;
+    RT_TRY(scratch.ensure(rt_png_scratch_bytes(width, height)));
+    RT_TRY(out.ensure(len_at + sizeof(unsigned long long)));
+    unsigned long long *len_word = reinterpret_cast<unsigned long long *>(out.ptr + len_at);
+    if (anim)
+        CUDA_TRY(rt_launch_apng_encode(rgba, pitch, width, height, frame, anim->n_frames, anim->delay_num,
+                                       anim->delay_den, scratch.ptr, out.ptr, len_word, stream));
+    else
+        CUDA_TRY(rt_launch_png_encode(rgba, pitch, width, height, scratch.ptr, out.ptr, len_word, stream));
+    CUDA_TRY(cudaMemcpyAsync(len_host, len_word, sizeof(unsigned long long), cudaMemcpyDeviceToHost, stream));
+    return RT_OK;
+}
+
+// Peer access from device `from` (the current device) to the memory of device `to`: *can = false when there is none.
+int enable_peer(int from, int to, bool *can) {
+    int c = 0;
+    CUDA_TRY(cudaDeviceCanAccessPeer(&c, from, to));
+    *can = c != 0;
+    if (!c) return RT_OK;
+    cudaError_t e = cudaDeviceEnablePeerAccess(to, 0);
+    if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) return fail(RT_ERR_CUDA, "enable peer access %d->%d: %s", from, to, cudaGetErrorString(e));
+    cudaGetLastError();
+    return RT_OK;
+}
+
+// One replica per GPU: the same scene twice would share one set of scratch buffers and one mutex.
+int check_distinct_scenes(rt_scene *const *scenes, int ngpu) {
+    std::vector<rt_scene *> order(scenes, scenes + ngpu);
+    std::sort(order.begin(), order.end());
+    if (std::adjacent_find(order.begin(), order.end()) != order.end())
+        return fail(RT_ERR_INVALID, "the same scene was passed twice: one replica per GPU is needed");
+    return RT_OK;
+}
+
 // rt_encode_png's device buffers for one (device, stream); `mu` serialises the calls that share them.
 struct PngEncodeScratch {
     std::mutex mu;
-    uint8_t *scratch = nullptr, *out = nullptr;  // out: the file, then its length word
-    size_t scratch_cap = 0, out_cap = 0;
+    DeviceBuffer scratch, out;  // out: the file, then its length word
 };
-
-int launches_per_frame(const rt::RenderParams &p) { return kernel_variant(p) == RT_KERNEL_PHASED ? 4 : 1; }
-// RT_KERNEL_* and RT_VARIANT_* share their numbering (rt_kernels.h, rtrace.h)
-uint32_t variant_used(const rt::RenderParams &p) { return (uint32_t)kernel_variant(p); }
 
 }  // namespace
 
@@ -416,13 +508,7 @@ int rt_scene_create(uint32_t level, const float origin[3], float radius, const f
     rt::flatten_pyramid(level, origin, radius, s->flat);
     rt::normalize3(light_unnormalised, s->flat.light);
     memcpy(s->flat.eye, eye, sizeof(float) * 3);
-    int rc = upload(s);
-    if (rc != RT_OK) {
-        rt_scene_destroy(s);
-        return rc;
-    }
-    *out = s;
-    return RT_OK;
+    return finish_scene(s, out);
 }
 
 int rt_scene_create_default(rt_scene **out) {
@@ -448,49 +534,12 @@ int rt_scene_create_from_nodes(uint32_t n, const float *spheres4, const uint32_t
     s->flat.items = it;
     memcpy(s->flat.light, light, sizeof(float) * 3);
     memcpy(s->flat.eye, eye, sizeof(float) * 3);
-    int rc = upload(s);
-    if (rc != RT_OK) {
-        rt_scene_destroy(s);
-        return rc;
-    }
-    *out = s;
-    return RT_OK;
+    return finish_scene(s, out);
 }
 
 void rt_scene_destroy(rt_scene *s) {
     if (!s) return;
-    {
-        DeviceGuard g(s->device);
-        if (s->d_sph) cudaFree(s->d_sph);
-        if (s->d_skip) cudaFree(s->d_skip);
-        if (s->d_fb) cudaFree(s->d_fb);
-        if (s->d_kinds) cudaFree(s->d_kinds);
-        if (s->d_frame) cudaFree(s->d_frame);
-        if (s->d_ctr) cudaFree(s->d_ctr);
-        if (s->ev0) cudaEventDestroy(s->ev0);
-        if (s->ev1) cudaEventDestroy(s->ev1);
-        if (s->own_stream) cudaStreamDestroy(s->own_stream);
-        for (int k = 0; k < rt_scene::SWEEP_RING; k++) {
-            if (s->sweep_dev[k]) cudaFree(s->sweep_dev[k]);
-            if (s->sweep_rgb[k]) cudaFree(s->sweep_rgb[k]);
-            if (s->sweep_host[k]) cudaFreeHost(s->sweep_host[k]);
-            if (s->sweep_rendered[k]) cudaEventDestroy(s->sweep_rendered[k]);
-            if (s->sweep_copied[k]) cudaEventDestroy(s->sweep_copied[k]);
-            if (s->sweep_png[k]) cudaFree(s->sweep_png[k]);
-            if (s->sweep_len_ready[k]) cudaEventDestroy(s->sweep_len_ready[k]);
-        }
-        if (s->sweep_len_host) cudaFreeHost(s->sweep_len_host);
-        for (auto &kv : s->png_scratch)
-            if (kv.second.first) cudaFree(kv.second.first);
-        if (s->copy_stream) cudaStreamDestroy(s->copy_stream);
-        if (s->render2) cudaStreamDestroy(s->render2);
-        for (auto &kv : s->phased) {
-            if (kv.second.winner) cudaFree(kv.second.winner);
-            if (kv.second.hdr) cudaFree(kv.second.hdr);
-            if (kv.second.pool) cudaFree(kv.second.pool);
-            if (kv.second.pool_count) cudaFree(kv.second.pool_count);
-        }
-    }
+    DeviceGuard g(s->device);  // its buffers, events and streams are released on its device
     delete s;
 }
 
@@ -508,8 +557,8 @@ int rt_scene_export_nodes(const rt_scene *s, float *spheres4, uint32_t *skip, ui
     if (cap < s->n) return fail(RT_ERR_BUFFER, "need room for %u nodes, got %u", s->n, cap);
     // read back from the device: this is what the kernels traverse
     DeviceGuard g(s->device);
-    if (spheres4) CUDA_TRY(cudaMemcpy(spheres4, s->d_sph, sizeof(float4) * s->n, cudaMemcpyDeviceToHost));
-    if (skip) CUDA_TRY(cudaMemcpy(skip, s->d_skip, sizeof(uint32_t) * s->n, cudaMemcpyDeviceToHost));
+    if (spheres4) CUDA_TRY(cudaMemcpy(spheres4, s->d_sph.ptr, sizeof(float4) * s->n, cudaMemcpyDeviceToHost));
+    if (skip) CUDA_TRY(cudaMemcpy(skip, s->d_skip.ptr, sizeof(uint32_t) * s->n, cudaMemcpyDeviceToHost));
     return RT_OK;
 }
 
@@ -571,12 +620,9 @@ static int render_rows_impl(rt_scene *s, const rt_camera *camera, uint32_t width
     const bool out_on_device = rgba_out && is_device_ptr(rgba_out, &out_dev);
     if (out_on_device && out_dev != s->device) {
         // a peer GPU's memory (e.g. rank 0's frame): the kernel stores over NVLink
-        int can = 0;
-        CUDA_TRY(cudaDeviceCanAccessPeer(&can, s->device, out_dev));
+        bool can = false;
+        RT_TRY(enable_peer(s->device, out_dev, &can));
         if (!can) return fail(RT_ERR_INVALID, "rgba_out lives on device %d, which device %d cannot access", out_dev, s->device);
-        cudaError_t pe = cudaDeviceEnablePeerAccess(out_dev, 0);
-        if (pe != cudaSuccess && pe != cudaErrorPeerAccessAlreadyEnabled) return fail(RT_ERR_CUDA, "enable peer access %d->%d: %s", s->device, out_dev, cudaGetErrorString(pe));
-        cudaGetLastError();
     }
     if (out_on_device && (((uintptr_t)rgba_out) & 3)) return fail(RT_ERR_INVALID, "device rgba_out must be 4-byte aligned");
     int kinds_dev = -1;
@@ -596,9 +642,8 @@ static int render_rows_impl(rt_scene *s, const rt_camera *camera, uint32_t width
         p.out = rgba_out;
         p.pitch = pitch_bytes;
     } else {
-        rc = ensure(&s->d_fb, &s->d_fb_cap, row_bytes * row_count);
-        if (rc != RT_OK) return rc;
-        p.out = s->d_fb;
+        RT_TRY(s->d_fb.ensure(row_bytes * row_count));
+        p.out = s->d_fb.ptr;
         p.pitch = row_bytes;
     }
     bool diag = false;
@@ -607,34 +652,33 @@ static int render_rows_impl(rt_scene *s, const rt_camera *camera, uint32_t width
         if (kinds_on_device) {
             p.kinds = kinds_out;
         } else {
-            rc = ensure(&s->d_kinds, &s->d_kinds_cap, kinds_bytes ? kinds_bytes : 1);
-            if (rc != RT_OK) return rc;
-            p.kinds = s->d_kinds;
+            RT_TRY(s->d_kinds.ensure(kinds_bytes ? kinds_bytes : 1));
+            p.kinds = s->d_kinds.ptr;
         }
     }
     if (counting) {
         diag = true;
-        p.ray_counters = s->d_ctr;
-        CUDA_TRY(cudaMemsetAsync(s->d_ctr, 0, sizeof(unsigned long long) * 16, stream));
+        p.ray_counters = s->d_ctr.as<unsigned long long>();
+        CUDA_TRY(cudaMemsetAsync(s->d_ctr.ptr, 0, sizeof(unsigned long long) * 16, stream));
     }
 
     if (stats) CUDA_TRY(cudaEventRecord(s->ev0, stream));
-    rc = launch(s, p, diag, stream);
-    if (rc != RT_OK) return rc;
+    int variant = 0;
+    RT_TRY(launch(s, p, diag, stream, &variant));
     if (stats) CUDA_TRY(cudaEventRecord(s->ev1, stream));
 
     bool must_sync = false;
     if (!out_on_device && rgba_out) {
-        CUDA_TRY(cudaMemcpy2DAsync(rgba_out, pitch_bytes, s->d_fb, row_bytes, row_bytes, row_count, cudaMemcpyDeviceToHost, stream));
+        CUDA_TRY(cudaMemcpy2DAsync(rgba_out, pitch_bytes, s->d_fb.ptr, row_bytes, row_bytes, row_count, cudaMemcpyDeviceToHost, stream));
         must_sync = true;
     }
     if (kinds_out && !kinds_on_device && kinds_bytes) {
-        CUDA_TRY(cudaMemcpyAsync(kinds_out, s->d_kinds, kinds_bytes, cudaMemcpyDeviceToHost, stream));
+        CUDA_TRY(cudaMemcpyAsync(kinds_out, s->d_kinds.ptr, kinds_bytes, cudaMemcpyDeviceToHost, stream));
         must_sync = true;
     }
     unsigned long long ctr[16] = {0};
     if (counting) {
-        CUDA_TRY(cudaMemcpyAsync(ctr, s->d_ctr, sizeof(ctr), cudaMemcpyDeviceToHost, stream));
+        CUDA_TRY(cudaMemcpyAsync(ctr, s->d_ctr.ptr, sizeof(ctr), cudaMemcpyDeviceToHost, stream));
         must_sync = true;
     }
     if (must_sync || stats) CUDA_TRY(cudaStreamSynchronize(stream));
@@ -654,9 +698,9 @@ static int render_rows_impl(rt_scene *s, const rt_camera *camera, uint32_t width
         stats->total_ms = now_ms() - t0;
         stats->primary_rays = (uint64_t)cols * row_count * spp * spp;
         stats->shadow_rays = counting ? ctr[1] : 0;
-        stats->kernel_launches = (uint32_t)launches_per_frame(p);
+        stats->kernel_launches = launches_of(variant);
         stats->gpus = 1;
-        stats->variant_used = variant_used(p);
+        stats->variant_used = (uint32_t)variant;
     }
     return RT_OK;
 }
@@ -733,14 +777,13 @@ int rt_render_preview(const rt_scene *cs, const rt_camera *camera, uint32_t widt
     if (out_on_device) {
         p.out = rgba_out;
     } else {
-        rc = ensure(&s->d_fb, &s->d_fb_cap, frame_bytes);
-        if (rc != RT_OK) return rc;
-        p.out = s->d_fb;
+        RT_TRY(s->d_fb.ensure(frame_bytes));
+        p.out = s->d_fb.ptr;
     }
     cudaError_t e = rt_launch_render_preview(p, stream);
     if (e != cudaSuccess) return fail(RT_ERR_CUDA, "kernel launch: %s", cudaGetErrorString(e));
     if (!out_on_device) {
-        CUDA_TRY(cudaMemcpyAsync(rgba_out, s->d_fb, frame_bytes, cudaMemcpyDeviceToHost, stream));
+        CUDA_TRY(cudaMemcpyAsync(rgba_out, s->d_fb.ptr, frame_bytes, cudaMemcpyDeviceToHost, stream));
         CUDA_TRY(cudaStreamSynchronize(stream));
     }
     return RT_OK;
@@ -780,19 +823,10 @@ struct CallbackSource : FrameSource {
 };
 
 static int sweep_locked(rt_scene *s, FrameSource &src, uint32_t width, uint32_t height, uint32_t spp, rt_frame_callback cb,
-                        void *user, rt_stats *stats, OutKind kind, const Animation &anim);
-
-// The PNG encoder's scratch for this render stream (allocated on first use, grown on demand): two frames in flight
-// on two streams encode at the same time.
-static int png_scratch_for(rt_scene *s, cudaStream_t stream, uint32_t width, uint32_t height, uint8_t **out) {
-    std::pair<uint8_t *, size_t> &sc = s->png_scratch[stream];
-    int rc = ensure(&sc.first, &sc.second, rt_png_scratch_bytes(width, height));
-    *out = sc.first;
-    return rc;
-}
+                        void *user, rt_stats *stats, OutKind kind, const Animation *anim);
 
 static int sweep_impl(const rt_scene *cs, FrameSource &src, uint32_t width, uint32_t height, uint32_t spp,
-                      rt_frame_callback cb, void *user, rt_stats *stats, OutKind kind, const Animation &anim = Animation()) {
+                      rt_frame_callback cb, void *user, rt_stats *stats, OutKind kind, const Animation *anim = nullptr) {
     rt_scene *s = const_cast<rt_scene *>(cs);
     int rc = check_frame_args(s, width, height, spp, 0, 1, height);
     if (rc != RT_OK) return rc;
@@ -810,16 +844,14 @@ static int sweep_impl(const rt_scene *cs, FrameSource &src, uint32_t width, uint
     return rc;
 }
 
+// anim != nullptr (PNG only): every frame is its payload of that animated PNG
 static int sweep_locked(rt_scene *s, FrameSource &src, uint32_t width, uint32_t height, uint32_t spp, rt_frame_callback cb,
-                        void *user, rt_stats *stats, OutKind kind, const Animation &anim) {
-    int rc = RT_OK;
+                        void *user, rt_stats *stats, OutKind kind, const Animation *anim) {
     const double t0 = now_ms();
-    // an APNG frame takes the PNG path with another bound and another encode launch
-    const bool rgb = kind == OutKind::RGB, apng = kind == OutKind::APNG, png = kind == OutKind::PNG || apng;
+    const bool rgb = kind == OutKind::RGB, png = kind == OutKind::PNG;
     const size_t row_bytes = (size_t)width * 4, frame_bytes = row_bytes * height;
     const size_t out_bytes = rgb ? (size_t)width * height * 3 : frame_bytes;
-    const size_t png_bytes = apng ? rt_apng_bound_bytes(width, height) : png ? rt_png_bound_bytes(width, height) : 0;
-    const size_t png_len_at = (png_bytes + 7) / 8 * 8;
+    const size_t png_bytes = !png ? 0 : anim ? rt_apng_bound_bytes(width, height) : rt_png_bound_bytes(width, height);
     const size_t host_bytes = std::max(frame_bytes, png_bytes);
     // `depth` frames render at a time, each on its own stream (depth 2: the launch tails of frame f are filled
     // by the first launches of frame f+1), while an earlier frame is copied out: depth + 1 device frames and
@@ -831,42 +863,8 @@ static int sweep_locked(rt_scene *s, FrameSource &src, uint32_t width, uint32_t 
         if (*e == '1') depth = 1;
     }
     const int nb = depth + 1;
-    if (s->sweep_bytes < frame_bytes || s->sweep_host_bytes < host_bytes || s->sweep_nb < nb) {
-        for (int k = 0; k < rt_scene::SWEEP_RING; k++) {
-            if (s->sweep_dev[k]) cudaFree(s->sweep_dev[k]);
-            if (s->sweep_host[k]) cudaFreeHost(s->sweep_host[k]);
-            s->sweep_dev[k] = s->sweep_host[k] = nullptr;
-        }
-        s->sweep_bytes = 0;
-        s->sweep_host_bytes = 0;
-        s->sweep_nb = 0;
-        for (int k = 0; k < nb; k++) {
-            if (s->sweep_rgb[k]) cudaFree(s->sweep_rgb[k]);
-            s->sweep_rgb[k] = nullptr;
-            CUDA_TRY(cudaMalloc(&s->sweep_dev[k], frame_bytes));
-            CUDA_TRY(cudaMalloc(&s->sweep_rgb[k], frame_bytes / 4 * 3 + 16));
-            CUDA_TRY(cudaHostAlloc((void **)&s->sweep_host[k], host_bytes, cudaHostAllocPortable));
-        }
-        s->sweep_bytes = frame_bytes;
-        s->sweep_host_bytes = host_bytes;
-        s->sweep_nb = nb;
-    }
-    if (png) {
-        for (int k = 0; k < nb; k++) {
-            rc = ensure(&s->sweep_png[k], &s->sweep_png_cap[k], png_len_at + sizeof(unsigned long long));
-            if (rc != RT_OK) return rc;
-        }
-        if (!s->sweep_len_host) CUDA_TRY(cudaHostAlloc((void **)&s->sweep_len_host, sizeof(unsigned long long) * rt_scene::SWEEP_RING, cudaHostAllocPortable));
-    }
-    if (depth == 2 && !s->render2) CUDA_TRY(cudaStreamCreateWithFlags(&s->render2, cudaStreamNonBlocking));
-    if (!s->copy_stream) {
-        CUDA_TRY(cudaStreamCreateWithFlags(&s->copy_stream, cudaStreamNonBlocking));
-        for (int k = 0; k < rt_scene::SWEEP_RING; k++) {
-            CUDA_TRY(cudaEventCreateWithFlags(&s->sweep_rendered[k], cudaEventDisableTiming));
-            CUDA_TRY(cudaEventCreateWithFlags(&s->sweep_copied[k], cudaEventDisableTiming));
-            CUDA_TRY(cudaEventCreateWithFlags(&s->sweep_len_ready[k], cudaEventDisableTiming));
-        }
-    }
+    if (depth == 2) RT_TRY(s->render2.create());
+    RT_TRY(s->copy_stream.create());
     uint32_t launches = 0, used = 0;
     uint64_t issued = 0, delivered = 0;  // frames put into / handed out of the ring, in this order
     int64_t ids[rt_scene::SWEEP_RING] = {0, 0, 0};
@@ -880,41 +878,42 @@ static int sweep_locked(rt_scene *s, FrameSource &src, uint32_t width, uint32_t 
                 more = false;
             } else {
                 const int k = (int)(issued % (uint64_t)nb);
+                SweepSlot &sl = s->sweep[k];
                 ids[k] = id;
+                RT_TRY(sl.frame.ensure(frame_bytes));
+                RT_TRY(sl.host.ensure(host_bytes));
+                if (rgb) RT_TRY(sl.rgb.ensure(frame_bytes / 4 * 3 + 16));
+                if (png) RT_TRY(sl.len.ensure(sizeof(unsigned long long)));
+                for (Event *e : {&sl.rendered, &sl.copied, &sl.len_ready}) RT_TRY(e->create(cudaEventDisableTiming));
                 cudaStream_t rs = (depth == 2 && (issued & 1u)) ? s->render2 : s->own_stream;  // PHASED scratch is per stream
                 rt::RenderParams p;
                 fill_params(s, use_cam ? &cam : nullptr, width, height, spp, 0, 1, height, p);
-                p.out = s->sweep_dev[k];
+                p.out = sl.frame.ptr;
                 p.pitch = row_bytes;
-                if (issued >= (uint64_t)nb) CUDA_TRY(cudaStreamWaitEvent(rs, s->sweep_copied[k], 0));  // its previous frame has left this buffer
-                rc = launch(s, p, false, rs);
-                if (rc != RT_OK) return rc;
-                launches += (uint32_t)launches_per_frame(p);
-                used = variant_used(p);
+                if (issued >= (uint64_t)nb) CUDA_TRY(cudaStreamWaitEvent(rs, sl.copied, 0));  // its previous frame has left this buffer
+                int variant = 0;
+                RT_TRY(launch(s, p, false, rs, &variant));
+                launches += launches_of(variant);
+                used = (uint32_t)variant;
                 if (rgb) {  // the sink only needs RGB: pack on the device, copy 3 bytes per pixel
-                    CUDA_TRY(rt_launch_pack_rgb(s->sweep_dev[k], s->sweep_rgb[k], (size_t)width * height, rs));
+                    CUDA_TRY(rt_launch_pack_rgb(sl.frame.ptr, sl.rgb.ptr, (size_t)width * height, rs));
                     launches += 1;
                 }
                 if (png) {
                     // encode behind the frame's launches; only the length word comes back now (on the render
                     // stream, so that the copy stream never waits for a later frame); the file is copied at hand-over
-                    uint8_t *scratch = nullptr;
-                    rc = png_scratch_for(s, rs, width, height, &scratch);
-                    if (rc != RT_OK) return rc;
-                    unsigned long long *len_word = reinterpret_cast<unsigned long long *>(s->sweep_png[k] + png_len_at);
-                    if (apng)
-                        CUDA_TRY(rt_launch_apng_encode(s->sweep_dev[k], row_bytes, width, height, (uint32_t)id, anim.n_frames,
-                                                       anim.delay_num, anim.delay_den, scratch, s->sweep_png[k], len_word, rs));
-                    else
-                        CUDA_TRY(rt_launch_png_encode(s->sweep_dev[k], row_bytes, width, height, scratch, s->sweep_png[k], len_word, rs));
-                    CUDA_TRY(cudaMemcpyAsync(&s->sweep_len_host[k], len_word, sizeof(unsigned long long), cudaMemcpyDeviceToHost, rs));
-                    CUDA_TRY(cudaEventRecord(s->sweep_len_ready[k], rs));
+                    {
+                        std::lock_guard<std::mutex> lock(s->mu_scratch);
+                        RT_TRY(queue_encode(sl.frame.ptr, row_bytes, width, height, anim, (uint32_t)id, png_bytes,
+                                            s->scratch[rs].png, sl.png, sl.len.as<unsigned long long>(), rs));
+                    }
+                    CUDA_TRY(cudaEventRecord(sl.len_ready, rs));
                     launches += 2;
                 } else {
-                    CUDA_TRY(cudaEventRecord(s->sweep_rendered[k], rs));
-                    CUDA_TRY(cudaStreamWaitEvent(s->copy_stream, s->sweep_rendered[k], 0));
-                    CUDA_TRY(cudaMemcpyAsync(s->sweep_host[k], rgb ? s->sweep_rgb[k] : s->sweep_dev[k], out_bytes, cudaMemcpyDeviceToHost, s->copy_stream));
-                    CUDA_TRY(cudaEventRecord(s->sweep_copied[k], s->copy_stream));
+                    CUDA_TRY(cudaEventRecord(sl.rendered, rs));
+                    CUDA_TRY(cudaStreamWaitEvent(s->copy_stream, sl.rendered, 0));
+                    CUDA_TRY(cudaMemcpyAsync(sl.host.ptr, rgb ? sl.rgb.ptr : sl.frame.ptr, out_bytes, cudaMemcpyDeviceToHost, s->copy_stream));
+                    CUDA_TRY(cudaEventRecord(sl.copied, s->copy_stream));
                 }
                 issued++;
             }
@@ -922,16 +921,17 @@ static int sweep_locked(rt_scene *s, FrameSource &src, uint32_t width, uint32_t 
         if (issued - delivered > (uint64_t)depth || (!more && delivered < issued)) {
             // hand the oldest frame to the caller while the later ones render
             const int k = (int)(delivered % (uint64_t)nb);
+            SweepSlot &sl = s->sweep[k];
             size_t len = out_bytes;
             if (png) {  // the file's length first, then just that many bytes
-                CUDA_TRY(cudaEventSynchronize(s->sweep_len_ready[k]));
-                len = (size_t)s->sweep_len_host[k];
+                CUDA_TRY(cudaEventSynchronize(sl.len_ready));
+                len = (size_t)*sl.len.as<unsigned long long>();
                 if (len > png_bytes) return fail(RT_ERR_CUDA, "PNG encoder returned %zu bytes, more than the bound %zu", len, png_bytes);
-                CUDA_TRY(cudaMemcpyAsync(s->sweep_host[k], s->sweep_png[k], len, cudaMemcpyDeviceToHost, s->copy_stream));
-                CUDA_TRY(cudaEventRecord(s->sweep_copied[k], s->copy_stream));
+                CUDA_TRY(cudaMemcpyAsync(sl.host.ptr, sl.png.ptr, len, cudaMemcpyDeviceToHost, s->copy_stream));
+                CUDA_TRY(cudaEventRecord(sl.copied, s->copy_stream));
             }
-            CUDA_TRY(cudaEventSynchronize(s->sweep_copied[k]));
-            if (cb) cb(user, (uint32_t)ids[k], s->sweep_host[k], len);
+            CUDA_TRY(cudaEventSynchronize(sl.copied));
+            if (cb) cb(user, (uint32_t)ids[k], sl.host.ptr, len);
             delivered++;
         }
     }
@@ -991,16 +991,7 @@ static int frame_multi_locked(rt_scene *const *scenes, int ngpu, const rt_camera
         DeviceGuard guard(s->device);
         if (!guard.ok) return fail(RT_ERR_CUDA, "cannot select device %d", s->device);
         bool peer = g == 0 || !to_device;
-        if (to_device && g > 0) {
-            int can = 0;
-            CUDA_TRY(cudaDeviceCanAccessPeer(&can, s->device, root->device));
-            if (can) {
-                cudaError_t e = cudaDeviceEnablePeerAccess(root->device, 0);
-                if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) return fail(RT_ERR_CUDA, "enable peer %d->%d: %s", s->device, root->device, cudaGetErrorString(e));
-                cudaGetLastError();
-                peer = true;
-            }
-        }
+        if (!peer) RT_TRY(enable_peer(s->device, root->device, &peer));
         rt::RenderParams p;
         uint32_t rows;
         const uint32_t first = (uint32_t)g * B, stride = (uint32_t)ngpu * B;
@@ -1015,37 +1006,33 @@ static int frame_multi_locked(rt_scene *const *scenes, int ngpu, const rt_camera
             if (to_device) {
                 p.out = frame;
             } else {
-                int rc = ensure(&s->d_frame, &s->d_frame_cap, row_bytes * height);
-                if (rc != RT_OK) return rc;
-                p.out = s->d_frame;
+                RT_TRY(s->d_frame.ensure(row_bytes * height));
+                p.out = s->d_frame.ptr;
             }
             p.pitch = row_bytes;
         } else {
             rows = (height > (uint32_t)g) ? (height - g + ngpu - 1) / ngpu : 0;
             if (rows == 0) continue;
             fill_params(s, camera, width, height, spp, (uint32_t)g, (uint32_t)ngpu, rows, p);
-            int rc = ensure(&s->d_fb, &s->d_fb_cap, row_bytes * rows);
-            if (rc != RT_OK) return rc;
-            p.out = s->d_fb;
+            RT_TRY(s->d_fb.ensure(row_bytes * rows));
+            p.out = s->d_fb.ptr;
             p.pitch = row_bytes;
         }
         if (stats) CUDA_TRY(cudaEventRecord(s->ev0, s->own_stream));
         launched[(size_t)g] = 1;  // from here on this GPU may have work in flight
-        {
-            int rc = launch(s, p, false, s->own_stream);
-            if (rc != RT_OK) return rc;
-        }
-        launches += (uint32_t)launches_per_frame(p);
-        if (g == 0) used = variant_used(p);
+        int variant = 0;
+        RT_TRY(launch(s, p, false, s->own_stream, &variant));
+        launches += launches_of(variant);
+        if (g == 0) used = (uint32_t)variant;
         if (stats) CUDA_TRY(cudaEventRecord(s->ev1, s->own_stream));
         if (!to_device) {
             // this GPU's blocks -> the host frame: whole blocks as one strided copy, then the partial last block
             const size_t blk = (size_t)B * row_bytes, pitch = (size_t)stride * row_bytes, off = (size_t)first * row_bytes;
             const uint32_t whole = rows / B, tail = rows % B;
-            if (whole) CUDA_TRY(cudaMemcpy2DAsync(rgba_out + off, pitch, s->d_frame + off, pitch, blk, whole, cudaMemcpyDeviceToHost, s->own_stream));
-            if (tail) CUDA_TRY(cudaMemcpyAsync(rgba_out + off + (size_t)whole * pitch, s->d_frame + off + (size_t)whole * pitch, (size_t)tail * row_bytes, cudaMemcpyDeviceToHost, s->own_stream));
+            if (whole) CUDA_TRY(cudaMemcpy2DAsync(rgba_out + off, pitch, s->d_frame.ptr + off, pitch, blk, whole, cudaMemcpyDeviceToHost, s->own_stream));
+            if (tail) CUDA_TRY(cudaMemcpyAsync(rgba_out + off + (size_t)whole * pitch, s->d_frame.ptr + off + (size_t)whole * pitch, (size_t)tail * row_bytes, cudaMemcpyDeviceToHost, s->own_stream));
         } else if (!peer) {  // no peer access: strided copy, the pitch de-interleaves the band into the frame
-            CUDA_TRY(cudaMemcpy2DAsync(frame + row_bytes * g, row_bytes * ngpu, s->d_fb, row_bytes, row_bytes, rows, cudaMemcpyDefault, s->own_stream));
+            CUDA_TRY(cudaMemcpy2DAsync(frame + row_bytes * g, row_bytes * ngpu, s->d_fb.ptr, row_bytes, row_bytes, rows, cudaMemcpyDefault, s->own_stream));
         }
     }
     double kmax = 0.0;
@@ -1071,13 +1058,12 @@ static int frame_multi_locked(rt_scene *const *scenes, int ngpu, const rt_camera
 }
 
 // Distinct scenes, locked in address order (two threads passing the same scenes in different orders cannot
-// deadlock; the same scene twice would lock one mutex twice, so it is rejected).
+// deadlock).
 static int lock_scenes(rt_scene *const *scenes, int ngpu, std::vector<std::unique_lock<std::mutex>> &locks) {
+    RT_TRY(check_distinct_scenes(scenes, ngpu));
     std::vector<rt_scene *> order(scenes, scenes + ngpu);
     std::sort(order.begin(), order.end());
-    for (int g = 1; g < ngpu; g++)
-        if (order[(size_t)g] == order[(size_t)g - 1]) return fail(RT_ERR_INVALID, "the same scene was passed twice: one replica per GPU is needed");
-    for (int g = 0; g < ngpu; g++) locks.emplace_back(order[(size_t)g]->mu);
+    for (rt_scene *s : order) locks.emplace_back(s->mu);
     return RT_OK;
 }
 
@@ -1172,7 +1158,7 @@ void board_offer(void *user, uint32_t frame, const uint8_t *data, size_t len) {
 
 static int sweep_multi_impl(rt_scene *const *scenes, int ngpu, const rt_camera *cameras, uint32_t n_frames, uint32_t width,
                             uint32_t height, uint32_t spp, OutKind kind, rt_frame_callback cb, void *user, rt_stats *stats,
-                            const Animation &anim = Animation()) {
+                            const Animation *anim = nullptr) {
     if (!scenes || ngpu < 1) return fail(RT_ERR_INVALID, "need at least one scene");
     for (int g = 0; g < ngpu; g++) {
         int rc = check_frame_args(scenes[g], width, height, spp, 0, 1, height);
@@ -1184,12 +1170,7 @@ static int sweep_multi_impl(rt_scene *const *scenes, int ngpu, const rt_camera *
         ListSource src(cameras, n_frames);
         return sweep_impl(scenes[0], src, width, height, spp, cb, user, stats, kind, anim);
     }
-    {   // distinct scenes (each worker locks its own)
-        std::vector<rt_scene *> order(scenes, scenes + ngpu);
-        std::sort(order.begin(), order.end());
-        for (int g = 1; g < ngpu; g++)
-            if (order[(size_t)g] == order[(size_t)g - 1]) return fail(RT_ERR_INVALID, "the same scene was passed twice: one replica per GPU is needed");
-    }
+    RT_TRY(check_distinct_scenes(scenes, ngpu));  // each worker locks its own
     const double t0 = now_ms();
     const int variant = g_variant;  // the caller's choice travels to the workers (it is thread-local)
     SweepBoard board;
@@ -1272,7 +1253,7 @@ int rt_render_sweep_apng(rt_scene *const *scenes, int ngpu, const rt_camera *cam
     if (rc != RT_OK) return rc;
     Animation anim;
     anim.n_frames = n_frames, anim.delay_num = delay_num, anim.delay_den = delay_den;
-    return sweep_multi_impl(scenes, ngpu, cameras, n_frames, width, height, spp, OutKind::APNG, cb, user, stats, anim);
+    return sweep_multi_impl(scenes, ngpu, cameras, n_frames, width, height, spp, OutKind::PNG, cb, user, stats, &anim);
 }
 
 uint64_t rt_atomic_fetch_add_u64(void *addr, uint64_t value) {
@@ -1298,7 +1279,7 @@ int rt_trace_rays(const rt_scene *s, size_t n, const rt_ray *rays, rt_hit *hits)
     CUDA_TRY(cudaMalloc(&d_rays, n * sizeof(rt_ray)));
     cudaError_t e = cudaMalloc(&d_hits, n * sizeof(rt_hit));
     if (e == cudaSuccess) e = cudaMemcpy(d_rays, rays, n * sizeof(rt_ray), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = rt_launch_trace_rays(s->d_sph, s->d_skip, s->n, n, d_rays, d_hits, nullptr);
+    if (e == cudaSuccess) e = rt_launch_trace_rays(s->d_sph.as<float4>(), s->d_skip.as<uint32_t>(), s->n, n, d_rays, d_hits, nullptr);
     if (e == cudaSuccess) e = cudaMemcpy(hits, d_hits, n * sizeof(rt_hit), cudaMemcpyDeviceToHost);
     cudaFree(d_rays);
     if (d_hits) cudaFree(d_hits);
@@ -1372,18 +1353,19 @@ int rt_debug_phased_tiles(const rt_scene *cs, uint32_t cap_tiles, uint32_t *n_ti
     if (!s || !n_tiles) return fail(RT_ERR_INVALID, "NULL argument");
     DeviceGuard guard(s->device);
     CUDA_TRY(cudaDeviceSynchronize());
-    std::lock_guard<std::mutex> lock(s->mu_phased);
-    if (s->phased.empty()) return fail(RT_ERR_INVALID, "no PHASED frame rendered yet");
-    rt_scene::Phased &ph = s->phased.begin()->second;
-    const uint32_t nt = (uint32_t)(ph.hdr_cap / sizeof(uint4));
+    std::lock_guard<std::mutex> lock(s->mu_scratch);
+    auto it = std::find_if(s->scratch.begin(), s->scratch.end(), [](const auto &kv) { return kv.second.pool_count.ptr != nullptr; });
+    if (it == s->scratch.end()) return fail(RT_ERR_INVALID, "no PHASED frame rendered yet");
+    const StreamScratch &ph = it->second;
+    const uint32_t nt = (uint32_t)(ph.hdr.cap / sizeof(uint4));
     *n_tiles = nt;
     if (!counts) return RT_OK;
     uint32_t used = 0;
-    CUDA_TRY(cudaMemcpy(&used, ph.pool_count, sizeof(used), cudaMemcpyDeviceToHost));
+    CUDA_TRY(cudaMemcpy(&used, ph.pool_count.ptr, sizeof(used), cudaMemcpyDeviceToHost));
     used = std::min(used, ph.pool_units);
     std::vector<uint4> hdr(nt), pool(used);
-    CUDA_TRY(cudaMemcpy(hdr.data(), ph.hdr, (size_t)nt * sizeof(uint4), cudaMemcpyDeviceToHost));
-    CUDA_TRY(cudaMemcpy(pool.data(), ph.pool, (size_t)used * sizeof(uint4), cudaMemcpyDeviceToHost));
+    CUDA_TRY(cudaMemcpy(hdr.data(), ph.hdr.ptr, (size_t)nt * sizeof(uint4), cudaMemcpyDeviceToHost));
+    CUDA_TRY(cudaMemcpy(pool.data(), ph.pool.ptr, (size_t)used * sizeof(uint4), cudaMemcpyDeviceToHost));
     for (uint32_t t = 0; t < nt && t < cap_tiles; t++) {
         const uint32_t heads[2] = {hdr[t].x, hdr[t].y};
         for (int k = 0; k < 2; k++) {
@@ -1499,33 +1481,22 @@ static int encode_impl(const uint8_t *rgba, uint32_t width, uint32_t height, siz
     cudaStream_t stream = (cudaStream_t)stream_;
     // scratch per (device, stream), kept for the life of the process: no allocation per call once it has grown
     static std::mutex g_mu;
-    static std::map<std::pair<int, cudaStream_t>, std::unique_ptr<PngEncodeScratch>> g_scratch;
+    // never deleted on purpose: no buffer is released in static destruction at process exit
+    static auto *g_scratch = new std::map<std::pair<int, cudaStream_t>, PngEncodeScratch>();
     PngEncodeScratch *sc;
     {
         std::lock_guard<std::mutex> lock(g_mu);
-        std::unique_ptr<PngEncodeScratch> &slot = g_scratch[std::make_pair(cur, stream)];
-        if (!slot) slot.reset(new (std::nothrow) PngEncodeScratch());
-        if (!slot) return fail(RT_ERR_NOMEM, "out of host memory");
-        sc = slot.get();
+        sc = &(*g_scratch)[std::make_pair(cur, stream)];
     }
     std::lock_guard<std::mutex> lock(sc->mu);
-    const size_t len_at = (bound + 7) / 8 * 8;
-    rc = ensure(&sc->scratch, &sc->scratch_cap, rt_png_scratch_bytes(width, height));
-    if (rc == RT_OK) rc = ensure(&sc->out, &sc->out_cap, len_at + sizeof(unsigned long long));
-    if (rc != RT_OK) return rc;
-    unsigned long long *len_word = reinterpret_cast<unsigned long long *>(sc->out + len_at), len = 0;
-    if (anim)
-        CUDA_TRY(rt_launch_apng_encode(rgba, pitch_bytes, width, height, frame, anim->n_frames, anim->delay_num,
-                                       anim->delay_den, sc->scratch, sc->out, len_word, stream));
-    else
-        CUDA_TRY(rt_launch_png_encode(rgba, pitch_bytes, width, height, sc->scratch, sc->out, len_word, stream));
-    CUDA_TRY(cudaMemcpyAsync(&len, len_word, sizeof(len), cudaMemcpyDeviceToHost, stream));
+    unsigned long long len = 0;
+    RT_TRY(queue_encode(rgba, pitch_bytes, width, height, anim, frame, bound, sc->scratch, sc->out, &len, stream));
     CUDA_TRY(cudaStreamSynchronize(stream));
     if (len == 0 || len > bound) return fail(RT_ERR_CUDA, "PNG encoder returned %llu bytes (bound %zu)", len, bound);
     *len_out = (size_t)len;
     if (len > cap) return fail(RT_ERR_BUFFER, "%s holds %zu bytes, the %s needs %llu", anim ? "out" : "png_out", cap,
                                anim ? "frame" : "file", len);
-    CUDA_TRY(cudaMemcpyAsync(file_out, sc->out, (size_t)len, cudaMemcpyDefault, stream));
+    CUDA_TRY(cudaMemcpyAsync(file_out, sc->out.ptr, (size_t)len, cudaMemcpyDefault, stream));
     CUDA_TRY(cudaStreamSynchronize(stream));
     return RT_OK;
 }
