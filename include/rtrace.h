@@ -62,7 +62,8 @@ typedef struct rt_stats {
     uint32_t gpus;
     uint32_t variant_used; /* RT_VARIANT_* the call actually ran (AUTO resolved; LANE when the arguments leave
                               the candidate-list variants' domain: spp > 8, level > 10, eye inside the root
-                              bound, non-orthonormal camera, scene far from the coordinate origin)        */
+                              bound, camera basis whose row dot products are more than 1e-6 off orthonormal,
+                              scene far from the coordinate origin)                                         */
     uint32_t reserved;
 } rt_stats;
 

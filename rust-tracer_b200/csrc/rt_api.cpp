@@ -299,12 +299,16 @@ int check_frame_args(const rt_scene *s, uint32_t w, uint32_t h, uint32_t spp, ui
     return RT_OK;
 }
 
-// A camera basis must be orthonormal for the TILE variant's cone bounds to hold.
+// A camera basis must be orthonormal for the TILE variant's cone bounds and PHASED's image-space boxes to hold.
+// screen_box (rt_phased.cu) maps a centre into camera space with the basis rows, which inverts the ray rotation
+// only up to (B B^T - I) v: row dot products off by 1e-5 move a box by up to ~1 px on a 65535-wide frame and past
+// its 0.05 px slack from 4K up.  At 1e-6 every width keeps >= 0.05 px of margin (tests/test_camera_margin.py),
+// and a rotation rounded to f32 is off by ~1e-7, so orbit and look-at cameras stay on the fast path.
 bool orthonormal(const float b[9]) {
     for (int i = 0; i < 3; i++)
         for (int j = i; j < 3; j++) {
             float d = b[3 * i] * b[3 * j] + b[3 * i + 1] * b[3 * j + 1] + b[3 * i + 2] * b[3 * j + 2];
-            if (fabsf(d - (i == j ? 1.0f : 0.0f)) > 1e-5f) return false;
+            if (fabsf(d - (i == j ? 1.0f : 0.0f)) > 1e-6f) return false;
         }
     return true;
 }
