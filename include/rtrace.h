@@ -296,7 +296,9 @@ int rt_selftest_math(uint32_t n, uint32_t seed, uint64_t mismatches[6]);
 
 /* Diagnostics: candidate counts per cull tile of the scene's most recent PHASED frame
  * (counts[2t] = primary, counts[2t+1] = shadow candidates, 0xffffffff = tile rendered by the
- * per-lane walk); *n_tiles = number of tiles, counts may be NULL to query it. */
+ * per-lane walk, 0xfffffffd = shadow rays of the tile all occluded by one leaf, no list and no
+ * test); *n_tiles = number of tiles (the capacity of a buffer that only grows: the tiles of the
+ * last frame come first), counts may be NULL to query it. */
 int rt_debug_phased_tiles(const rt_scene *s, uint32_t cap_tiles, uint32_t *n_tiles, uint32_t *counts);
 
 /* Device memory on the current device, and CUDA IPC handles for it: how the ranks of a

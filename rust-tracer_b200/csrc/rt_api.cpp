@@ -1351,7 +1351,8 @@ int rt_measure_fp32_peak(int device, double *tflops, double *sm_clock_mhz) {
 
 // Diagnostic: candidate counts per cull tile of the most recent PHASED frame of this scene
 // (walks the chunk chains on the host).  counts[2*t] = primary, counts[2*t+1] = shadow candidates;
-// 0xffffffff = tile handled by the per-lane walk.  Returns the number of tiles through *n_tiles.
+// 0xffffffff = tile handled by the per-lane walk, 0xfffffffd (shadow only) = every shadow ray of the tile occluded
+// by one leaf, no list.  Returns the number of tiles through *n_tiles.
 int rt_debug_phased_tiles(const rt_scene *cs, uint32_t cap_tiles, uint32_t *n_tiles, uint32_t *counts) {
     rt_scene *s = const_cast<rt_scene *>(cs);
     if (!s || !n_tiles) return fail(RT_ERR_INVALID, "NULL argument");
@@ -1375,7 +1376,7 @@ int rt_debug_phased_tiles(const rt_scene *cs, uint32_t cap_tiles, uint32_t *n_ti
         for (int k = 0; k < 2; k++) {
             uint32_t n = 0, b = heads[k];
             if (b == 0xfffffffeu) n = 0xffffffffu;
-            else if (b == 0xfffffffdu) n = 1;  // COVERED: one leaf occludes every shadow ray of the tile
+            else if (b == 0xfffffffdu) n = 0xfffffffdu;  // COVERED: one leaf occludes every shadow ray of the tile
             else
                 for (int guard_n = 0; b != 0xffffffffu && b < used && guard_n < 100000; guard_n++) n += pool[b].x, b = pool[b].y;
             counts[2 * t + k] = n;

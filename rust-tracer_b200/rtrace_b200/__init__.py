@@ -509,7 +509,10 @@ def selftest_math(n=1 << 24, seed=1):
 
 
 def debug_phased_tiles(scene):
-    """(n_tiles, 2) uint32 array: primary / shadow candidates per cull tile of the last PHASED frame."""
+    """(n_tiles, 2) uint32 array: primary / shadow candidates per cull tile of the last PHASED frame.
+    0xffffffff marks a tile rendered by the per-lane walk, 0xfffffffd (shadow column) a tile whose shadow rays
+    one leaf occludes (no list, no test).  n_tiles is the capacity of the tile-header buffer, which only grows:
+    the last frame's tiles are the first rows."""
     n = C.c_uint32()
     L = lib()
     L.rt_debug_phased_tiles.argtypes = [C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32), C.c_void_p]
