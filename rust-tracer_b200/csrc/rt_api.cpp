@@ -43,12 +43,6 @@ struct RowLayout {
 // Animation: the frame's payload of an animated PNG).
 enum class OutKind { RGBA, RGB, PNG };
 
-// The animation an APNG frame belongs to: its frame count and how long each frame shows (delay_num / delay_den s).
-struct Animation {
-    uint32_t n_frames = 0;
-    uint16_t delay_num = 0, delay_den = 0;
-};
-
 int fail(int code, const char *fmt, ...) {
     va_list ap;
     va_start(ap, fmt);
@@ -428,7 +422,7 @@ uint32_t launches_of(int variant) { return variant == RT_KERNEL_PHASED ? 4 : 1; 
 
 // Queues on `stream` the PNG encode of the RGBA8 frame `rgba` (anim != nullptr: frame `frame`'s payload of that
 // animated PNG) into `out` -- the file, then its length word -- and the copy of the length word to *len_host.
-// `bound` is the bound of that file (rt_png_bound_bytes / rt_apng_bound_bytes).
+// `bound` is the bound of that file (rt_png_bound_bytes).
 int queue_encode(const uint8_t *rgba, size_t pitch, uint32_t width, uint32_t height, const Animation *anim,
                  uint32_t frame, size_t bound, DeviceBuffer &scratch, DeviceBuffer &out, unsigned long long *len_host,
                  cudaStream_t stream) {
@@ -436,11 +430,7 @@ int queue_encode(const uint8_t *rgba, size_t pitch, uint32_t width, uint32_t hei
     RT_TRY(scratch.ensure(rt_png_scratch_bytes(width, height)));
     RT_TRY(out.ensure(len_at + sizeof(unsigned long long)));
     unsigned long long *len_word = reinterpret_cast<unsigned long long *>(out.ptr + len_at);
-    if (anim)
-        CUDA_TRY(rt_launch_apng_encode(rgba, pitch, width, height, frame, anim->n_frames, anim->delay_num,
-                                       anim->delay_den, scratch.ptr, out.ptr, len_word, stream));
-    else
-        CUDA_TRY(rt_launch_png_encode(rgba, pitch, width, height, scratch.ptr, out.ptr, len_word, stream));
+    CUDA_TRY(rt_launch_png_encode(rgba, pitch, width, height, anim, frame, scratch.ptr, out.ptr, len_word, stream));
     CUDA_TRY(cudaMemcpyAsync(len_host, len_word, sizeof(unsigned long long), cudaMemcpyDeviceToHost, stream));
     return RT_OK;
 }
@@ -855,7 +845,7 @@ static int sweep_locked(rt_scene *s, FrameSource &src, uint32_t width, uint32_t 
     const bool rgb = kind == OutKind::RGB, png = kind == OutKind::PNG;
     const size_t row_bytes = (size_t)width * 4, frame_bytes = row_bytes * height;
     const size_t out_bytes = rgb ? (size_t)width * height * 3 : frame_bytes;
-    const size_t png_bytes = !png ? 0 : anim ? rt_apng_bound_bytes(width, height) : rt_png_bound_bytes(width, height);
+    const size_t png_bytes = png ? rt_png_bound_bytes(width, height, anim) : 0;
     const size_t host_bytes = std::max(frame_bytes, png_bytes);
     // `depth` frames render at a time, each on its own stream (depth 2: the launch tails of frame f are filled
     // by the first launches of frame f+1), while an earlier frame is copied out: depth + 1 device frames and
@@ -1449,7 +1439,7 @@ int rt_png_bound(uint32_t width, uint32_t height, size_t *bytes) {
     if (!bytes) return fail(RT_ERR_INVALID, "NULL argument");
     if (width == 0 || height == 0 || width > 65535u || height > 65535u)
         return fail(RT_ERR_INVALID, "width/height must be in 1..65535 (got %u x %u)", width, height);
-    *bytes = rt_png_bound_bytes(width, height);
+    *bytes = rt_png_bound_bytes(width, height, nullptr);
     return RT_OK;
 }
 
@@ -1463,7 +1453,8 @@ int rt_apng_bound(uint32_t width, uint32_t height, uint32_t n_frames, size_t *fr
     const uint64_t last_seq = (uint64_t)(n_frames - 1) * ((height + 15u) / 16u + 3u);
     if (last_seq > 0x7fffffffu)
         return fail(RT_ERR_INVALID, "%u frames of height %u need sequence numbers beyond 2^31 - 1", n_frames, height);
-    *frame_bytes = rt_apng_bound_bytes(width, height);
+    const Animation anim{n_frames};
+    *frame_bytes = rt_png_bound_bytes(width, height, &anim);
     return RT_OK;
 }
 

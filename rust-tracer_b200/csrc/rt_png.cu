@@ -13,10 +13,11 @@
 //
 // Two launches: png_encode_rows (one CTA per band, one warp per row: run masks, token bit offsets by warp scans,
 // bits packed in shared memory and flushed to a global staging slot per row, the piece's CRC-32 and Adler-32
-// partials), then png_assemble (one CTA per band: the chunk's place from a scan of the band sizes, the copy of its
-// pieces into the file; CTA 0 writes the header, one more CTA the last IDAT, IEND and the file length).
-// apng_assemble (rt_encode_apng_frame, rt_render_sweep_apng) takes png_assemble's place for one frame of an animated
-// PNG: the same zlib stream, framed as that frame's piece of the animation (DESIGN.md "Animated PNG").
+// partials), then the assemble kernel (one CTA per band: the chunk's place from a scan of the band sizes, the copy of
+// its pieces into the file; CTA 0 writes the header, one more CTA the last zlib chunk, IEND and the length).  Its one
+// body, assemble<ANIMATED>, is png_assemble for a PNG file and apng_assemble for one frame of an animated PNG
+// (rt_encode_apng_frame, rt_render_sweep_apng): the same zlib stream, framed as that frame's piece of the animation
+// (DESIGN.md "Animated PNG").
 #include "rt_png.h"
 
 namespace {
@@ -307,8 +308,7 @@ __global__ void __launch_bounds__(WARPS * 32) png_encode_rows(const uint8_t *__r
     }
 }
 
-// ---- apng_assemble's steps.  They are png_assemble's with the chunk framing as a parameter; png_assemble keeps its
-// own copy so that the PNG path runs exactly the machine code measured in DESIGN.md "PNG output". ---------------
+// ---- the assemble kernels' steps ------------------------------------------------------------------------------
 // The offset of CTA b's chunk (`head` bytes, then every earlier band's chunk of `framing` +
 // data bytes), and in s_rowoff the offsets of its rows' pieces within the chunk's data.
 __device__ __forceinline__ unsigned long long chunk_offset(const Scratch &sc, uint32_t height, uint32_t b,
@@ -380,102 +380,26 @@ __device__ __forceinline__ uint32_t adler_of_rows(const Scratch &sc, uint32_t wi
     return (uint32_t)((bb << 16) | a);
 }
 
-// CTA b < bands: band b's chunk; CTA `bands`: the last IDAT, IEND and the file length.
-__global__ void __launch_bounds__(WARPS * 32) png_assemble(uint32_t width, uint32_t height, Scratch sc,
-                                                             uint8_t *__restrict__ out, unsigned long long *len_word) {
-    __shared__ uint32_t s_table[256], s_x2n[32];
-    __shared__ unsigned long long s_red[WARPS], s_red2[WARPS];
-    __shared__ uint32_t s_rowoff[BAND + 1];
-    const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31u, b = blockIdx.x;
-    const uint32_t bands = (height + BAND - 1) / BAND;
-    init_crc_tables(s_table, s_x2n);
-    // this chunk's offset: the header and every earlier band's chunk
-    unsigned long long acc = 0;
-    for (uint32_t i = threadIdx.x; i < b; i += blockDim.x) acc += 12u + sc.bands[i].x;
-    for (uint32_t d = 16; d; d >>= 1) acc += __shfl_xor_sync(FULL, acc, d);
-    if (lane == 0) s_red[warp] = acc;
-    if (threadIdx.x == 0) {
-        const uint32_t rows = b < bands ? min(BAND, height - b * BAND) : 0u;
-        s_rowoff[0] = 0;
-        for (uint32_t w = 0; w < rows; w++) s_rowoff[w + 1] = s_rowoff[w] + piece_bytes(sc.rows[b * BAND + w].x);
-    }
-    __syncthreads();
-    unsigned long long off = HEADER_BYTES;
-    for (uint32_t w = 0; w < WARPS; w++) off += s_red[w];
-
-    if (b < bands) {
-        const uint32_t r = b * BAND + warp;
-        if (r < height) {
-            const uint32_t bits = sc.rows[r].x, len = piece_bytes(bits);
-            const uint8_t *staged = reinterpret_cast<const uint8_t *>(sc.stage + (size_t)r * sc.slot_words);
-            uint8_t *dst = out + off + 8 + s_rowoff[warp];
-            for (uint32_t q = lane; q < len; q += 32u) dst[q] = (uint8_t)piece_byte(staged, bits, len, q);
-        }
-        if (threadIdx.x == 0) {
-            const uint2 band = sc.bands[b];
-            put_be32(out + off, band.x);
-            out[off + 4] = 'I', out[off + 5] = 'D', out[off + 6] = 'A', out[off + 7] = 'T';
-            put_be32(out + off + 8 + band.x, band.y);
-        }
-        if (b == 0 && threadIdx.x == 0) {
-            const uint8_t sig[8] = {0x89, 'P', 'N', 'G', '\r', '\n', 0x1a, '\n'};
-            for (int k = 0; k < 8; k++) out[k] = sig[k];
-            uint8_t *ihdr = out + 8;
-            put_be32(ihdr + 8, width);
-            put_be32(ihdr + 12, height);
-            ihdr[16] = 8, ihdr[17] = 2, ihdr[18] = 0, ihdr[19] = 0, ihdr[20] = 0;
-            write_chunk(ihdr, "IHDR", 13, s_table);
-            uint8_t *zhdr = out + 33;
-            zhdr[8] = 0x78, zhdr[9] = 0x01;
-            write_chunk(zhdr, "IDAT", 2, s_table);
-        }
-        return;
-    }
-    // Adler-32 of all raw rows from the per-row partials: for row r of n bytes starting at byte r*n of N = n*h,
-    // b gains W_r + n*(h-1-r)*S_r, where S_r = sum of its bytes and W_r = sum of (n - k) * byte k
-    const uint32_t n = 1u + 3u * width, nm = n % ADLER_MOD;
-    unsigned long long sa = 0, sb = 0;
-    for (uint32_t r = threadIdx.x; r < height; r += blockDim.x) {
-        const uint4 ri = sc.rows[r];
-        const unsigned long long wgt = (unsigned long long)nm * ((height - 1u - r) % ADLER_MOD) % ADLER_MOD;
-        sa += ri.z;
-        sb += (ri.w + wgt * ri.z) % ADLER_MOD;
-    }
-    for (uint32_t d = 16; d; d >>= 1) sa += __shfl_xor_sync(FULL, sa, d), sb += __shfl_xor_sync(FULL, sb, d);
-    __syncthreads();  // s_red is reused
-    if (lane == 0) s_red[warp] = sa, s_red2[warp] = sb;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        unsigned long long a = 1, bb = (unsigned long long)n * height % ADLER_MOD;
-        for (uint32_t w = 0; w < WARPS; w++) a += s_red[w], bb += s_red2[w];
-        a %= ADLER_MOD, bb %= ADLER_MOD;
-        uint8_t *last = out + off;
-        last[8] = 0x03, last[9] = 0x00;  // BFINAL 1, BTYPE 01, end-of-block
-        put_be32(last + 10, (uint32_t)((bb << 16) | a));
-        write_chunk(last, "IDAT", 6, s_table);
-        write_chunk(last + 18, "IEND", 0, s_table);
-        *len_word = off + TRAILER_BYTES;
-    }
-}
-
-// Frame `frame` of an n_frames animation (delay = delay_num << 16 | delay_den), same grid as png_assemble.  The
-// payload is frame 0: signature, IHDR, acTL, fcTL 0, then the frame's IDAT chunks exactly as png_assemble writes them;
-// frame f >= 1: fcTL s_f, then the same C = bands + 2 chunks as fdAT, chunk k carrying sequence number s_f + 1 + k
-// before its data, where s_f = 1 + (f - 1)(C + 1).  The last frame also ends with IEND.  The animation is the payloads
-// in frame order, so no frame depends on another.
-__global__ void __launch_bounds__(WARPS * 32) apng_assemble(uint32_t width, uint32_t height, Scratch sc,
-                                                              uint32_t frame, uint32_t n_frames, uint32_t delay,
-                                                              uint8_t *__restrict__ out, unsigned long long *len_word) {
+// The file (ANIMATED = false) or frame `frame`'s payload of an n_frames animated PNG (ANIMATED, delay = delay_num << 16
+// | delay_den).  CTA b < bands: band b's chunk, CTA 0 also the header; CTA `bands`: the last zlib chunk, IEND and the
+// length.  A file is signature, IHDR, the IDAT chunks, IEND.  A payload is frame 0: signature, IHDR, acTL, fcTL 0, then
+// the frame's IDAT chunks exactly as its file has them; frame f >= 1: fcTL s_f, then the same C = bands + 2 chunks as
+// fdAT, chunk k carrying sequence number s_f + 1 + k before its data, where s_f = 1 + (f - 1)(C + 1).  The last frame
+// also ends with IEND.  The animation is the payloads in frame order, so no frame depends on another.
+template <bool ANIMATED>
+__device__ __forceinline__ void assemble(uint32_t width, uint32_t height, const Scratch &sc, uint32_t frame,
+                                         uint32_t n_frames, uint32_t delay, uint8_t *__restrict__ out,
+                                         unsigned long long *len_word) {
     __shared__ uint32_t s_table[256], s_x2n[32];
     __shared__ unsigned long long s_red[WARPS], s_red2[WARPS];
     __shared__ uint32_t s_rowoff[BAND + 1];
     const uint32_t b = blockIdx.x;
     const uint32_t bands = (height + BAND - 1) / BAND;
-    const bool first = frame == 0;
+    const bool first = !ANIMATED || frame == 0;  // the payload starts the file
     const uint32_t seq_bytes = first ? 0u : 4u;  // an fdAT's sequence number, before the data
     const uint32_t fctl_seq = first ? 0u : 1u + (frame - 1u) * (bands + 3u);
     init_crc_tables(s_table, s_x2n);
-    const uint32_t head = (first ? 8u + 25u + ACTL_BYTES : 0u) + FCTL_BYTES + 14u + seq_bytes;
+    const uint32_t head = (first ? 8u + 25u : 0u) + (ANIMATED ? (first ? ACTL_BYTES : 0u) + FCTL_BYTES : 0u) + 14u + seq_bytes;
     const unsigned long long off = chunk_offset(sc, height, b, 12u + seq_bytes, head, s_red, s_rowoff);
 
     if (b < bands) {
@@ -501,20 +425,25 @@ __global__ void __launch_bounds__(WARPS * 32) apng_assemble(uint32_t width, uint
             uint8_t *p = out;
             if (first) {
                 write_signature_ihdr(p, width, height, s_table);
-                put_be32(p + 33 + 8, n_frames);
-                put_be32(p + 33 + 12, 0u);  // num_plays 0: loop for ever
-                write_chunk(p + 33, "acTL", 8, s_table);
-                p += 33 + ACTL_BYTES;
+                p += 33;
+                if constexpr (ANIMATED) {
+                    put_be32(p + 8, n_frames);
+                    put_be32(p + 12, 0u);  // num_plays 0: loop for ever
+                    write_chunk(p, "acTL", 8, s_table);
+                    p += ACTL_BYTES;
+                }
             }
-            put_be32(p + 8, fctl_seq);
-            put_be32(p + 12, width);
-            put_be32(p + 16, height);
-            put_be32(p + 20, 0u);  // x and y offsets: every frame is full size
-            put_be32(p + 24, 0u);
-            put_be32(p + 28, delay);
-            p[32] = 0, p[33] = 0;  // dispose_op NONE, blend_op SOURCE
-            write_chunk(p, "fcTL", 26, s_table);
-            p += FCTL_BYTES;
+            if constexpr (ANIMATED) {
+                put_be32(p + 8, fctl_seq);
+                put_be32(p + 12, width);
+                put_be32(p + 16, height);
+                put_be32(p + 20, 0u);  // x and y offsets: every frame is full size
+                put_be32(p + 24, 0u);
+                put_be32(p + 28, delay);
+                p[32] = 0, p[33] = 0;  // dispose_op NONE, blend_op SOURCE
+                write_chunk(p, "fcTL", 26, s_table);
+                p += FCTL_BYTES;
+            }
             if (first) {
                 p[8] = 0x78, p[9] = 0x01;
                 write_chunk(p, "IDAT", 2, s_table);
@@ -530,13 +459,24 @@ __global__ void __launch_bounds__(WARPS * 32) apng_assemble(uint32_t width, uint
     if (threadIdx.x == 0) {
         uint8_t *last = out + off, *d = last + 8 + seq_bytes;
         if (!first) put_be32(last + 8, fctl_seq + bands + 2u);
-        d[0] = 0x03, d[1] = 0x00;
+        d[0] = 0x03, d[1] = 0x00;  // BFINAL 1, BTYPE 01, end-of-block
         put_be32(d + 2, adler);
         write_chunk(last, first ? "IDAT" : "fdAT", 6 + seq_bytes, s_table);
         unsigned long long end = off + 18 + seq_bytes;
-        if (frame + 1u == n_frames) write_chunk(out + end, "IEND", 0, s_table), end += 12;
+        if (!ANIMATED || frame + 1u == n_frames) write_chunk(out + end, "IEND", 0, s_table), end += 12;
         *len_word = end;
     }
+}
+
+__global__ void __launch_bounds__(WARPS * 32) png_assemble(uint32_t width, uint32_t height, Scratch sc,
+                                                             uint8_t *__restrict__ out, unsigned long long *len_word) {
+    assemble<false>(width, height, sc, 0, 1, 0, out, len_word);
+}
+
+__global__ void __launch_bounds__(WARPS * 32) apng_assemble(uint32_t width, uint32_t height, Scratch sc,
+                                                              uint32_t frame, uint32_t n_frames, uint32_t delay,
+                                                              uint8_t *__restrict__ out, unsigned long long *len_word) {
+    assemble<true>(width, height, sc, frame, n_frames, delay, out, len_word);
 }
 
 // The scratch block's pieces (rt_png_scratch_bytes) for a frame of layout `l`.
@@ -554,15 +494,11 @@ Scratch scratch_at(const Layout &l, void *scratch) {
 
 }  // namespace
 
-size_t rt_png_bound_bytes(uint32_t width, uint32_t height) {
+size_t rt_png_bound_bytes(uint32_t width, uint32_t height, const Animation *anim) {
     const Layout l = layout_of(width, height);
     const size_t piece = (3 + 9ull * l.n + 10 + 7) / 8 + 4;
-    return HEADER_BYTES + 12ull * l.bands + (size_t)height * piece + TRAILER_BYTES;
-}
-
-size_t rt_apng_bound_bytes(uint32_t width, uint32_t height) {
-    const Layout l = layout_of(width, height);
-    return rt_png_bound_bytes(width, height) + ACTL_BYTES + FCTL_BYTES + 4ull * (l.bands + 2);
+    const size_t png = HEADER_BYTES + 12ull * l.bands + (size_t)height * piece + TRAILER_BYTES;
+    return anim ? png + ACTL_BYTES + FCTL_BYTES + 4ull * (l.bands + 2) : png;
 }
 
 size_t rt_png_scratch_bytes(uint32_t width, uint32_t height) {
@@ -570,24 +506,18 @@ size_t rt_png_scratch_bytes(uint32_t width, uint32_t height) {
     return l.stage_bytes + l.mask_bytes + l.rows_bytes + l.bands_bytes;
 }
 
-cudaError_t rt_launch_png_encode(const uint8_t *rgba, size_t pitch, uint32_t width, uint32_t height, void *scratch,
-                                 uint8_t *out, unsigned long long *len_word, cudaStream_t stream) {
-    if (width == 0 || height == 0) return cudaErrorInvalidValue;
+cudaError_t rt_launch_png_encode(const uint8_t *rgba, size_t pitch, uint32_t width, uint32_t height, const Animation *anim,
+                                 uint32_t frame, void *scratch, uint8_t *out, unsigned long long *len_word,
+                                 cudaStream_t stream) {
+    if (width == 0 || height == 0 || (anim && frame >= anim->n_frames)) return cudaErrorInvalidValue;
     const Layout l = layout_of(width, height);
     const Scratch sc = scratch_at(l, scratch);
     png_encode_rows<<<l.bands, WARPS * 32, 0, stream>>>(rgba, pitch, width, height, sc);
-    png_assemble<<<l.bands + 1, WARPS * 32, 0, stream>>>(width, height, sc, out, len_word);
-    return cudaGetLastError();
-}
-
-cudaError_t rt_launch_apng_encode(const uint8_t *rgba, size_t pitch, uint32_t width, uint32_t height, uint32_t frame,
-                                  uint32_t n_frames, uint16_t delay_num, uint16_t delay_den, void *scratch, uint8_t *out,
-                                  unsigned long long *len_word, cudaStream_t stream) {
-    if (width == 0 || height == 0 || frame >= n_frames) return cudaErrorInvalidValue;
-    const Layout l = layout_of(width, height);
-    const Scratch sc = scratch_at(l, scratch);
-    png_encode_rows<<<l.bands, WARPS * 32, 0, stream>>>(rgba, pitch, width, height, sc);
-    apng_assemble<<<l.bands + 1, WARPS * 32, 0, stream>>>(width, height, sc, frame, n_frames,
-                                                          (uint32_t)delay_num << 16 | delay_den, out, len_word);
+    if (anim)
+        apng_assemble<<<l.bands + 1, WARPS * 32, 0, stream>>>(width, height, sc, frame, anim->n_frames,
+                                                              (uint32_t)anim->delay_num << 16 | anim->delay_den, out,
+                                                              len_word);
+    else
+        png_assemble<<<l.bands + 1, WARPS * 32, 0, stream>>>(width, height, sc, out, len_word);
     return cudaGetLastError();
 }

@@ -4,7 +4,8 @@
 
 * encode: C1..C4 frames resident on the device, 50 back-to-back rt_encode_png calls into a device buffer after
   warm-up (host clock around the calls, each of which waits for its stream), then the two encoder kernels' own
-  device time from torch.profiler in a separate pass; bytes out and GB/s of RGBA read over the kernel time.
+  device time from torch.profiler in a separate pass; bytes out and GB/s of RGBA read over the kernel time.  The same
+  profile of rt_encode_apng_frame (frame 1 of 120) gives apng_assemble's time against png_assemble's.
 * sweep: the C5 orbit (120 frames, 3840x2160, 4x4 samples, level 9) delivered end to end through
   rt_render_sweep_png and rt_render_sweep_multi(rgb=1), alternating, three rounds each, at N = 1 and at N = 2 and 8
   GPUs when the box has them.  The callback keeps each frame's length and a CRC of its first KB, never a full hash.
@@ -38,8 +39,8 @@ def encode_case(name, w, h, spp, level, iters):
     L = rt.lib()
     scene = rt.Scene(level=level)
     frame = rt.device_alloc(w * h * 4)
-    cap = rt.png_bound(w, h)
-    out = rt.device_alloc(cap)
+    cap, apng_cap = rt.png_bound(w, h), rt.apng_bound(w, h, 120)
+    out = rt.device_alloc(apng_cap)
     n = C.c_size_t()
     try:
         rt.Renderer.render(rt.RenderOptions(w, h, spp), scene, out_ptr=frame, want_stats=True)
@@ -55,11 +56,22 @@ def encode_case(name, w, h, spp, level, iters):
             one()
         call_ms = (time.perf_counter() - t0) * 1e3 / iters
         kernel_us = profile_kernels(one, iters)
+        bytes_out = n.value
+
+        def one_apng():
+            rc = L.rt_encode_apng_frame(C.c_void_p(frame), w, h, 0, 1, 120, 1, 24, C.c_void_p(out), apng_cap, C.byref(n),
+                                        None)
+            if rc != rt.RT_OK:
+                raise rt.RtError(rc, L.rt_last_error().decode())
+        for _ in range(5):
+            one_apng()
+        apng_kernel_us = profile_kernels(one_apng, iters)
         rgba = w * h * 4
         return {"case": name, "width": w, "height": h, "spp": spp, "level": level, "iters": iters,
-                "bytes_out": n.value, "rgb_bytes": w * h * 3, "ratio": round(w * h * 3 / n.value, 2),
+                "bytes_out": bytes_out, "rgb_bytes": w * h * 3, "ratio": round(w * h * 3 / bytes_out, 2),
                 "call_ms": round(call_ms, 4), "kernel_us": {k: round(v, 2) for k, v in kernel_us.items()},
                 "kernel_total_us": round(sum(kernel_us.values()), 2),
+                "apng_frame_kernel_us": {k: round(v, 2) for k, v in apng_kernel_us.items()},
                 "rgba_read_gb_per_s": round(rgba / (sum(kernel_us.values()) * 1e-6) / 1e9, 1)}
     finally:
         rt.device_free(frame)
@@ -77,9 +89,10 @@ def profile_kernels(fn, iters):
         torch.cuda.synchronize()
     tot = {}
     for e in prof.events():
-        for k in ("png_encode_rows", "png_assemble"):
+        for k in ("png_encode_rows", "apng_assemble", "png_assemble"):
             if k in e.name and e.device_type.name == "CUDA":
                 tot[k] = tot.get(k, 0.0) + e.device_time
+                break
     return {k: v / iters for k, v in tot.items()}
 
 
