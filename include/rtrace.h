@@ -325,7 +325,10 @@ void rt_host_free(void *p);
 /* RGBA8 -> RGB8 on the device for the row blocks one GPU owns (blocks of row_block rows at image rows row_start +
  * k * row_stride) of a frame-shaped RGBA buffer, into the same rows of a frame-shaped RGB buffer (width*3 bytes per
  * row): the sink drops alpha anyway (render.rs:389-397), so a rank packs before it copies its blocks out and a
- * quarter of the PCIe traffic is saved.  Both buffers live on the current device; asynchronous on `stream`. */
+ * quarter of the PCIe traffic is saved.  Rows from `height` on are left untouched.  Asynchronous on `stream`.
+ * RT_ERR_INVALID unless both buffers are device memory of the current device, width and height are in 1..65535,
+ * 0 < row_block <= row_stride, row_start * width and row_stride * width are multiples of 4 pixels, rgba_frame is
+ * 16-byte aligned and rgb_frame 4-byte aligned.  row_start >= height packs nothing and succeeds. */
 int rt_pack_rgb_rows(const uint8_t *rgba_frame, uint8_t *rgb_frame, uint32_t width, uint32_t height,
                      uint32_t row_start, uint32_t row_stride, uint32_t row_block, void *stream);
 /* Page-lock host memory the caller already owns (e.g. a frame in a shared-memory segment that several

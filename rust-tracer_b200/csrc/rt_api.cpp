@@ -1427,6 +1427,15 @@ int rt_memcpy2d_async(void *dst, size_t dpitch, const void *src, size_t spitch, 
 int rt_pack_rgb_rows(const uint8_t *rgba_frame, uint8_t *rgb_frame, uint32_t width, uint32_t height, uint32_t row_start,
                      uint32_t row_stride, uint32_t row_block, void *stream) {
     if (!rgba_frame || !rgb_frame) return fail(RT_ERR_INVALID, "NULL argument");
+    // height is also the grid's y extent at row_stride 1, whose limit is 65535
+    if (width == 0 || height == 0 || width > 65535u || height > 65535u)
+        return fail(RT_ERR_INVALID, "width/height must be in 1..65535 (got %u x %u)", width, height);
+    int in_dev = -1, out_dev = -1, cur = -1;
+    if (!is_device_ptr(rgba_frame, &in_dev) || !is_device_ptr(rgb_frame, &out_dev))
+        return fail(RT_ERR_INVALID, "rgba_frame and rgb_frame must be device memory");
+    CUDA_TRY(cudaGetDevice(&cur));
+    if (in_dev != cur || out_dev != cur)
+        return fail(RT_ERR_INVALID, "rgba_frame (device %d) and rgb_frame (device %d) must live on the current device %d", in_dev, out_dev, cur);
     if (row_block == 0 || row_stride < row_block) return fail(RT_ERR_INVALID, "row_stride %u is smaller than the row block %u", row_stride, row_block);
     if (((uint64_t)row_start * width) % 4 || ((uint64_t)row_stride * width) % 4)
         return fail(RT_ERR_INVALID, "row blocks must start at multiples of 4 pixels (row_start %u, row_stride %u, width %u)", row_start, row_stride, width);
