@@ -200,6 +200,27 @@ int rt_render_frame_multi(rt_scene *const *scenes, int ngpu, const rt_camera *ca
                           uint32_t width, uint32_t height, uint32_t spp,
                           uint8_t *rgba_out, size_t rgba_len, rt_stats *stats);
 
+/* ---- float output ----------------------------------------------------------------------------------------------
+ * The pixel before quantisation: four f32 per pixel {r, g, b, alpha}, 16 bytes, the sums of the spp*spp samples
+ * times 1/(spp*spp) (render.rs:249-250), equal bit for bit to the reference's values.  Blue equals green.
+ * Quantising each component with trunc(0.5 + 255 v), saturating to 0..255 (NaN -> 0), gives exactly the RGBA8
+ * bytes of rt_render_rows (render.rs:96-103).  Float frames are rendered by the PHASED variant (where AUTO would
+ * run TILE or PHASED, and for a forced TILE or PHASED) or by LANE (a forced LANE or WARP, and every argument
+ * outside PHASED's domain); stats->variant_used says which.  A device output pointer must be 16-byte aligned and
+ * a pitch a multiple of 16, else RT_ERR_INVALID. */
+/* rt_render_rows with float output and no kinds_out: rows row_start, row_start+row_stride, ... (row_count of
+ * them), pitch in bytes (0 = width*16).  With a device output pointer the call is asynchronous on `stream`
+ * (e.g. straight into a torch CUDA tensor on torch's current stream). */
+int rt_render_rows_f32(const rt_scene *s, const rt_camera *camera,
+                       uint32_t width, uint32_t height, uint32_t spp,
+                       uint32_t row_start, uint32_t row_stride, uint32_t row_count,
+                       float *rgba_out, size_t pitch_bytes, void *stream, rt_stats *stats);
+/* rt_render_frame_multi with float output: rgba_out holds width*height*16 bytes (RT_ERR_BUFFER when rgba_bytes
+ * is less), in host memory or in device memory of scenes[0]'s GPU; ngpu == 1 is a single-GPU frame. */
+int rt_render_frame_multi_f32(rt_scene *const *scenes, int ngpu, const rt_camera *camera,
+                              uint32_t width, uint32_t height, uint32_t spp,
+                              float *rgba_out, size_t rgba_bytes, rt_stats *stats);
+
 /* The same sweep with the frames PULLED instead of listed: whenever the pipeline has room for another frame the
  * library calls `next(next_user, &camera, &use_camera)`, which fills the camera (or sets *use_camera = 0 for the
  * reference camera; it is 1 on entry) and returns the frame's id (>= 0; handed back to `cb` as its frame argument)

@@ -331,12 +331,16 @@ bool within_analysed_range(const rt::RenderParams &p) {
     return m <= 16.0f && p.scene_radius > 0.0f;
 }
 
+// what the candidate-list variants need beyond their template ranges (rt_tile_supported: spp <= 4,
+// rt_phased_supported: spp <= 8; both: regular pyramid of level <= 10)
+bool geometry_ok(const rt::RenderParams &p) {
+    return (!p.has_basis || orthonormal(p.basis)) && eye_outside_root_bound(p) && within_analysed_range(p);
+}
+
 int kernel_variant(const rt::RenderParams &p) {
     if (p.col_count) return g_variant == RT_VARIANT_WARP ? RT_KERNEL_WARP : RT_KERNEL_LANE;  // bucket-sized window
-    // what the candidate-list variants need beyond their template ranges (rt_tile_supported: spp <= 4,
-    // rt_phased_supported: spp <= 8; both: regular pyramid of level <= 10)
-    const bool geometry_ok = (!p.has_basis || orthonormal(p.basis)) && eye_outside_root_bound(p) && within_analysed_range(p);
-    const bool tile_ok = rt_tile_supported(p) && geometry_ok, phased_ok = rt_phased_supported(p) && geometry_ok;
+    const bool geo_ok = geometry_ok(p);
+    const bool tile_ok = rt_tile_supported(p) && geo_ok, phased_ok = rt_phased_supported(p) && geo_ok;
     switch (g_variant) {
         case RT_VARIANT_LANE:
             return RT_KERNEL_LANE;
@@ -363,6 +367,22 @@ int kernel_variant(const rt::RenderParams &p) {
     if (leaf_px < 1.5f) return RT_KERNEL_LANE;
     const uint64_t pixel_tiles = (uint64_t)p.width * p.row_count / (p.spp == 1 ? 128u : 32u);  // one warp each
     return (pixel_tiles < 8000 && tile_ok) ? RT_KERNEL_TILE : RT_KERNEL_PHASED;
+}
+
+// Float frames have PHASED and LANE kernels only: PHASED wherever RGBA8 would run TILE or PHASED (PHASED is
+// correct at every size) and for a forced TILE or PHASED inside PHASED's domain; LANE for everything else,
+// including a forced LANE or WARP.
+int kernel_variant_f32(const rt::RenderParams &p) {
+    switch (g_variant) {
+        case RT_VARIANT_LANE:
+        case RT_VARIANT_WARP:
+            return RT_KERNEL_LANE;
+        case RT_VARIANT_TILE:
+        case RT_VARIANT_PHASED:
+            return rt_phased_supported(p) && geometry_ok(p) ? RT_KERNEL_PHASED : RT_KERNEL_LANE;
+        default:
+            return kernel_variant(p) == RT_KERNEL_LANE ? RT_KERNEL_LANE : RT_KERNEL_PHASED;
+    }
 }
 
 // RTRACE_TILE_SHAPE (kernel experiments): the tile shape forced on the TILE and PHASED variants, -1 when unset
@@ -399,20 +419,20 @@ int prepare_phased(rt_scene *s, rt::RenderParams &p, cudaStream_t stream, int sh
 
 // Launches the kernel(s) of one frame on `stream`; *variant receives the kernel that renders it (RT_KERNEL_*,
 // numbered like RT_VARIANT_*).
-int launch(rt_scene *s, rt::RenderParams &p, bool diag, cudaStream_t stream, int *variant) {
-    const int v = kernel_variant(p), shape = forced_tile_shape();
+int launch(rt_scene *s, rt::RenderParams &p, bool diag, cudaStream_t stream, int *variant, RtPixels fmt = RT_PIXELS_RGBA8) {
+    const int v = fmt == RT_PIXELS_F32 ? kernel_variant_f32(p) : kernel_variant(p), shape = forced_tile_shape();
     *variant = v;
     cudaError_t e;
     if (v == RT_KERNEL_PHASED) {
         const int phased_shape = std::max(shape, 0);
         RT_TRY(prepare_phased(s, p, stream, phased_shape));
-        e = rt_launch_render_phased(diag, p, stream, phased_shape);
+        e = rt_launch_render_phased(diag, fmt, p, stream, phased_shape);
     } else if (v == RT_KERNEL_TILE) {
         // AUTO picks the fused kernel only for small frames, where one independent warp per tile
         // (shape 2) beats CTA-shared culls (warps waiting at barriers with too few CTAs to cover them)
         e = rt_launch_render_tile(diag, p, stream, shape >= 0 ? shape : (g_variant == RT_VARIANT_AUTO ? 2 : 0));
     } else {
-        e = rt_launch_render(v, diag, p, stream);
+        e = rt_launch_render(v, diag, fmt, p, stream);
     }
     if (e != cudaSuccess) return fail(RT_ERR_CUDA, "kernel launch: %s", cudaGetErrorString(e));
     return RT_OK;
@@ -592,7 +612,7 @@ static int render_rows_impl(rt_scene *s, const rt_camera *camera, uint32_t width
                             uint32_t row_start, uint32_t row_stride, uint32_t row_count, uint8_t *rgba_out,
                             size_t pitch_bytes, uint8_t *kinds_out, cudaStream_t stream, rt_stats *stats,
                             uint64_t *count_hits, uint64_t *count_shadow, uint32_t col_start = 0,
-                            uint32_t col_count = 0, RowLayout layout = RowLayout()) {
+                            uint32_t col_count = 0, RowLayout layout = RowLayout(), RtPixels fmt = RT_PIXELS_RGBA8) {
     int rc = check_frame_args(s, width, height, spp, row_start, row_stride, row_count, layout);
     if (rc != RT_OK) return rc;
     const bool counting = count_shadow != nullptr;
@@ -600,9 +620,10 @@ static int render_rows_impl(rt_scene *s, const rt_camera *camera, uint32_t width
     // col_count > 0: only columns col_start .. col_start + col_count - 1, packed from byte 0 of each output row
     if ((uint64_t)col_start + col_count > width) return fail(RT_ERR_INVALID, "columns %u..%u leave the %u-pixel row", col_start, col_start + col_count, width);
     const uint32_t cols = col_count ? col_count : width;
-    const size_t row_bytes = (size_t)cols * 4;
+    const size_t bpp = fmt == RT_PIXELS_F32 ? 16 : 4;  // bytes per pixel; pitches and device pointers are multiples of it
+    const size_t row_bytes = (size_t)cols * bpp;
     if (pitch_bytes == 0) pitch_bytes = row_bytes;
-    if (pitch_bytes < row_bytes || (pitch_bytes & 3)) return fail(RT_ERR_INVALID, "pitch %zu too small or not a multiple of 4", pitch_bytes);
+    if (pitch_bytes < row_bytes || (pitch_bytes & (bpp - 1))) return fail(RT_ERR_INVALID, "pitch %zu too small or not a multiple of %zu", pitch_bytes, bpp);
     if (stats) memset(stats, 0, sizeof(*stats));
     if (row_count == 0) return RT_OK;
 
@@ -618,7 +639,7 @@ static int render_rows_impl(rt_scene *s, const rt_camera *camera, uint32_t width
         RT_TRY(enable_peer(s->device, out_dev, &can));
         if (!can) return fail(RT_ERR_INVALID, "rgba_out lives on device %d, which device %d cannot access", out_dev, s->device);
     }
-    if (out_on_device && (((uintptr_t)rgba_out) & 3)) return fail(RT_ERR_INVALID, "device rgba_out must be 4-byte aligned");
+    if (out_on_device && (((uintptr_t)rgba_out) & (bpp - 1))) return fail(RT_ERR_INVALID, "device rgba_out must be %zu-byte aligned", bpp);
     int kinds_dev = -1;
     const bool kinds_on_device = kinds_out && is_device_ptr(kinds_out, &kinds_dev);
     const size_t kinds_bytes = (size_t)cols * row_count * spp * spp;
@@ -658,7 +679,7 @@ static int render_rows_impl(rt_scene *s, const rt_camera *camera, uint32_t width
 
     if (stats) CUDA_TRY(cudaEventRecord(s->ev0, stream));
     int variant = 0;
-    RT_TRY(launch(s, p, diag, stream, &variant));
+    RT_TRY(launch(s, p, diag, stream, &variant, fmt));
     if (stats) CUDA_TRY(cudaEventRecord(s->ev1, stream));
 
     bool must_sync = false;
@@ -704,6 +725,15 @@ int rt_render_rows(const rt_scene *s, const rt_camera *camera, uint32_t width, u
                    uint8_t *kinds_out, void *stream, rt_stats *stats) {
     return render_rows_impl(const_cast<rt_scene *>(s), camera, width, height, spp, row_start, row_stride, row_count,
                             rgba_out, pitch_bytes, kinds_out, (cudaStream_t)stream, stats, nullptr, nullptr);
+}
+
+int rt_render_rows_f32(const rt_scene *s, const rt_camera *camera, uint32_t width, uint32_t height, uint32_t spp,
+                       uint32_t row_start, uint32_t row_stride, uint32_t row_count, float *rgba_out, size_t pitch_bytes,
+                       void *stream, rt_stats *stats) {
+    if (!rgba_out) return fail(RT_ERR_INVALID, "rgba_out is NULL");
+    return render_rows_impl(const_cast<rt_scene *>(s), camera, width, height, spp, row_start, row_stride, row_count,
+                            reinterpret_cast<uint8_t *>(rgba_out), pitch_bytes, nullptr, (cudaStream_t)stream, stats,
+                            nullptr, nullptr, 0, 0, RowLayout(), RT_PIXELS_F32);
 }
 
 int rt_render_row_blocks(const rt_scene *s, const rt_camera *camera, uint32_t width, uint32_t height, uint32_t spp,
@@ -970,9 +1000,10 @@ int rt_render_sweep_pull(const rt_scene *s, rt_next_frame_callback next, void *n
 //    pixels straight into that frame through peer memory over NVLink -- the stores are the gather.  Without
 //    peer access GPU g renders rows g, g+G, ... into a band of its own and a strided peer copy de-interleaves it.
 static int frame_multi_locked(rt_scene *const *scenes, int ngpu, const rt_camera *camera, uint32_t width, uint32_t height,
-                              uint32_t spp, uint8_t *rgba_out, rt_stats *stats, std::vector<char> &launched) {
+                              uint32_t spp, uint8_t *rgba_out, rt_stats *stats, std::vector<char> &launched,
+                              RtPixels fmt) {
     const double t0 = now_ms();
-    const size_t row_bytes = (size_t)width * 4;
+    const size_t row_bytes = (size_t)width * (fmt == RT_PIXELS_F32 ? 16 : 4);
     rt_scene *root = scenes[0];
     int out_dev = -1;
     const bool to_device = is_device_ptr(rgba_out, &out_dev);
@@ -1015,7 +1046,7 @@ static int frame_multi_locked(rt_scene *const *scenes, int ngpu, const rt_camera
         if (stats) CUDA_TRY(cudaEventRecord(s->ev0, s->own_stream));
         launched[(size_t)g] = 1;  // from here on this GPU may have work in flight
         int variant = 0;
-        RT_TRY(launch(s, p, false, s->own_stream, &variant));
+        RT_TRY(launch(s, p, false, s->own_stream, &variant, fmt));
         launches += launches_of(variant);
         if (g == 0) used = (uint32_t)variant;
         if (stats) CUDA_TRY(cudaEventRecord(s->ev1, s->own_stream));
@@ -1061,23 +1092,29 @@ static int lock_scenes(rt_scene *const *scenes, int ngpu, std::vector<std::uniqu
     return RT_OK;
 }
 
-int rt_render_frame_multi(rt_scene *const *scenes, int ngpu, const rt_camera *camera, uint32_t width, uint32_t height,
-                          uint32_t spp, uint8_t *rgba_out, size_t rgba_len, rt_stats *stats) {
+// rt_render_frame_multi and rt_render_frame_multi_f32: the frame at 4 or 16 bytes per pixel.
+static int frame_multi_impl(rt_scene *const *scenes, int ngpu, const rt_camera *camera, uint32_t width, uint32_t height,
+                            uint32_t spp, uint8_t *rgba_out, size_t rgba_len, rt_stats *stats, RtPixels fmt) {
     if (!scenes || ngpu < 1) return fail(RT_ERR_INVALID, "need at least one scene");
     if (!rgba_out) return fail(RT_ERR_INVALID, "rgba_out is NULL");
-    if (rgba_len < (size_t)width * height * 4) return fail(RT_ERR_BUFFER, "rgba_out holds %zu bytes, frame needs %zu", rgba_len, (size_t)width * height * 4);
+    const size_t bpp = fmt == RT_PIXELS_F32 ? 16 : 4, frame_bytes = (size_t)width * height * bpp;
+    if (rgba_len < frame_bytes) return fail(RT_ERR_BUFFER, "rgba_out holds %zu bytes, frame needs %zu", rgba_len, frame_bytes);
     for (int g = 0; g < ngpu; g++) {
         int rc = check_frame_args(scenes[g], width, height, spp, 0, 1, height);
         if (rc != RT_OK) return rc;
     }
     if (stats) memset(stats, 0, sizeof(*stats));
-    if (ngpu == 1) return rt_render_frame(scenes[0], camera, width, height, spp, rgba_out, rgba_len, stats);
+    if (ngpu == 1)
+        return render_rows_impl(scenes[0], camera, width, height, spp, 0, 1, height, rgba_out, 0, nullptr, nullptr,
+                                stats, nullptr, nullptr, 0, 0, RowLayout(), fmt);
+    if (fmt == RT_PIXELS_F32 && is_device_ptr(rgba_out, nullptr) && ((uintptr_t)rgba_out & 15))
+        return fail(RT_ERR_INVALID, "device rgba_out must be 16-byte aligned");
 
     std::vector<std::unique_lock<std::mutex>> locks;
     int rc = lock_scenes(scenes, ngpu, locks);
     if (rc != RT_OK) return rc;
     std::vector<char> launched((size_t)ngpu, 0);  // GPUs whose share of the rows is not empty
-    rc = frame_multi_locked(scenes, ngpu, camera, width, height, spp, rgba_out, stats, launched);
+    rc = frame_multi_locked(scenes, ngpu, camera, width, height, spp, rgba_out, stats, launched, fmt);
     if (rc != RT_OK) {
         // Kernels already launched on other GPUs may still be storing into GPU 0's frame through peer memory:
         // drain every GPU before the locks are released (a later call may free or reuse that frame).  Keeps
@@ -1090,6 +1127,17 @@ int rt_render_frame_multi(rt_scene *const *scenes, int ngpu, const rt_camera *ca
         cudaGetLastError();
     }
     return rc;
+}
+
+int rt_render_frame_multi(rt_scene *const *scenes, int ngpu, const rt_camera *camera, uint32_t width, uint32_t height,
+                          uint32_t spp, uint8_t *rgba_out, size_t rgba_len, rt_stats *stats) {
+    return frame_multi_impl(scenes, ngpu, camera, width, height, spp, rgba_out, rgba_len, stats, RT_PIXELS_RGBA8);
+}
+
+int rt_render_frame_multi_f32(rt_scene *const *scenes, int ngpu, const rt_camera *camera, uint32_t width, uint32_t height,
+                              uint32_t spp, float *rgba_out, size_t rgba_bytes, rt_stats *stats) {
+    return frame_multi_impl(scenes, ngpu, camera, width, height, spp, reinterpret_cast<uint8_t *>(rgba_out), rgba_bytes,
+                            stats, RT_PIXELS_F32);
 }
 
 // ---------------------------------------------------------------------------

@@ -71,12 +71,14 @@ RT_DEV void warp_traverse(const float4 *__restrict__ sph, const uint32_t *__rest
 }
 
 // ---------------------------------------------------------------------------
-// The fused pixel kernel.
+// The fused pixel kernel.  F32: the pixel is stored as the float4 {r, g, b, alpha} that RGBA8 output quantises.
+// `tid` is threadIdx.x read in the __global__ function: there the compiler knows its range from the launch bounds,
+// in a device function it does not, and the RGBA8 kernels would lose instructions that depend on it.
 // ---------------------------------------------------------------------------
-template <int VARIANT, bool DIAG, bool PREVIEW = false>
-__global__ void __launch_bounds__(BLOCK_THREADS) render_kernel(const RenderParams p) {
-    const int lane = threadIdx.x & 31;
-    const int warp = threadIdx.x >> 5;
+template <int VARIANT, bool DIAG, bool PREVIEW, bool F32>
+__device__ __forceinline__ void render_body(const RenderParams &p, const uint32_t tid) {
+    const int lane = tid & 31;
+    const int warp = tid >> 5;
     const uint32_t lx = blockIdx.x * (TILE_W * WARPS_X) + (warp % WARPS_X) * TILE_W + (lane % TILE_W);
     const uint32_t j = blockIdx.y * (TILE_H * WARPS_Y) + (warp / WARPS_X) * TILE_H + (lane / TILE_W);
     const uint32_t cols = p.col_count ? p.col_count : p.width;  // column window (render_region buckets)
@@ -154,6 +156,10 @@ __global__ void __launch_bounds__(BLOCK_THREADS) render_kernel(const RenderParam
         float recip = frecip(fmul((float)p.spp, (float)p.spp));  // render.rs:219-220
         c = vmulf(c, recip);
         alpha = fmul(alpha, recip);
+        if constexpr (F32) {
+            *reinterpret_cast<float4 *>(p.out + (size_t)out_row(p, j) * p.pitch + (size_t)lx * 16) = make_float4(c.x, c.y, c.z, alpha);
+            return;
+        }
         uint32_t px = scale_u8(c.x) | (scale_u8(c.y) << 8) | (scale_u8(c.z) << 16) | (scale_u8(alpha) << 24);
         if (PREVIEW) {  // the block's pixels that lie inside the image, each row of the block contiguous
             const uint32_t x1 = min(x + step, p.width), y1 = min(y + step, p.height);
@@ -182,6 +188,16 @@ __global__ void __launch_bounds__(BLOCK_THREADS) render_kernel(const RenderParam
             }
         }
     }
+}
+
+template <int VARIANT, bool DIAG, bool PREVIEW = false>
+__global__ void __launch_bounds__(BLOCK_THREADS) render_kernel(const RenderParams p) {
+    render_body<VARIANT, DIAG, PREVIEW, false>(p, threadIdx.x);
+}
+
+// LANE with float output: the fallback of float frames outside PHASED's domain.
+__global__ void __launch_bounds__(BLOCK_THREADS) render_lane_f32_kernel(const RenderParams p) {
+    render_body<RT_KERNEL_LANE, false, false, true>(p, threadIdx.x);
 }
 
 // Closest-hit traversal of arbitrary rays (rt_trace_rays): group.rs:72-83 from Hit::missed().
@@ -296,13 +312,15 @@ __global__ void __launch_bounds__(256) fp32_peak_kernel(float *out, int iters, f
 // ---------------------------------------------------------------------------
 using namespace rt;
 
-cudaError_t rt_launch_render(int variant, bool diag, const RenderParams &p, cudaStream_t stream) {
+cudaError_t rt_launch_render(int variant, bool diag, RtPixels fmt, const RenderParams &p, cudaStream_t stream) {
     dim3 block(BLOCK_THREADS);
     const uint32_t cols = p.col_count ? p.col_count : p.width;
     dim3 grid((cols + TILE_W * WARPS_X - 1) / (TILE_W * WARPS_X),
               (p.row_count + TILE_H * WARPS_Y - 1) / (TILE_H * WARPS_Y));
     if (grid.x == 0 || grid.y == 0) return cudaSuccess;
-    if (variant == RT_KERNEL_LANE) {
+    if (fmt == RT_PIXELS_F32) {
+        render_lane_f32_kernel<<<grid, block, 0, stream>>>(p);
+    } else if (variant == RT_KERNEL_LANE) {
         if (diag)
             render_kernel<RT_KERNEL_LANE, true><<<grid, block, 0, stream>>>(p);
         else

@@ -542,12 +542,15 @@ __global__ void __launch_bounds__(32 * P_WARPS) phase_cull_shadow(const RenderPa
 // ---------------------------------------------------------------------------
 // K4: shading, shadow tests, accumulation, store; one warp per pixel tile
 // ---------------------------------------------------------------------------
-template <int SPP, int PXW, int PXH, int CW, int CH, bool DIAG>
-__global__ void __launch_bounds__(32 * CW * CH, phased_min_blocks(CW * CH)) phase_shade_store(const RenderParams p) {
+// F32: each pixel is stored as the float4 {r, g, b, alpha} that RGBA8 output quantises (16 bytes at x * 16 of its
+// row) instead of those four bytes.  Everything before the store is the same code.  `tid` is threadIdx.x read in the
+// __global__ function, where the compiler knows its range from the launch bounds (render_body, rt_kernels.cu).
+template <int SPP, int PXW, int PXH, int CW, int CH, bool DIAG, bool F32>
+__device__ __forceinline__ void shade_store_body(const RenderParams &p, const uint32_t tid) {
     using G = Geo<SPP, PXW, PXH, CW, CH>;
     constexpr int S = G::S, NS = G::NS;
     __shared__ uint4 stage[1 + SU * T_CAND];  // the cull tile's first shadow-candidate chunk
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int lane = tid & 31, warp = tid >> 5;
     const G geo(p.width, p.row_count);
     // one block per cull tile, one warp per pixel tile of it
     const uint32_t ct = blockIdx.y * geo.ctiles_x + blockIdx.x;  // 2-D grid of cull tiles: no division
@@ -576,7 +579,7 @@ __global__ void __launch_bounds__(32 * CW * CH, phased_min_blocks(CW * CH)) phas
     const bool staged = head < COVERED;
     if (staged) {  // stage the first chunk (almost always the only one) in shared memory, asynchronously
         const uint32_t units = 1u + SU * __ldg(&p.pool[head]).x;
-        for (uint32_t u = threadIdx.x; u < units; u += blockDim.x) {
+        for (uint32_t u = tid; u < units; u += blockDim.x) {
             if (LAZY) stage_async(&stage[u], &p.pool[head + u]);
             else stage[u] = __ldg(&p.pool[head + u]);
         }
@@ -595,6 +598,16 @@ __global__ void __launch_bounds__(32 * CW * CH, phased_min_blocks(CW * CH)) phas
         // no ray of this cull tile hit anything: every sample adds BACKGROUND (render.rs:190-193)
         if (lane_in) {
             for (int smp = 0; smp < NS; smp++) cr = fadd(cr, BG_R), cg = fadd(cg, BG_G);
+            if constexpr (F32) {
+                const float4 v = make_float4(fmul(cr, recip), fmul(cg, recip), fmul(cg, recip), fmul(0.0f, recip));
+                for (int pi = 0; pi < G::NPX; pi++) {
+                    uint32_t x, j;
+                    slot_pixel<PXW, PXH>(tile_x0, tile_j0, lane, pi, x, j);
+                    if (x < p.width && j < p.row_count)
+                        *reinterpret_cast<float4 *>(p.out + (size_t)out_row(p, j) * p.pitch + (size_t)x * 16) = v;
+                }
+                return;
+            }
             const uint32_t g8 = scale_u8_fast(fmul(cg, recip));
             const uint32_t px = scale_u8_fast(fmul(cr, recip)) | (g8 << 8) | (g8 << 16) | (scale_u8_fast(fmul(0.0f, recip)) << 24);
             for (int pi = 0; pi < G::NPX; pi++) {
@@ -824,6 +837,14 @@ __global__ void __launch_bounds__(32 * CW * CH, phased_min_blocks(CW * CH)) phas
                         // render.rs:249-250: * 1/(spp*spp); for one sample that factor is exactly 1.0f and x * 1 == x
                         const float qr = NS == 1 ? cr : fmul(cr, recip), qg = NS == 1 ? cg : fmul(cg, recip);
                         const float al = NS == 1 ? alpha : fmul(alpha, recip);
+                        // Floats are stored as the pixel completes (a pair of them would be two 16-byte stores anyway);
+                        // px_ok stays false, so the RGBA8 stores below store nothing.
+                        if constexpr (F32) {
+                            if (inside)
+                                *reinterpret_cast<float4 *>(p.out + (size_t)out_row(p, j) * p.pitch + (size_t)x * 16) =
+                                    make_float4(qr, qg, qg, al);
+                            continue;
+                        }
                         const uint32_t g8 = scale_u8_fast(qg);
                         // one sample: alpha is exactly 0 or 1, and trunc(0.5 + 255 * 1) = 255
                         const uint32_t a8 = NS == 1 ? (al != 0.0f ? 255u : 0u) : scale_u8_fast(al);
@@ -861,12 +882,22 @@ __global__ void __launch_bounds__(32 * CW * CH, phased_min_blocks(CW * CH)) phas
     }
 }
 
+template <int SPP, int PXW, int PXH, int CW, int CH, bool DIAG>
+__global__ void __launch_bounds__(32 * CW * CH, phased_min_blocks(CW * CH)) phase_shade_store(const RenderParams p) {
+    shade_store_body<SPP, PXW, PXH, CW, CH, DIAG, false>(p, threadIdx.x);
+}
+
+template <int SPP, int PXW, int PXH, int CW, int CH>
+__global__ void __launch_bounds__(32 * CW * CH, phased_min_blocks(CW * CH)) phase_shade_store_f32(const RenderParams p) {
+    shade_store_body<SPP, PXW, PXH, CW, CH, false, true>(p, threadIdx.x);
+}
+
 }  // namespace rt
 
 using namespace rt;
 
 template <int SPP, int PXW, int PXH, int CW, int CH>
-static cudaError_t launch_phased(bool diag, const RenderParams &p, cudaStream_t stream) {
+static cudaError_t launch_phased(bool diag, RtPixels fmt, const RenderParams &p, cudaStream_t stream) {
     using G = Geo<SPP, PXW, PXH, CW, CH>;
     const G geo(p.width, p.row_count);
     const uint32_t nc = geo.n_ctiles(), np = geo.n_ptiles();
@@ -883,7 +914,9 @@ static cudaError_t launch_phased(bool diag, const RenderParams &p, cudaStream_t 
     }
     phase_test_primary<SPP, PXW, PXH, CW, CH><<<tiles2d, 32 * CW * CH, 0, stream>>>(p);
     phase_cull_shadow<SPP, PXW, PXH, CW, CH><<<cb, 32 * P_WARPS, 0, stream>>>(p);
-    if (diag)
+    if (fmt == RT_PIXELS_F32)
+        phase_shade_store_f32<SPP, PXW, PXH, CW, CH><<<tiles2d, 32 * CW * CH, 0, stream>>>(p);
+    else if (diag)
         phase_shade_store<SPP, PXW, PXH, CW, CH, true><<<tiles2d, 32 * CW * CH, 0, stream>>>(p);
     else
         phase_shade_store<SPP, PXW, PXH, CW, CH, false><<<tiles2d, 32 * CW * CH, 0, stream>>>(p);
@@ -936,31 +969,31 @@ void rt_phased_scratch(uint32_t width, uint32_t rows, uint32_t spp, int shape, s
     *pool_units = (uint32_t)units;
 }
 
-cudaError_t rt_launch_render_phased(bool diag, const RenderParams &p, cudaStream_t stream, int shape) {
+cudaError_t rt_launch_render_phased(bool diag, RtPixels fmt, const RenderParams &p, cudaStream_t stream, int shape) {
     // shape 0: cull tile = 2x2 pixel tiles; shape 1: 4x4 pixel tiles
     switch (p.spp) {
         case 1:
-            if (shape == 5) return launch_phased<1, 2, 2, 4, 2>(diag, p, stream);  // 64x16 cull tile
-            if (shape == 6) return launch_phased<1, 2, 2, 2, 4>(diag, p, stream);  // 32x32 cull tile
-            if (shape == 2) return launch_phased<1, 4, 2, 1, 2>(diag, p, stream);  // 8 pixels per lane
-            if (shape == 3) return launch_phased<1, 2, 1, 2, 4>(diag, p, stream);  // 2 pixels per lane, 32x16 cull tile
-            if (shape == 4) return launch_phased<1, 2, 1, 1, 2>(diag, p, stream);  // 2 pixels per lane, 16x8 cull tile
-            return shape == 1 ? launch_phased<1, 2, 2, 4, 4>(diag, p, stream) : launch_phased<1, 2, 2, 2, 2>(diag, p, stream);
+            if (shape == 5) return launch_phased<1, 2, 2, 4, 2>(diag, fmt, p, stream);  // 64x16 cull tile
+            if (shape == 6) return launch_phased<1, 2, 2, 2, 4>(diag, fmt, p, stream);  // 32x32 cull tile
+            if (shape == 2) return launch_phased<1, 4, 2, 1, 2>(diag, fmt, p, stream);  // 8 pixels per lane
+            if (shape == 3) return launch_phased<1, 2, 1, 2, 4>(diag, fmt, p, stream);  // 2 pixels per lane, 32x16 cull tile
+            if (shape == 4) return launch_phased<1, 2, 1, 1, 2>(diag, fmt, p, stream);  // 2 pixels per lane, 16x8 cull tile
+            return shape == 1 ? launch_phased<1, 2, 2, 4, 4>(diag, fmt, p, stream) : launch_phased<1, 2, 2, 2, 2>(diag, fmt, p, stream);
         case 2:
-            return shape == 1 ? launch_phased<2, 1, 1, 4, 4>(diag, p, stream) : launch_phased<2, 1, 1, 2, 2>(diag, p, stream);
+            return shape == 1 ? launch_phased<2, 1, 1, 4, 4>(diag, fmt, p, stream) : launch_phased<2, 1, 1, 2, 2>(diag, fmt, p, stream);
         case 3:
-            return launch_phased<3, 1, 1, 2, 2>(diag, p, stream);
+            return launch_phased<3, 1, 1, 2, 2>(diag, fmt, p, stream);
         case 4:
-            return shape == 1 ? launch_phased<4, 1, 1, 4, 4>(diag, p, stream) : launch_phased<4, 1, 1, 2, 2>(diag, p, stream);
+            return shape == 1 ? launch_phased<4, 1, 1, 4, 4>(diag, fmt, p, stream) : launch_phased<4, 1, 1, 2, 2>(diag, fmt, p, stream);
         // 25 .. 64 samples per pixel: one pixel per lane, its samples in groups of four slots like the 4x4 case
         case 5:
-            return launch_phased<5, 1, 1, 2, 2>(diag, p, stream);
+            return launch_phased<5, 1, 1, 2, 2>(diag, fmt, p, stream);
         case 6:
-            return launch_phased<6, 1, 1, 2, 2>(diag, p, stream);
+            return launch_phased<6, 1, 1, 2, 2>(diag, fmt, p, stream);
         case 7:
-            return launch_phased<7, 1, 1, 2, 2>(diag, p, stream);
+            return launch_phased<7, 1, 1, 2, 2>(diag, fmt, p, stream);
         case 8:
-            return launch_phased<8, 1, 1, 2, 2>(diag, p, stream);
+            return launch_phased<8, 1, 1, 2, 2>(diag, fmt, p, stream);
         default:
             return cudaErrorInvalidValue;
     }

@@ -14,7 +14,8 @@
 // frames from one queue), --frames=K (orbit sweep; frame f goes to <stem>.f.tga, frame 0 is the reference camera), --stats (summary on stderr), --buckets (the reference's 64x64 bucket
 // schedule through Renderer::render_region instead of one launch per frame), --format=tga|png|apng (a real TGA, a PNG
 // encoded on the GPU: the output is then named *.png and sweep frames <stem>.f.png, or all frames in ONE animated PNG
-// named *.png), --fps=F (frame rate of --format apng).
+// named *.png), --fps=F (frame rate of --format apng), --format=pfm (the pixels before quantisation as a colour PFM
+// of 32-bit floats, named *.pfm; sweep frames <stem>.f.pfm).
 #include <cerrno>
 #include <chrono>
 #include <cmath>
@@ -58,6 +59,7 @@ const char *USAGE =
     "        --format <ppm|tga|png>             File contents: the reference's binary PPM, a real TGA, or a PNG encoded\n"
     "                                           on the GPU (the output is then named *.png) [default: ppm]\n"
     "        --format apng                      All frames in one animated PNG encoded on the GPU (named *.png)\n"
+    "        --format pfm                       The unquantised pixels as a colour PFM of 32-bit floats (named *.pfm)\n"
     "        --fps <F>                          Frames per second of --format apng, 1..65535 [default: 24]\n"
     "        --preview <N>                      Undersampled preview: trace one pixel per NxN block (1 sample) [default: off]\n"
     "        --stats                            Print a timing summary to stderr\n"
@@ -65,7 +67,8 @@ const char *USAGE =
     "                                           be multiples of 64, as in the reference); default is whole frames\n"
     "\n"
     "ARGS:\n"
-    "    <output>    Either a file with .tga extension (.png with --format png or apng), or - to write file to stdout\n";
+    "    <output>    Either a file with .tga extension (.png with --format png or apng, .pfm with --format pfm), or - to\n"
+    "                write file to stdout\n";
 
 [[noreturn]] void usage_error(const std::string &msg) {
     // clap 2: message + usage hint on stderr, exit status 1
@@ -224,8 +227,8 @@ int main(int argc, char **argv) {
     const std::string &output_file = args.output;
     FileOrAnyWriter output;
     FILE *fp = nullptr;
-    const bool png = args.format == "png", apng = args.format == "apng";
-    const std::string ext = png || apng ? "png" : "tga";
+    const bool png = args.format == "png", apng = args.format == "apng", pfm = args.format == "pfm";
+    const std::string ext = png || apng ? "png" : pfm ? "pfm" : "tga";
     // before the output's name is checked: a misused --fps is a usage error whatever the name
     if (!args.fps.empty() && !apng) usage_error("The argument '--fps' can only be used with '--format apng'");
     unsigned long long fps = 24;
@@ -249,10 +252,12 @@ int main(int argc, char **argv) {
     unsigned frames = (unsigned)parse_or_panic(args.frames.empty() ? "1" : args.frames, 100000, "frames");
     if (gpus < 1) gpus = 1;
     if (frames < 1) frames = 1;
-    if (!args.format.empty() && args.format != "ppm" && args.format != "tga" && !png && !apng)
-        usage_error("'" + args.format + "' isn't a valid value for '--format <ppm|tga|png|apng>'");
-    // the bucket schedule exists to drive the host writer seam; a PNG is encoded on the GPU from a whole frame
-    if ((png || apng) && args.buckets) usage_error("The argument '--buckets' cannot be used with '--format " + args.format + "'");
+    if (!args.format.empty() && args.format != "ppm" && args.format != "tga" && !png && !apng && !pfm)
+        usage_error("'" + args.format + "' isn't a valid value for '--format <ppm|tga|png|apng|pfm>'");
+    // the bucket schedule exists to drive the host writer seam; a PNG is encoded on the GPU from a whole frame,
+    // and a PFM is the float frame of the whole-frame path
+    if ((png || apng || pfm) && args.buckets) usage_error("The argument '--buckets' cannot be used with '--format " + args.format + "'");
+    if (pfm && !args.preview.empty()) usage_error("The argument '--preview' cannot be used with '--format pfm'");
     const bool real_tga = args.format == "tga";
     const unsigned preview = args.preview.empty() ? 0u : (unsigned)parse_or_panic(args.preview, 1024, "preview");
     if (options.width == 0 || options.height == 0) {
@@ -278,7 +283,7 @@ int main(int argc, char **argv) {
             if (!fp) throw Panic(std::string("called `Result::unwrap()` on an `Err` value: ") + strerror(errno));
             return FileOrAnyWriter::file_writer(fp);
         };
-        if (frames > 1 && !preview && !args.buckets) {
+        if (frames > 1 && !preview && !args.buckets && !pfm) {
             // orbit sweep: the GPUs draw frames from one queue, copy-out of a frame overlapping the render of the next ones;
             // the frames come back in order (rt_render_sweep_multi)
             std::vector<rt_camera> cams;
@@ -320,7 +325,12 @@ int main(int argc, char **argv) {
                 if (!apng || f == 0) output = open_output(f);  // an animation is one file
                 rt_camera cam = orbit_camera(f, frames);
                 rt_stats st;
-                if (png || apng) {
+                if (pfm) {  // <stem>.f.pfm per frame, or the frames back to back on stdout
+                    auto r0 = clk::now();
+                    Renderer::render_pfm(options, scene, output.f, frames > 1 ? &cam : nullptr, &st);
+                    render_ms += std::chrono::duration<double, std::milli>(clk::now() - r0).count();
+                    kernel_ms += st.kernel_ms;
+                } else if (png || apng) {
                     const Renderer::ApngFrame af{f, frames, 1, (uint16_t)fps};
                     auto r0 = clk::now();
                     Renderer::render_png(options, scene, output.f, frames > 1 ? &cam : nullptr, preview, &st, apng ? &af : nullptr);

@@ -208,6 +208,25 @@ inline void write_tga(FILE *f, uint16_t width, uint16_t height, const uint8_t *p
     fflush(f);
 }
 
+// Extension: a colour PFM of a frame's pixels before quantisation -- "PF", the size, scale -1.0 (little-endian
+// samples), then the rows from the bottom up as 32-bit float RGB.  `px` holds `height` rows of {r, g, b, alpha}
+// floats, `stride` floats apart; alpha is dropped, as the P6 sink drops it.
+inline void write_pfm(FILE *f, uint16_t width, uint16_t height, const float *px, size_t stride) {
+    fprintf(f, "PF\n%u %u\n-1.0\n", (unsigned)width, (unsigned)height);
+    std::vector<uint8_t> line((size_t)width * 12);
+    for (uint32_t y = height; y-- > 0;) {  // bottom row first
+        const float *row = px + (size_t)y * stride;
+        for (uint32_t x = 0; x < width; x++)
+            for (int c = 0; c < 3; c++) {
+                uint32_t bits;
+                memcpy(&bits, &row[x * 4 + c], 4);
+                for (int b = 0; b < 4; b++) line[(x * 3 + c) * 4 + b] = (uint8_t)(bits >> (8 * b));
+            }
+        if (fwrite(line.data(), 1, line.size(), f) != line.size()) throw Panic("write_all failed");
+    }
+    fflush(f);
+}
+
 class TGARGBABufferWriter : public RGBABufferWriter {
   public:
     explicit TGARGBABufferWriter(FileOrAnyWriter *writer) : out_(writer) {}
@@ -420,6 +439,23 @@ struct Renderer {
                  "Renderer::render_png");
         if (fwrite(b.file, 1, len, f) != len) throw Panic("write_all failed");
         fflush(f);
+    }
+
+    // One frame before quantisation as a colour PFM on `f` (extension): rendered on the scene's GPUs into pinned host
+    // memory as float RGBA (rt_render_frame_multi_f32), then written by write_pfm.
+    static void render_pfm(const RenderOptions &o, const Scene &scene, FILE *f, const rt_camera *camera = nullptr,
+                           rt_stats *stats = nullptr) {
+        struct Frame {
+            void *p = nullptr;
+            ~Frame() { rt_host_free(p); }
+        } b;
+        const size_t frame_bytes = (size_t)o.width * o.height * 16;
+        rt_check(rt_host_alloc(frame_bytes, &b.p), "Renderer::render_pfm");
+        float *frame = static_cast<float *>(b.p);
+        rt_check(rt_render_frame_multi_f32(scene.replicas(), scene.gpus(), camera, o.width, o.height, o.samples_per_pixel,
+                                           frame, frame_bytes, stats),
+                 "Renderer::render_pfm");
+        write_pfm(f, o.width, o.height, frame, (size_t)o.width * 4);
     }
 
   private:

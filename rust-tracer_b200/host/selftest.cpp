@@ -178,6 +178,22 @@ void sink_error() {
     printf("ok sink_error\n");
 }
 
+// write_pfm on a synthetic 3x2 frame, no GPU: pixel (x, y) component c = ((y * 3 + x) * 4 + c) / 7 in f32, with a
+// pitch of 5 pixels so that the writer must follow the stride.  tests/test_f32.py checks the file's bytes.
+void pfm(const char *path) {
+    const uint16_t w = 3, h = 2;
+    const size_t stride = 5 * 4;
+    std::vector<float> px(stride * h, -1.0f);
+    for (uint32_t y = 0; y < h; y++)
+        for (uint32_t x = 0; x < w; x++)
+            for (uint32_t c = 0; c < 4; c++) px[y * stride + x * 4 + c] = (float)((y * w + x) * 4 + c) / 7.0f;
+    FILE *f = fopen(path, "wb");
+    if (!f) throw Panic(std::string("cannot create ") + path);
+    write_pfm(f, w, h, px.data(), stride);
+    fclose(f);
+    printf("ok pfm\n");
+}
+
 }  // namespace
 
 int main(int argc, char **argv) {
@@ -187,6 +203,7 @@ int main(int argc, char **argv) {
         if (what == "basic_rendering" || what == "all") basic_rendering();
         if (what == "sink_error" || what == "all") sink_error();
         if (what == "progressive" || what == "all") progressive(argc > 2 ? argv[2] : "/tmp/rtrace_selftest.tga");
+        if (what == "pfm" || what == "all") pfm(argc > 2 ? argv[2] : "/tmp/rtrace_selftest.pfm");
     } catch (const Panic &p) {
         fprintf(stderr, "FAILED: panicked at '%s'\n", p.what());
         return 1;

@@ -27,6 +27,7 @@ ABI_SYMBOLS = [
     "rt_count_rays", "rt_trace_rays", "rt_measure_fp32_peak", "rt_microbench_fp32", "rt_selftest_math", "rt_debug_phased_tiles", "rt_host_alloc", "rt_host_free", "rt_host_register", "rt_host_unregister", "rt_microbench_d2h", "rt_device_alloc", "rt_device_free", "rt_ipc_export", "rt_ipc_open", "rt_ipc_close", "rt_memcpy", "rt_memcpy2d_async", "rt_pack_rgb_rows",
     "rt_png_bound", "rt_encode_png", "rt_render_sweep_png",
     "rt_apng_bound", "rt_encode_apng_frame", "rt_render_sweep_apng",
+    "rt_render_rows_f32", "rt_render_frame_multi_f32",
 ]
 
 
@@ -134,6 +135,10 @@ def lib():
                                        C.POINTER(C.c_size_t), vp]
     L.rt_render_sweep_apng.argtypes = [C.POINTER(vp), C.c_int, C.POINTER(Camera), u32, u32, u32, u32, u16, u16,
                                        FRAME_CALLBACK, vp, C.POINTER(Stats)]
+    L.rt_render_rows_f32.argtypes = [vp, C.POINTER(Camera), u32, u32, u32, u32, u32, u32, vp, C.c_size_t, vp,
+                                     C.POINTER(Stats)]
+    L.rt_render_frame_multi_f32.argtypes = [C.POINTER(vp), C.c_int, C.POINTER(Camera), u32, u32, u32, vp, C.c_size_t,
+                                            C.POINTER(Stats)]
     if os.environ.get("RTRACE_B200_LIB"):
         L = real
     _lib = L
@@ -348,6 +353,42 @@ class Renderer:
         st = Stats() if want_stats else None
         _check(lib().rt_render_frame(scene.handle, C.byref(camera) if camera is not None else None, w, h, spp,
                                      out_ptr, w * h * 4, C.byref(st) if st is not None else None))
+        return (out, st) if want_stats else out
+
+    @staticmethod
+    def render_f32(options, scene_or_scenes, camera=None, out_ptr=None, want_stats=False):
+        """The frame before quantisation (rt_render_frame_multi_f32): (h, w, 4) float32 {r, g, b, alpha}, equal bit
+        for bit to the reference's values.  A list of scenes renders on their GPUs; with out_ptr (device memory of
+        the first scene's GPU, h * w * 16 bytes) the frame is stored there and None is returned in its place."""
+        w, h, spp = options.width, options.height, options.samples_per_pixel
+        scenes = list(scene_or_scenes) if isinstance(scene_or_scenes, (list, tuple)) else [scene_or_scenes]
+        out = None
+        if out_ptr is None:
+            out = np.empty((h, w, 4), np.float32)
+            out_ptr = out.ctypes.data
+        arr = (C.c_void_p * len(scenes))(*[s.handle for s in scenes])
+        st = Stats() if want_stats else None
+        _check(lib().rt_render_frame_multi_f32(arr, len(scenes), C.byref(camera) if camera is not None else None, w, h,
+                                               spp, out_ptr, w * h * 16, C.byref(st) if st is not None else None))
+        return (out, st) if want_stats else out
+
+    @staticmethod
+    def render_rows_f32(options, scene, row_start=0, row_stride=1, row_count=None, camera=None, out=None,
+                        out_ptr=None, pitch=0, stream=None, want_stats=False):
+        """render_rows before quantisation (rt_render_rows_f32): (row_count, w, 4) float32 for host output; with
+        out_ptr (host or device memory, `pitch` bytes per row, 0 = w * 16) the call is asynchronous on `stream` for
+        device memory and None is returned in place of the array."""
+        w, h, spp = options.width, options.height, options.samples_per_pixel
+        if row_count is None:
+            row_count = (h - row_start + row_stride - 1) // row_stride
+        if out_ptr is None:
+            if out is None:
+                out = np.empty((row_count, w, 4), np.float32)
+            out_ptr = out.ctypes.data
+        st = Stats() if want_stats else None
+        _check(lib().rt_render_rows_f32(scene.handle, C.byref(camera) if camera is not None else None, w, h, spp,
+                                        row_start, row_stride, row_count, out_ptr, pitch, stream,
+                                        C.byref(st) if st is not None else None))
         return (out, st) if want_stats else out
 
     @staticmethod
