@@ -221,6 +221,32 @@ int rt_render_frame_multi_f32(rt_scene *const *scenes, int ngpu, const rt_camera
                               uint32_t width, uint32_t height, uint32_t spp,
                               float *rgba_out, size_t rgba_bytes, rt_stats *stats);
 
+/* ---- geometry output (AOVs) ------------------------------------------------------------------------------------
+ * The geometry behind each pixel: eight f32 per pixel, 32 bytes, as two float4 {nx, ny, nz, coverage}
+ * {distance, px, py, pz}.  Over the pixel's spp*spp primary rays in reference order (render.rs:236-243, with the
+ * camera extension), each traced from a miss (render.rs:188-189), the samples that hit contribute:
+ *   n   += the hit's unit normal (primitive.rs:83);  cnt += 1.0f;
+ *   if distance < dmin (strict: the first sample wins a tie): dmin = distance, pos = ray.pos + ray.dir * distance
+ *   (the first term of the shadow origin, render.rs:199).
+ * From n = (0,0,0), cnt = 0, dmin = +inf, pos = (0,0,0), with r = 1/(spp*spp) (render.rs:219-220): normal = n * r
+ * (box-filtered, not renormalised: shorter at silhouettes, zero where nothing was hit), coverage = cnt * r (like
+ * alpha, not exactly 1.0 for full coverage at spp 3, 5, 6, 7), distance = dmin (+inf where nothing was hit, as in
+ * rt_hit), position = pos.  Equal bit for bit to the reference's f32 arithmetic.  No shadow ray is traced
+ * (stats->shadow_rays = 0).  The variant rule is the float output's (PHASED or LANE; stats->variant_used).  A device
+ * output pointer must be 16-byte aligned and a pitch a multiple of 16 and at least width*32, else RT_ERR_INVALID. */
+/* rt_render_rows with AOV output: rows row_start, row_start+row_stride, ... (row_count of them), pitch in bytes
+ * (0 = width*32).  Host (pageable or pinned) or device output; with a device pointer the call is asynchronous on
+ * `stream`. */
+int rt_render_rows_aov(const rt_scene *s, const rt_camera *camera,
+                       uint32_t width, uint32_t height, uint32_t spp,
+                       uint32_t row_start, uint32_t row_stride, uint32_t row_count,
+                       float *aov_out, size_t pitch_bytes, void *stream, rt_stats *stats);
+/* rt_render_frame_multi with AOV output: aov_out holds width*height*32 bytes (RT_ERR_BUFFER when aov_bytes is
+ * less), in host memory or in device memory of scenes[0]'s GPU; ngpu == 1 is a single-GPU frame. */
+int rt_render_frame_multi_aov(rt_scene *const *scenes, int ngpu, const rt_camera *camera,
+                              uint32_t width, uint32_t height, uint32_t spp,
+                              float *aov_out, size_t aov_bytes, rt_stats *stats);
+
 /* The same sweep with the frames PULLED instead of listed: whenever the pipeline has room for another frame the
  * library calls `next(next_user, &camera, &use_camera)`, which fills the camera (or sets *use_camera = 0 for the
  * reference camera; it is 1 on entry) and returns the frame's id (>= 0; handed back to `cb` as its frame argument)

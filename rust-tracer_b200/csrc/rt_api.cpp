@@ -369,10 +369,10 @@ int kernel_variant(const rt::RenderParams &p) {
     return (pixel_tiles < 8000 && tile_ok) ? RT_KERNEL_TILE : RT_KERNEL_PHASED;
 }
 
-// Float frames have PHASED and LANE kernels only: PHASED wherever RGBA8 would run TILE or PHASED (PHASED is
+// Float and AOV frames have PHASED and LANE kernels only: PHASED wherever RGBA8 would run TILE or PHASED (PHASED is
 // correct at every size) and for a forced TILE or PHASED inside PHASED's domain; LANE for everything else,
 // including a forced LANE or WARP.
-int kernel_variant_f32(const rt::RenderParams &p) {
+int kernel_variant_float(const rt::RenderParams &p) {
     switch (g_variant) {
         case RT_VARIANT_LANE:
         case RT_VARIANT_WARP:
@@ -420,7 +420,7 @@ int prepare_phased(rt_scene *s, rt::RenderParams &p, cudaStream_t stream, int sh
 // Launches the kernel(s) of one frame on `stream`; *variant receives the kernel that renders it (RT_KERNEL_*,
 // numbered like RT_VARIANT_*).
 int launch(rt_scene *s, rt::RenderParams &p, bool diag, cudaStream_t stream, int *variant, RtPixels fmt = RT_PIXELS_RGBA8) {
-    const int v = fmt == RT_PIXELS_F32 ? kernel_variant_f32(p) : kernel_variant(p), shape = forced_tile_shape();
+    const int v = fmt != RT_PIXELS_RGBA8 ? kernel_variant_float(p) : kernel_variant(p), shape = forced_tile_shape();
     *variant = v;
     cudaError_t e;
     if (v == RT_KERNEL_PHASED) {
@@ -438,7 +438,10 @@ int launch(rt_scene *s, rt::RenderParams &p, bool diag, cudaStream_t stream, int
     return RT_OK;
 }
 
-uint32_t launches_of(int variant) { return variant == RT_KERNEL_PHASED ? 4 : 1; }
+// PHASED: K1-K4, or K1, K2 and the AOV store
+uint32_t launches_of(int variant, RtPixels fmt = RT_PIXELS_RGBA8) {
+    return variant == RT_KERNEL_PHASED ? (fmt == RT_PIXELS_AOV ? 3 : 4) : 1;
+}
 
 // Queues on `stream` the PNG encode of the RGBA8 frame `rgba` (anim != nullptr: frame `frame`'s payload of that
 // animated PNG) into `out` -- the file, then its length word -- and the copy of the length word to *len_host.
@@ -620,10 +623,10 @@ static int render_rows_impl(rt_scene *s, const rt_camera *camera, uint32_t width
     // col_count > 0: only columns col_start .. col_start + col_count - 1, packed from byte 0 of each output row
     if ((uint64_t)col_start + col_count > width) return fail(RT_ERR_INVALID, "columns %u..%u leave the %u-pixel row", col_start, col_start + col_count, width);
     const uint32_t cols = col_count ? col_count : width;
-    const size_t bpp = fmt == RT_PIXELS_F32 ? 16 : 4;  // bytes per pixel; pitches and device pointers are multiples of it
-    const size_t row_bytes = (size_t)cols * bpp;
+    const size_t align = rt_pixel_align(fmt);  // pitches and device pointers are multiples of it
+    const size_t row_bytes = (size_t)cols * rt_pixel_bytes(fmt);
     if (pitch_bytes == 0) pitch_bytes = row_bytes;
-    if (pitch_bytes < row_bytes || (pitch_bytes & (bpp - 1))) return fail(RT_ERR_INVALID, "pitch %zu too small or not a multiple of %zu", pitch_bytes, bpp);
+    if (pitch_bytes < row_bytes || (pitch_bytes & (align - 1))) return fail(RT_ERR_INVALID, "pitch %zu too small or not a multiple of %zu", pitch_bytes, align);
     if (stats) memset(stats, 0, sizeof(*stats));
     if (row_count == 0) return RT_OK;
 
@@ -639,7 +642,7 @@ static int render_rows_impl(rt_scene *s, const rt_camera *camera, uint32_t width
         RT_TRY(enable_peer(s->device, out_dev, &can));
         if (!can) return fail(RT_ERR_INVALID, "rgba_out lives on device %d, which device %d cannot access", out_dev, s->device);
     }
-    if (out_on_device && (((uintptr_t)rgba_out) & (bpp - 1))) return fail(RT_ERR_INVALID, "device rgba_out must be %zu-byte aligned", bpp);
+    if (out_on_device && (((uintptr_t)rgba_out) & (align - 1))) return fail(RT_ERR_INVALID, "device rgba_out must be %zu-byte aligned", align);
     int kinds_dev = -1;
     const bool kinds_on_device = kinds_out && is_device_ptr(kinds_out, &kinds_dev);
     const size_t kinds_bytes = (size_t)cols * row_count * spp * spp;
@@ -713,7 +716,7 @@ static int render_rows_impl(rt_scene *s, const rt_camera *camera, uint32_t width
         stats->total_ms = now_ms() - t0;
         stats->primary_rays = (uint64_t)cols * row_count * spp * spp;
         stats->shadow_rays = counting ? ctr[1] : 0;
-        stats->kernel_launches = launches_of(variant);
+        stats->kernel_launches = launches_of(variant, fmt);
         stats->gpus = 1;
         stats->variant_used = (uint32_t)variant;
     }
@@ -734,6 +737,15 @@ int rt_render_rows_f32(const rt_scene *s, const rt_camera *camera, uint32_t widt
     return render_rows_impl(const_cast<rt_scene *>(s), camera, width, height, spp, row_start, row_stride, row_count,
                             reinterpret_cast<uint8_t *>(rgba_out), pitch_bytes, nullptr, (cudaStream_t)stream, stats,
                             nullptr, nullptr, 0, 0, RowLayout(), RT_PIXELS_F32);
+}
+
+int rt_render_rows_aov(const rt_scene *s, const rt_camera *camera, uint32_t width, uint32_t height, uint32_t spp,
+                       uint32_t row_start, uint32_t row_stride, uint32_t row_count, float *aov_out, size_t pitch_bytes,
+                       void *stream, rt_stats *stats) {
+    if (!aov_out) return fail(RT_ERR_INVALID, "aov_out is NULL");
+    return render_rows_impl(const_cast<rt_scene *>(s), camera, width, height, spp, row_start, row_stride, row_count,
+                            reinterpret_cast<uint8_t *>(aov_out), pitch_bytes, nullptr, (cudaStream_t)stream, stats,
+                            nullptr, nullptr, 0, 0, RowLayout(), RT_PIXELS_AOV);
 }
 
 int rt_render_row_blocks(const rt_scene *s, const rt_camera *camera, uint32_t width, uint32_t height, uint32_t spp,
@@ -1003,7 +1015,7 @@ static int frame_multi_locked(rt_scene *const *scenes, int ngpu, const rt_camera
                               uint32_t spp, uint8_t *rgba_out, rt_stats *stats, std::vector<char> &launched,
                               RtPixels fmt) {
     const double t0 = now_ms();
-    const size_t row_bytes = (size_t)width * (fmt == RT_PIXELS_F32 ? 16 : 4);
+    const size_t row_bytes = (size_t)width * rt_pixel_bytes(fmt);
     rt_scene *root = scenes[0];
     int out_dev = -1;
     const bool to_device = is_device_ptr(rgba_out, &out_dev);
@@ -1047,7 +1059,7 @@ static int frame_multi_locked(rt_scene *const *scenes, int ngpu, const rt_camera
         launched[(size_t)g] = 1;  // from here on this GPU may have work in flight
         int variant = 0;
         RT_TRY(launch(s, p, false, s->own_stream, &variant, fmt));
-        launches += launches_of(variant);
+        launches += launches_of(variant, fmt);
         if (g == 0) used = (uint32_t)variant;
         if (stats) CUDA_TRY(cudaEventRecord(s->ev1, s->own_stream));
         if (!to_device) {
@@ -1092,12 +1104,12 @@ static int lock_scenes(rt_scene *const *scenes, int ngpu, std::vector<std::uniqu
     return RT_OK;
 }
 
-// rt_render_frame_multi and rt_render_frame_multi_f32: the frame at 4 or 16 bytes per pixel.
+// rt_render_frame_multi, rt_render_frame_multi_f32 and rt_render_frame_multi_aov: the frame in format `fmt`.
 static int frame_multi_impl(rt_scene *const *scenes, int ngpu, const rt_camera *camera, uint32_t width, uint32_t height,
                             uint32_t spp, uint8_t *rgba_out, size_t rgba_len, rt_stats *stats, RtPixels fmt) {
     if (!scenes || ngpu < 1) return fail(RT_ERR_INVALID, "need at least one scene");
     if (!rgba_out) return fail(RT_ERR_INVALID, "rgba_out is NULL");
-    const size_t bpp = fmt == RT_PIXELS_F32 ? 16 : 4, frame_bytes = (size_t)width * height * bpp;
+    const size_t frame_bytes = (size_t)width * height * rt_pixel_bytes(fmt);
     if (rgba_len < frame_bytes) return fail(RT_ERR_BUFFER, "rgba_out holds %zu bytes, frame needs %zu", rgba_len, frame_bytes);
     for (int g = 0; g < ngpu; g++) {
         int rc = check_frame_args(scenes[g], width, height, spp, 0, 1, height);
@@ -1107,8 +1119,8 @@ static int frame_multi_impl(rt_scene *const *scenes, int ngpu, const rt_camera *
     if (ngpu == 1)
         return render_rows_impl(scenes[0], camera, width, height, spp, 0, 1, height, rgba_out, 0, nullptr, nullptr,
                                 stats, nullptr, nullptr, 0, 0, RowLayout(), fmt);
-    if (fmt == RT_PIXELS_F32 && is_device_ptr(rgba_out, nullptr) && ((uintptr_t)rgba_out & 15))
-        return fail(RT_ERR_INVALID, "device rgba_out must be 16-byte aligned");
+    if (fmt != RT_PIXELS_RGBA8 && is_device_ptr(rgba_out, nullptr) && ((uintptr_t)rgba_out & (rt_pixel_align(fmt) - 1)))
+        return fail(RT_ERR_INVALID, "device rgba_out must be %zu-byte aligned", rt_pixel_align(fmt));
 
     std::vector<std::unique_lock<std::mutex>> locks;
     int rc = lock_scenes(scenes, ngpu, locks);
@@ -1138,6 +1150,12 @@ int rt_render_frame_multi_f32(rt_scene *const *scenes, int ngpu, const rt_camera
                               uint32_t spp, float *rgba_out, size_t rgba_bytes, rt_stats *stats) {
     return frame_multi_impl(scenes, ngpu, camera, width, height, spp, reinterpret_cast<uint8_t *>(rgba_out), rgba_bytes,
                             stats, RT_PIXELS_F32);
+}
+
+int rt_render_frame_multi_aov(rt_scene *const *scenes, int ngpu, const rt_camera *camera, uint32_t width, uint32_t height,
+                              uint32_t spp, float *aov_out, size_t aov_bytes, rt_stats *stats) {
+    return frame_multi_impl(scenes, ngpu, camera, width, height, spp, reinterpret_cast<uint8_t *>(aov_out), aov_bytes,
+                            stats, RT_PIXELS_AOV);
 }
 
 // ---------------------------------------------------------------------------

@@ -200,6 +200,44 @@ __global__ void __launch_bounds__(BLOCK_THREADS) render_lane_f32_kernel(const Re
     render_body<RT_KERNEL_LANE, false, false, true>(p, threadIdx.x);
 }
 
+// The AOV pixel of one lane (rt_kernels.h RT_PIXELS_AOV): the primary closest hit of every sample in reference order,
+// no shadow ray.  Over the samples that hit: the sum of the unit normals (primitive.rs:83) and the hit count, both
+// times 1/(spp*spp), and the nearest hit's distance and point pos + dir * distance (render.rs:199, first term; the
+// first sample wins a tie).  `tid` as in render_body.
+__device__ __forceinline__ void aov_lane_body(const RenderParams &p, const uint32_t tid) {
+    const int lane = tid & 31;
+    const int warp = tid >> 5;
+    const uint32_t x = blockIdx.x * (TILE_W * WARPS_X) + (warp % WARPS_X) * TILE_W + (lane % TILE_W);
+    const uint32_t j = blockIdx.y * (TILE_H * WARPS_Y) + (warp / WARPS_X) * TILE_H + (lane / TILE_W);
+    if (x >= p.width || j >= p.row_count) return;
+    const uint32_t y = image_row(p, j);
+    const V3 eye = v3(p.eye[0], p.eye[1], p.eye[2]);
+    V3 n = v3(0.0f, 0.0f, 0.0f), pos = v3(0.0f, 0.0f, 0.0f);
+    float cnt = 0.0f, dmin = RT_INF;
+    for (uint32_t ssx = 0; ssx < p.spp; ssx++) {
+        for (uint32_t ssy = 0; ssy < p.spp; ssy++) {
+            const V3 d = primary_dir(p, x, y, ssx, ssy);
+            float hitd = RT_INF;
+            uint32_t hit_idx = 0;
+            lane_traverse<false>(p.sph, p.skip, p.n_nodes, eye, d, hitd, hit_idx);
+            if (hitd == RT_INF) continue;
+            n = vadd(n, hit_normal(__ldg(&p.sph[hit_idx]), eye, d, hitd));
+            cnt = fadd(cnt, 1.0f);
+            if (hitd < dmin) dmin = hitd, pos = vadd(eye, vmulf(d, hitd));
+        }
+    }
+    const float recip = frecip(fmul((float)p.spp, (float)p.spp));  // render.rs:219-220
+    n = vmulf(n, recip);
+    float4 *at = reinterpret_cast<float4 *>(p.out + (size_t)out_row(p, j) * p.pitch + (size_t)x * 32);
+    at[0] = make_float4(n.x, n.y, n.z, fmul(cnt, recip));
+    at[1] = make_float4(dmin, pos.x, pos.y, pos.z);
+}
+
+// LANE with AOV output: the fallback of AOV frames outside PHASED's domain.
+__global__ void __launch_bounds__(BLOCK_THREADS) render_lane_aov_kernel(const RenderParams p) {
+    aov_lane_body(p, threadIdx.x);
+}
+
 // Closest-hit traversal of arbitrary rays (rt_trace_rays): group.rs:72-83 from Hit::missed().
 __global__ void trace_rays_kernel(const float4 *__restrict__ sph, const uint32_t *__restrict__ skip, uint32_t n,
                                   size_t n_rays, const float *__restrict__ rays, float *__restrict__ hits) {
@@ -320,6 +358,8 @@ cudaError_t rt_launch_render(int variant, bool diag, RtPixels fmt, const RenderP
     if (grid.x == 0 || grid.y == 0) return cudaSuccess;
     if (fmt == RT_PIXELS_F32) {
         render_lane_f32_kernel<<<grid, block, 0, stream>>>(p);
+    } else if (fmt == RT_PIXELS_AOV) {
+        render_lane_aov_kernel<<<grid, block, 0, stream>>>(p);
     } else if (variant == RT_KERNEL_LANE) {
         if (diag)
             render_kernel<RT_KERNEL_LANE, true><<<grid, block, 0, stream>>>(p);

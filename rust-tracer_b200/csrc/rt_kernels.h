@@ -6,15 +6,21 @@
 
 enum { RT_KERNEL_LANE = 1, RT_KERNEL_WARP = 2, RT_KERNEL_TILE = 3, RT_KERNEL_PHASED = 4 };
 
-// What a frame's kernels store per pixel: RGBA8 (4 bytes), or the four f32 values RGBA8 quantises (16 bytes, at
-// out + row * pitch + x * 16).  Float output has LANE and PHASED kernels only, without diagnostics.
-enum RtPixels { RT_PIXELS_RGBA8 = 0, RT_PIXELS_F32 = 1 };
+// What a frame's kernels store per pixel: RGBA8 (4 bytes), the four f32 values RGBA8 quantises (16 bytes, at
+// out + row * pitch + x * 16), or the AOV pixel: eight f32 {nx, ny, nz, coverage} {distance, px, py, pz} (32 bytes,
+// include/rtrace.h "geometry output").  Float and AOV output have LANE and PHASED kernels only, without diagnostics.
+enum RtPixels { RT_PIXELS_RGBA8 = 0, RT_PIXELS_F32 = 1, RT_PIXELS_AOV = 2 };
+
+// Bytes per pixel of a format.  Pitches and device output pointers must be multiples of the widest store the
+// kernels issue for it, min(bytes per pixel, 16): a float4.
+constexpr size_t rt_pixel_bytes(RtPixels fmt) { return fmt == RT_PIXELS_AOV ? 32 : fmt == RT_PIXELS_F32 ? 16 : 4; }
+constexpr size_t rt_pixel_align(RtPixels fmt) { return rt_pixel_bytes(fmt) < 16 ? rt_pixel_bytes(fmt) : 16; }
 
 namespace rt {
 struct RenderParams;
 }
 
-// RT_PIXELS_F32 runs the LANE kernel whatever `variant` is.
+// RT_PIXELS_F32 and RT_PIXELS_AOV run their LANE kernel whatever `variant` is.
 cudaError_t rt_launch_render(int variant, bool diag, RtPixels fmt, const rt::RenderParams &p, cudaStream_t stream);
 cudaError_t rt_launch_render_preview(const rt::RenderParams &p, cudaStream_t stream);
 cudaError_t rt_launch_trace_rays(const float4 *sph, const uint32_t *skip, uint32_t n, size_t n_rays,

@@ -892,6 +892,84 @@ __global__ void __launch_bounds__(32 * CW * CH, phased_min_blocks(CW * CH)) phas
     shade_store_body<SPP, PXW, PXH, CW, CH, false, true>(p, threadIdx.x);
 }
 
+// ---------------------------------------------------------------------------
+// AOV store: the geometry of K2's winners, in place of K3 + K4; one warp per pixel tile
+// ---------------------------------------------------------------------------
+// Per pixel, over the samples that hit (reference sample order): the sum of the unit normals and the hit count,
+// both times 1/(spp*spp), and the nearest hit's distance and point (the first sample wins a tie).  Stored as two
+// float4 {nx, ny, nz, coverage} {distance, px, py, pz} at x * 32 of the pixel's row.  The normal and the hit point
+// are phase A of K4 (render.rs:194, :199 first term), so the normal is the one K4 shades with.
+template <int SPP, int PXW, int PXH, int CW, int CH>
+__global__ void __launch_bounds__(32 * CW * CH, phased_min_blocks(CW * CH)) phase_aov_store(const RenderParams p) {
+    using G = Geo<SPP, PXW, PXH, CW, CH>;
+    constexpr int S = G::S, NS = G::NS;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const G geo(p.width, p.row_count);
+    const uint32_t ct = blockIdx.y * geo.ctiles_x + blockIdx.x;
+    const uint32_t pt_x = blockIdx.x * CW + (uint32_t)(warp % CW), pt_y = blockIdx.y * CH + (uint32_t)(warp / CW);
+    if (pt_x >= geo.ptiles_x || pt_y >= geo.ptiles_y) return;
+    const uint32_t pt = pt_y * geo.ptiles_x + pt_x;
+    const uint32_t tile_x0 = pt_x * G::TW, tile_j0 = pt_y * G::TH;
+    const uint2 *winner = reinterpret_cast<const uint2 *>(p.winner) + (size_t)pt * S * 32;  // {leaf index, hit distance} per slot (K2)
+    const ONE2 one = f2s(p.one);
+    const V3x2 eye2 = v3x2s(v3(p.eye[0], p.eye[1], p.eye[2]));
+    const float recip = frecip(fmul((float)SPP, (float)SPP));  // render.rs:219-220
+    auto store = [&](uint32_t x, uint32_t j, float4 a, float4 b) {
+        float4 *at = reinterpret_cast<float4 *>(p.out + (size_t)out_row(p, j) * p.pitch + (size_t)x * 32);
+        at[0] = a;
+        at[1] = b;
+    };
+
+    if (p.tile_hdr[ct].z == 0x7f800000u) {
+        // no ray of this cull tile hit anything, and K2 wrote no winners: every sample is a miss
+        const float4 a = make_float4(0.0f, 0.0f, 0.0f, 0.0f), b = make_float4(RT_INF, 0.0f, 0.0f, 0.0f);  // 0 * recip = +0
+        for (int pi = 0; pi < G::NPX; pi++) {
+            uint32_t x, j;
+            slot_pixel<PXW, PXH>(tile_x0, tile_j0, lane, pi, x, j);
+            if (x < p.width && j < p.row_count) store(x, j, a, b);
+        }
+        return;
+    }
+    float nx = 0.0f, ny = 0.0f, nz = 0.0f, cnt = 0.0f, dmin = RT_INF, px = 0.0f, py = 0.0f, pz = 0.0f;
+#pragma unroll 1
+    for (int s0 = 0; s0 < S; s0 += 2) {
+        const int s1 = (s0 + 1 < S) ? s0 + 1 : s0;  // a pair past the end repeats the last slot
+        uint32_t x0, j0, x1, j1;
+        slot_pixel<PXW, PXH>(tile_x0, tile_j0, lane, s0 / NS, x0, j0);
+        slot_pixel<PXW, PXH>(tile_x0, tile_j0, lane, s1 / NS, x1, j1);
+        const V3x2 d = slot_dir2<SPP>(one, p, x0, image_row(p, j0), s0 % NS, x1, image_row(p, j1), s1 % NS);
+        const uint2 a = __ldcs(&winner[s0 * 32 + lane]), b = __ldcs(&winner[s1 * 32 + lane]);
+        const bool hit0 = a.x != NO_HIT, hit1 = b.x != NO_HIT;
+        F2 dist = f2(__uint_as_float(a.y), __uint_as_float(b.y));  // primitive.rs:55-72, as K2 computed it
+        const float4 w0 = __ldg(&p.sph[hit0 ? a.x : 0u]), w1 = __ldg(&p.sph[hit1 ? b.x : 0u]);
+        const V3x2 cen = V3x2{f2(w0.x, w1.x), f2(w0.y, w1.y), f2(w0.z, w1.z)};
+        if (!hit0) dist.x = 1.0f;
+        if (!hit1) dist.y = 1.0f;
+        // primitive.rs:83 normal; render.rs:199 hit point (pos + dir * distance)
+        const V3x2 nrm = vnormalized2<(NS > 1)>(one, vadd2(one, eye2, vsub2(one, vmulf2(d, dist), cen)));
+        const V3x2 hp = vadd2(one, eye2, vmulf2(d, dist));
+#pragma unroll
+        for (int k = 0; k < 2; k++) {
+            const int s = s0 + k;
+            if (k == 1 && s1 == s0) break;
+            const bool hit = k ? hit1 : hit0;
+            if (s % NS == 0) nx = ny = nz = cnt = 0.0f, dmin = RT_INF, px = py = pz = 0.0f;
+            if (hit) {
+                const float t = k ? dist.y : dist.x;
+                nx = fadd(nx, k ? nrm.x.y : nrm.x.x), ny = fadd(ny, k ? nrm.y.y : nrm.y.x), nz = fadd(nz, k ? nrm.z.y : nrm.z.x);
+                cnt = fadd(cnt, 1.0f);
+                if (t < dmin) dmin = t, px = k ? hp.x.y : hp.x.x, py = k ? hp.y.y : hp.y.x, pz = k ? hp.z.y : hp.z.x;
+            }
+            if (s % NS == NS - 1) {
+                const uint32_t x = k ? x1 : x0, j = k ? j1 : j0;
+                if (x < p.width && j < p.row_count)
+                    store(x, j, make_float4(fmul(nx, recip), fmul(ny, recip), fmul(nz, recip), fmul(cnt, recip)),
+                          make_float4(dmin, px, py, pz));
+            }
+        }
+    }
+}
+
 }  // namespace rt
 
 using namespace rt;
@@ -913,6 +991,10 @@ static cudaError_t launch_phased(bool diag, RtPixels fmt, const RenderParams &p,
         phase_cull_primary<SPP, PXW, PXH, CW, CH, 1><<<cb, 32 * P_WARPS, 0, stream>>>(p);
     }
     phase_test_primary<SPP, PXW, PXH, CW, CH><<<tiles2d, 32 * CW * CH, 0, stream>>>(p);
+    if (fmt == RT_PIXELS_AOV) {  // geometry only: no shadow cull, no shading
+        phase_aov_store<SPP, PXW, PXH, CW, CH><<<tiles2d, 32 * CW * CH, 0, stream>>>(p);
+        return cudaGetLastError();
+    }
     phase_cull_shadow<SPP, PXW, PXH, CW, CH><<<cb, 32 * P_WARPS, 0, stream>>>(p);
     if (fmt == RT_PIXELS_F32)
         phase_shade_store_f32<SPP, PXW, PXH, CW, CH><<<tiles2d, 32 * CW * CH, 0, stream>>>(p);

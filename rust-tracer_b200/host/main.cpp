@@ -15,7 +15,8 @@
 // schedule through Renderer::render_region instead of one launch per frame), --format=tga|png|apng (a real TGA, a PNG
 // encoded on the GPU: the output is then named *.png and sweep frames <stem>.f.png, or all frames in ONE animated PNG
 // named *.png), --fps=F (frame rate of --format apng), --format=pfm (the pixels before quantisation as a colour PFM
-// of 32-bit floats, named *.pfm; sweep frames <stem>.f.pfm).
+// of 32-bit floats, named *.pfm; sweep frames <stem>.f.pfm), --aov (with --format pfm: the geometry behind each
+// pixel beside it, as <stem>.normal.pfm, <stem>.coverage.pfm, <stem>.distance.pfm and <stem>.position.pfm).
 #include <cerrno>
 #include <chrono>
 #include <cmath>
@@ -60,6 +61,9 @@ const char *USAGE =
     "                                           on the GPU (the output is then named *.png) [default: ppm]\n"
     "        --format apng                      All frames in one animated PNG encoded on the GPU (named *.png)\n"
     "        --format pfm                       The unquantised pixels as a colour PFM of 32-bit floats (named *.pfm)\n"
+    "        --aov                              With --format pfm: also write <stem>.normal.pfm, <stem>.coverage.pfm,\n"
+    "                                           <stem>.distance.pfm and <stem>.position.pfm (the geometry behind each\n"
+    "                                           pixel; not with the output -)\n"
     "        --fps <F>                          Frames per second of --format apng, 1..65535 [default: 24]\n"
     "        --preview <N>                      Undersampled preview: trace one pixel per NxN block (1 sample) [default: off]\n"
     "        --stats                            Print a timing summary to stderr\n"
@@ -103,7 +107,7 @@ unsigned long long parse_or_panic(const std::string &s, unsigned long long max, 
 
 struct Args {
     std::string width, height, ssp, numcores, output, level, gpus, frames, format, preview, fps;
-    bool has_output = false, stats = false, buckets = false;
+    bool has_output = false, stats = false, buckets = false, aov = false;
 };
 
 Args parse_args(int argc, char **argv) {
@@ -137,6 +141,10 @@ Args parse_args(int argc, char **argv) {
         }
         if (!only_positional && arg == "--buckets") {
             a.buckets = true;
+            continue;
+        }
+        if (!only_positional && arg == "--aov") {
+            a.aov = true;
             continue;
         }
         if (!only_positional && arg.size() > 2 && arg[0] == '-' && arg[1] == '-') {
@@ -231,6 +239,9 @@ int main(int argc, char **argv) {
     const std::string ext = png || apng ? "png" : pfm ? "pfm" : "tga";
     // before the output's name is checked: a misused --fps is a usage error whatever the name
     if (!args.fps.empty() && !apng) usage_error("The argument '--fps' can only be used with '--format apng'");
+    if (args.aov && !pfm) usage_error("The argument '--aov' can only be used with '--format pfm'");
+    // the AOV images are files named after the output's stem
+    if (args.aov && output_file == "-") usage_error("The argument '--aov' cannot be used with the output '-'");
     unsigned long long fps = 24;
     if (!args.fps.empty() && (!parse_unsigned(args.fps, 65535, &fps) || fps == 0))
         usage_error("Invalid value for '--fps <F>': '" + args.fps + "' is not a whole number in 1..65535");
@@ -328,8 +339,24 @@ int main(int argc, char **argv) {
                 if (pfm) {  // <stem>.f.pfm per frame, or the frames back to back on stdout
                     auto r0 = clk::now();
                     Renderer::render_pfm(options, scene, output.f, frames > 1 ? &cam : nullptr, &st);
-                    render_ms += std::chrono::duration<double, std::milli>(clk::now() - r0).count();
                     kernel_ms += st.kernel_ms;
+                    if (args.aov) {  // <stem>[.f].<name>.pfm beside the colour file
+                        struct Files {
+                            FILE *f[4] = {nullptr, nullptr, nullptr, nullptr};
+                            ~Files() {
+                                for (FILE *x : f)
+                                    if (x) fclose(x);
+                            }
+                        } files;
+                        for (int k = 0; k < 4; k++) {
+                            const std::string path = with_extension(frame_path(f), std::string(AOV_IMAGES[k].name) + ".pfm");
+                            files.f[k] = fopen(path.c_str(), "wb");
+                            if (!files.f[k]) throw Panic(std::string("called `Result::unwrap()` on an `Err` value: ") + strerror(errno));
+                        }
+                        Renderer::render_aov_pfms(options, scene, files.f, frames > 1 ? &cam : nullptr, &st);
+                        kernel_ms += st.kernel_ms;
+                    }
+                    render_ms += std::chrono::duration<double, std::milli>(clk::now() - r0).count();
                 } else if (png || apng) {
                     const Renderer::ApngFrame af{f, frames, 1, (uint16_t)fps};
                     auto r0 = clk::now();

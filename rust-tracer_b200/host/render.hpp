@@ -208,24 +208,34 @@ inline void write_tga(FILE *f, uint16_t width, uint16_t height, const uint8_t *p
     fflush(f);
 }
 
-// Extension: a colour PFM of a frame's pixels before quantisation -- "PF", the size, scale -1.0 (little-endian
-// samples), then the rows from the bottom up as 32-bit float RGB.  `px` holds `height` rows of {r, g, b, alpha}
-// floats, `stride` floats apart; alpha is dropped, as the P6 sink drops it.
-inline void write_pfm(FILE *f, uint16_t width, uint16_t height, const float *px, size_t stride) {
-    fprintf(f, "PF\n%u %u\n-1.0\n", (unsigned)width, (unsigned)height);
-    std::vector<uint8_t> line((size_t)width * 12);
+// Extension: a PFM of a frame's pixels before quantisation -- "PF" (colour) or "Pf" (greyscale), the size, scale -1.0
+// (little-endian samples), then the rows from the bottom up as 32-bit floats, `channels` (3 or 1) per pixel.  `px`
+// points at the first written float of pixel (0, 0); pixels are `pixel_floats` floats apart and rows `stride` floats
+// apart.  The defaults write {r, g, b} of a float frame {r, g, b, alpha}: alpha is dropped, as the P6 sink drops it.
+inline void write_pfm(FILE *f, uint16_t width, uint16_t height, const float *px, size_t stride, size_t pixel_floats = 4,
+                      int channels = 3) {
+    fprintf(f, "%s\n%u %u\n-1.0\n", channels == 1 ? "Pf" : "PF", (unsigned)width, (unsigned)height);
+    std::vector<uint8_t> line((size_t)width * channels * 4);
     for (uint32_t y = height; y-- > 0;) {  // bottom row first
         const float *row = px + (size_t)y * stride;
         for (uint32_t x = 0; x < width; x++)
-            for (int c = 0; c < 3; c++) {
+            for (int c = 0; c < channels; c++) {
                 uint32_t bits;
-                memcpy(&bits, &row[x * 4 + c], 4);
-                for (int b = 0; b < 4; b++) line[(x * 3 + c) * 4 + b] = (uint8_t)(bits >> (8 * b));
+                memcpy(&bits, &row[x * pixel_floats + c], 4);
+                for (int b = 0; b < 4; b++) line[(x * channels + c) * 4 + b] = (uint8_t)(bits >> (8 * b));
             }
         if (fwrite(line.data(), 1, line.size(), f) != line.size()) throw Panic("write_all failed");
     }
     fflush(f);
 }
+
+// The images `rtrace --aov` writes beside the colour PFM, as <stem>.<name>.pfm: which floats of the 8-float AOV pixel
+// {nx, ny, nz, coverage, distance, px, py, pz} (include/rtrace.h "geometry output") each one holds.
+struct AovImage {
+    const char *name;
+    int offset, channels;
+};
+constexpr AovImage AOV_IMAGES[4] = {{"normal", 0, 3}, {"coverage", 3, 1}, {"distance", 4, 1}, {"position", 5, 3}};
 
 class TGARGBABufferWriter : public RGBABufferWriter {
   public:
@@ -456,6 +466,25 @@ struct Renderer {
                                            frame, frame_bytes, stats),
                  "Renderer::render_pfm");
         write_pfm(f, o.width, o.height, frame, (size_t)o.width * 4);
+    }
+
+    // One frame's geometry (extension): rendered on the scene's GPUs into pinned host memory as AOV pixels
+    // (rt_render_frame_multi_aov), then written as the PFMs of AOV_IMAGES, image k to files[k].
+    static void render_aov_pfms(const RenderOptions &o, const Scene &scene, FILE *const files[4],
+                                const rt_camera *camera = nullptr, rt_stats *stats = nullptr) {
+        struct Frame {
+            void *p = nullptr;
+            ~Frame() { rt_host_free(p); }
+        } b;
+        const size_t frame_bytes = (size_t)o.width * o.height * 32;
+        rt_check(rt_host_alloc(frame_bytes, &b.p), "Renderer::render_aov_pfms");
+        float *frame = static_cast<float *>(b.p);
+        rt_check(rt_render_frame_multi_aov(scene.replicas(), scene.gpus(), camera, o.width, o.height, o.samples_per_pixel,
+                                           frame, frame_bytes, stats),
+                 "Renderer::render_aov_pfms");
+        for (int k = 0; k < 4; k++)
+            write_pfm(files[k], o.width, o.height, frame + AOV_IMAGES[k].offset, (size_t)o.width * 8, 8,
+                      AOV_IMAGES[k].channels);
     }
 
   private:

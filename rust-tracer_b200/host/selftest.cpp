@@ -179,7 +179,9 @@ void sink_error() {
 }
 
 // write_pfm on a synthetic 3x2 frame, no GPU: pixel (x, y) component c = ((y * 3 + x) * 4 + c) / 7 in f32, with a
-// pitch of 5 pixels so that the writer must follow the stride.  tests/test_f32.py checks the file's bytes.
+// pitch of 5 pixels so that the writer must follow the stride.  Writes the colour PFM to `path` and the greyscale one
+// of component 3 (the Pf variant, as `rtrace --aov` writes coverage and distance) to `path`.grey.pfm.
+// tests/test_f32.py and tests/test_aov.py check the files' bytes.
 void pfm(const char *path) {
     const uint16_t w = 3, h = 2;
     const size_t stride = 5 * 4;
@@ -190,6 +192,11 @@ void pfm(const char *path) {
     FILE *f = fopen(path, "wb");
     if (!f) throw Panic(std::string("cannot create ") + path);
     write_pfm(f, w, h, px.data(), stride);
+    fclose(f);
+    const std::string grey = std::string(path) + ".grey.pfm";
+    f = fopen(grey.c_str(), "wb");
+    if (!f) throw Panic("cannot create " + grey);
+    write_pfm(f, w, h, px.data() + 3, stride, 4, 1);
     fclose(f);
     printf("ok pfm\n");
 }

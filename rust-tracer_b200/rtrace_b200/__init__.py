@@ -28,6 +28,7 @@ ABI_SYMBOLS = [
     "rt_png_bound", "rt_encode_png", "rt_render_sweep_png",
     "rt_apng_bound", "rt_encode_apng_frame", "rt_render_sweep_apng",
     "rt_render_rows_f32", "rt_render_frame_multi_f32",
+    "rt_render_rows_aov", "rt_render_frame_multi_aov",
 ]
 
 
@@ -138,6 +139,10 @@ def lib():
     L.rt_render_rows_f32.argtypes = [vp, C.POINTER(Camera), u32, u32, u32, u32, u32, u32, vp, C.c_size_t, vp,
                                      C.POINTER(Stats)]
     L.rt_render_frame_multi_f32.argtypes = [C.POINTER(vp), C.c_int, C.POINTER(Camera), u32, u32, u32, vp, C.c_size_t,
+                                            C.POINTER(Stats)]
+    L.rt_render_rows_aov.argtypes = [vp, C.POINTER(Camera), u32, u32, u32, u32, u32, u32, vp, C.c_size_t, vp,
+                                     C.POINTER(Stats)]
+    L.rt_render_frame_multi_aov.argtypes = [C.POINTER(vp), C.c_int, C.POINTER(Camera), u32, u32, u32, vp, C.c_size_t,
                                             C.POINTER(Stats)]
     if os.environ.get("RTRACE_B200_LIB"):
         L = real
@@ -356,21 +361,43 @@ class Renderer:
         return (out, st) if want_stats else out
 
     @staticmethod
-    def render_f32(options, scene_or_scenes, camera=None, out_ptr=None, want_stats=False):
-        """The frame before quantisation (rt_render_frame_multi_f32): (h, w, 4) float32 {r, g, b, alpha}, equal bit
-        for bit to the reference's values.  A list of scenes renders on their GPUs; with out_ptr (device memory of
-        the first scene's GPU, h * w * 16 bytes) the frame is stored there and None is returned in its place."""
+    def _frame_floats(fn, channels, options, scene_or_scenes, camera, out_ptr, want_stats):
+        """rt_render_frame_multi_f32 / _aov: `channels` f32 per pixel."""
         w, h, spp = options.width, options.height, options.samples_per_pixel
         scenes = list(scene_or_scenes) if isinstance(scene_or_scenes, (list, tuple)) else [scene_or_scenes]
         out = None
         if out_ptr is None:
-            out = np.empty((h, w, 4), np.float32)
+            out = np.empty((h, w, channels), np.float32)
             out_ptr = out.ctypes.data
         arr = (C.c_void_p * len(scenes))(*[s.handle for s in scenes])
         st = Stats() if want_stats else None
-        _check(lib().rt_render_frame_multi_f32(arr, len(scenes), C.byref(camera) if camera is not None else None, w, h,
-                                               spp, out_ptr, w * h * 16, C.byref(st) if st is not None else None))
+        _check(fn(arr, len(scenes), C.byref(camera) if camera is not None else None, w, h, spp, out_ptr,
+                  w * h * 4 * channels, C.byref(st) if st is not None else None))
         return (out, st) if want_stats else out
+
+    @staticmethod
+    def _rows_floats(fn, channels, options, scene, row_start, row_stride, row_count, camera, out, out_ptr, pitch,
+                     stream, want_stats):
+        """rt_render_rows_f32 / _aov: `channels` f32 per pixel."""
+        w, h, spp = options.width, options.height, options.samples_per_pixel
+        if row_count is None:
+            row_count = (h - row_start + row_stride - 1) // row_stride
+        if out_ptr is None:
+            if out is None:
+                out = np.empty((row_count, w, channels), np.float32)
+            out_ptr = out.ctypes.data
+        st = Stats() if want_stats else None
+        _check(fn(scene.handle, C.byref(camera) if camera is not None else None, w, h, spp, row_start, row_stride,
+                  row_count, out_ptr, pitch, stream, C.byref(st) if st is not None else None))
+        return (out, st) if want_stats else out
+
+    @staticmethod
+    def render_f32(options, scene_or_scenes, camera=None, out_ptr=None, want_stats=False):
+        """The frame before quantisation (rt_render_frame_multi_f32): (h, w, 4) float32 {r, g, b, alpha}, equal bit
+        for bit to the reference's values.  A list of scenes renders on their GPUs; with out_ptr (device memory of
+        the first scene's GPU, h * w * 16 bytes) the frame is stored there and None is returned in its place."""
+        return Renderer._frame_floats(lib().rt_render_frame_multi_f32, 4, options, scene_or_scenes, camera, out_ptr,
+                                      want_stats)
 
     @staticmethod
     def render_rows_f32(options, scene, row_start=0, row_stride=1, row_count=None, camera=None, out=None,
@@ -378,18 +405,27 @@ class Renderer:
         """render_rows before quantisation (rt_render_rows_f32): (row_count, w, 4) float32 for host output; with
         out_ptr (host or device memory, `pitch` bytes per row, 0 = w * 16) the call is asynchronous on `stream` for
         device memory and None is returned in place of the array."""
-        w, h, spp = options.width, options.height, options.samples_per_pixel
-        if row_count is None:
-            row_count = (h - row_start + row_stride - 1) // row_stride
-        if out_ptr is None:
-            if out is None:
-                out = np.empty((row_count, w, 4), np.float32)
-            out_ptr = out.ctypes.data
-        st = Stats() if want_stats else None
-        _check(lib().rt_render_rows_f32(scene.handle, C.byref(camera) if camera is not None else None, w, h, spp,
-                                        row_start, row_stride, row_count, out_ptr, pitch, stream,
-                                        C.byref(st) if st is not None else None))
-        return (out, st) if want_stats else out
+        return Renderer._rows_floats(lib().rt_render_rows_f32, 4, options, scene, row_start, row_stride, row_count,
+                                     camera, out, out_ptr, pitch, stream, want_stats)
+
+    @staticmethod
+    def render_aov(options, scene_or_scenes, camera=None, out_ptr=None, want_stats=False):
+        """The geometry behind each pixel (rt_render_frame_multi_aov): (h, w, 8) float32
+        {nx, ny, nz, coverage, distance, px, py, pz} (include/rtrace.h "geometry output").  A list of scenes renders
+        on their GPUs; with out_ptr (device memory of the first scene's GPU, h * w * 32 bytes, 16-byte aligned) the
+        frame is stored there and None is returned in its place."""
+        return Renderer._frame_floats(lib().rt_render_frame_multi_aov, 8, options, scene_or_scenes, camera, out_ptr,
+                                      want_stats)
+
+    @staticmethod
+    def render_rows_aov(options, scene, row_start=0, row_stride=1, row_count=None, camera=None, out=None,
+                        out_ptr=None, pitch=0, stream=None, want_stats=False):
+        """render_rows with AOV output (rt_render_rows_aov): (row_count, w, 8) float32 for host output; with out_ptr
+        (host or device memory, `pitch` bytes per row, 0 = w * 32) the call is asynchronous on `stream` for device
+        memory (e.g. a torch CUDA tensor's data_ptr() on torch's current stream) and None is returned in place of
+        the array."""
+        return Renderer._rows_floats(lib().rt_render_rows_aov, 8, options, scene, row_start, row_stride, row_count,
+                                     camera, out, out_ptr, pitch, stream, want_stats)
 
     @staticmethod
     def render_preview(options, scene, step, camera=None, out_ptr=None, stream=None):

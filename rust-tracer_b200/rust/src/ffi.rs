@@ -49,6 +49,11 @@ extern "C" {
     pub fn rt_render_frame_multi_f32(scenes: *const *mut RtScene, ngpu: c_int, camera: *const RtCamera, width: u32,
                                      height: u32, spp: u32, rgba_out: *mut f32, rgba_bytes: usize,
                                      stats: *mut RtStats) -> c_int;
+    // the geometry behind each pixel: {nx, ny, nz, coverage} {distance, px, py, pz} as f32, 32 bytes per pixel
+    // (include/rtrace.h "geometry output")
+    pub fn rt_render_frame_multi_aov(scenes: *const *mut RtScene, ngpu: c_int, camera: *const RtCamera, width: u32,
+                                     height: u32, spp: u32, aov_out: *mut f32, aov_bytes: usize,
+                                     stats: *mut RtStats) -> c_int;
     pub fn rt_render_sweep(s: *const RtScene, cameras: *const RtCamera, n_frames: u32, width: u32, height: u32,
                            spp: u32, cb: RtFrameCallback, user: *mut c_void, stats: *mut RtStats) -> c_int;
     pub fn rt_render_sweep_rgb(s: *const RtScene, cameras: *const RtCamera, n_frames: u32, width: u32, height: u32,
@@ -64,6 +69,9 @@ extern "C" {
                           kinds_out: *mut u8, stream: *mut c_void, stats: *mut RtStats) -> c_int;
     pub fn rt_render_rows_f32(s: *const RtScene, camera: *const RtCamera, width: u32, height: u32, spp: u32,
                               row_start: u32, row_stride: u32, row_count: u32, rgba_out: *mut f32, pitch_bytes: usize,
+                              stream: *mut c_void, stats: *mut RtStats) -> c_int;
+    pub fn rt_render_rows_aov(s: *const RtScene, camera: *const RtCamera, width: u32, height: u32, spp: u32,
+                              row_start: u32, row_stride: u32, row_count: u32, aov_out: *mut f32, pitch_bytes: usize,
                               stream: *mut c_void, stats: *mut RtStats) -> c_int;
     pub fn rt_render_row_blocks(s: *const RtScene, camera: *const RtCamera, width: u32, height: u32, spp: u32,
                                 row_start: u32, row_stride: u32, row_block: u32, row_count: u32, rgba_out: *mut u8,
