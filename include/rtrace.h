@@ -314,6 +314,25 @@ int rt_render_sweep_apng(rt_scene *const *scenes, int ngpu, const rt_camera *cam
                          uint32_t width, uint32_t height, uint32_t spp, uint16_t delay_num, uint16_t delay_den,
                          rt_frame_callback cb, void *user, rt_stats *stats);
 
+/* ---- OpenEXR output, encoded on the GPU ----------------------------------------------------------------------
+ * One fixed layout, so there is exactly one file per image (DESIGN.md "OpenEXR output"): a single-part scanline
+ * OpenEXR 2 file, ZIP compression (16 scanlines per chunk), increasing Y (image row 0 first), every channel 32-bit
+ * FLOAT.  The channels are A B G R from the float pixel {r, g, b, alpha}, and with the AOV frame also Z (distance,
+ * +inf on a miss), coverage.Y, normal.X normal.Y normal.Z and position.X position.Y position.Z: 12 channels.  The
+ * values are the frames' floats bit for bit.  A chunk's zlib stream is fixed-Huffman literals and matches of
+ * distance 1 and 2W; a chunk whose stream would not be smaller than its raw bytes is stored raw. */
+/* Worst-case size of rt_encode_exr's output for a width x height frame (1..65535 each), with (aov != 0) or without
+ * the AOV channels: the header, the offset table and every chunk stored raw.  Pure arithmetic, no device. */
+int rt_exr_bound(uint32_t width, uint32_t height, int aov, size_t *bytes);
+/* EXR file (layout above) of a width x height float frame in the layout of rt_render_rows_f32 (`rgba`, pitch 0 =
+ * width*16) and, unless aov is NULL, the AOV frame in the layout of rt_render_rows_aov (`aov`, pitch 0 = width*32),
+ * both in device memory of the current device, 16-byte aligned with pitches a multiple of 16.  out: host or device
+ * memory.  Waits for `stream` and returns the file length in *len_out; RT_ERR_BUFFER (with *len_out = the needed
+ * size) if cap is short; RT_ERR_INVALID for a host or misaligned frame, a short pitch or a zero size.  Device scratch
+ * is kept per (device, stream). */
+int rt_encode_exr(const float *rgba, size_t rgba_pitch, const float *aov, size_t aov_pitch, uint32_t width,
+                  uint32_t height, uint8_t *out, size_t cap, size_t *len_out, void *stream);
+
 /* Count rays the way the reference's work is counted (SURVEY 8d): primary =
  * rows*width*spp^2, shadow = samples with a hit facing the light. */
 int rt_count_rays(const rt_scene *s, const rt_camera *camera,

@@ -23,6 +23,7 @@
 
 #include "rt_device.cuh"
 #include "rt_kernels.h"
+#include "rt_exr.h"
 #include "rt_png.h"
 #include "rt_scene.h"
 
@@ -481,6 +482,12 @@ int check_distinct_scenes(rt_scene *const *scenes, int ngpu) {
 
 // rt_encode_png's device buffers for one (device, stream); `mu` serialises the calls that share them.
 struct PngEncodeScratch {
+    std::mutex mu;
+    DeviceBuffer scratch, out;  // out: the file, then its length word
+};
+
+// rt_encode_exr's device buffers for one (device, stream), as PngEncodeScratch.
+struct ExrEncodeScratch {
     std::mutex mu;
     DeviceBuffer scratch, out;  // out: the file, then its length word
 };
@@ -1583,6 +1590,56 @@ int rt_encode_apng_frame(const uint8_t *rgba, uint32_t width, uint32_t height, s
     Animation anim;
     anim.n_frames = n_frames, anim.delay_num = delay_num, anim.delay_den = delay_den;
     return encode_impl(rgba, width, height, pitch_bytes, out, cap, len_out, stream, &anim, frame);
+}
+
+int rt_exr_bound(uint32_t width, uint32_t height, int aov, size_t *bytes) {
+    if (!bytes) return fail(RT_ERR_INVALID, "NULL argument");
+    if (width == 0 || height == 0 || width > 65535u || height > 65535u)
+        return fail(RT_ERR_INVALID, "width/height must be in 1..65535 (got %u x %u)", width, height);
+    *bytes = rt_exr_bound_bytes(width, height, aov != 0);
+    return RT_OK;
+}
+
+int rt_encode_exr(const float *rgba, size_t rgba_pitch, const float *aov, size_t aov_pitch, uint32_t width,
+                  uint32_t height, uint8_t *out, size_t cap, size_t *len_out, void *stream_) {
+    if (!rgba || !len_out || (!out && cap)) return fail(RT_ERR_INVALID, "NULL argument");
+    *len_out = 0;
+    size_t bound = 0;
+    const int rc = rt_exr_bound(width, height, aov != nullptr, &bound);
+    if (rc != RT_OK) return rc;
+    if (rgba_pitch == 0) rgba_pitch = (size_t)width * 16;
+    if (aov_pitch == 0) aov_pitch = (size_t)width * 32;
+    if (rgba_pitch < (size_t)width * 16 || (aov && aov_pitch < (size_t)width * 32))
+        return fail(RT_ERR_INVALID, "a pitch is smaller than a row (%zu / %zu bytes for width %u)", rgba_pitch, aov_pitch, width);
+    if (((uintptr_t)rgba & 15) || (rgba_pitch & 15) || ((uintptr_t)aov & 15) || (aov && (aov_pitch & 15)))
+        return fail(RT_ERR_INVALID, "frames must be 16-byte aligned with pitches a multiple of 16");
+    int dev = -1, cur = -1;
+    CUDA_TRY(cudaGetDevice(&cur));
+    if (!is_device_ptr(rgba, &dev) || dev != cur) return fail(RT_ERR_INVALID, "rgba must be device memory of the current device %d", cur);
+    if (aov && (!is_device_ptr(aov, &dev) || dev != cur)) return fail(RT_ERR_INVALID, "aov must be device memory of the current device %d", cur);
+    cudaStream_t stream = (cudaStream_t)stream_;
+    // scratch per (device, stream), kept for the life of the process, as rt_encode_png's
+    static std::mutex g_mu;
+    static auto *g_scratch = new std::map<std::pair<int, cudaStream_t>, ExrEncodeScratch>();
+    ExrEncodeScratch *sc;
+    {
+        std::lock_guard<std::mutex> lock(g_mu);
+        sc = &(*g_scratch)[std::make_pair(cur, stream)];
+    }
+    std::lock_guard<std::mutex> lock(sc->mu);
+    const size_t len_at = (bound + 7) / 8 * 8;
+    RT_TRY(sc->scratch.ensure(rt_exr_scratch_bytes(width, height, aov != nullptr)));
+    RT_TRY(sc->out.ensure(len_at + sizeof(unsigned long long)));
+    unsigned long long *len_word = reinterpret_cast<unsigned long long *>(sc->out.ptr + len_at), len = 0;
+    CUDA_TRY(rt_launch_exr_encode(rgba, rgba_pitch, aov, aov_pitch, width, height, sc->scratch.ptr, sc->out.ptr, len_word, stream));
+    CUDA_TRY(cudaMemcpyAsync(&len, len_word, sizeof(len), cudaMemcpyDeviceToHost, stream));
+    CUDA_TRY(cudaStreamSynchronize(stream));
+    if (len == 0 || len > bound) return fail(RT_ERR_CUDA, "EXR encoder returned %llu bytes (bound %zu)", len, bound);
+    *len_out = (size_t)len;
+    if (len > cap) return fail(RT_ERR_BUFFER, "out holds %zu bytes, the file needs %llu", cap, len);
+    CUDA_TRY(cudaMemcpyAsync(out, sc->out.ptr, (size_t)len, cudaMemcpyDefault, stream));
+    CUDA_TRY(cudaStreamSynchronize(stream));
+    return RT_OK;
 }
 
 int rt_host_register(void *p, size_t bytes) {

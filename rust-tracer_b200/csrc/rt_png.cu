@@ -19,20 +19,16 @@
 // (rt_encode_apng_frame, rt_render_sweep_apng): the same zlib stream, framed as that frame's piece of the animation
 // (DESIGN.md "Animated PNG").
 #include "rt_png.h"
+#include "rt_deflate.cuh"
 
 namespace {
 
 constexpr uint32_t BAND = 16;          // rows per IDAT chunk (the multi-GPU row-block unit)
 constexpr uint32_t WARPS = BAND;       // one warp per row of the band
-constexpr uint32_t ADLER_MOD = 65521u;
-constexpr uint32_t FULL = 0xffffffffu;
 constexpr uint32_t HEADER_BYTES = 8 + 25 + 14;  // signature, IHDR, IDAT(78 01)
 constexpr uint32_t TRAILER_BYTES = 18 + 12;     // IDAT(03 00 + Adler-32), IEND
 constexpr uint32_t ACTL_BYTES = 12 + 8, FCTL_BYTES = 12 + 26;
-
-__constant__ uint16_t c_len_base[29] = {3,  4,  5,  6,  7,  8,  9,  10, 11,  13,  15,  17,  19,  23, 27,
-                                        31, 35, 43, 51, 59, 67, 83, 99, 115, 131, 163, 195, 227, 258};
-__constant__ uint8_t c_len_extra[29] = {0, 0, 0, 0, 0, 0, 0, 0, 1, 1, 1, 1, 2, 2, 2, 2, 3, 3, 3, 3, 4, 4, 4, 4, 5, 5, 5, 5, 0};
+constexpr uint32_t DIST3 = 8u;  // distance 3: code 2 in 5 bits, bit-reversed (a match is at most 8 + 5 + 5 = 18 bits)
 
 struct Scratch {
     uint32_t *stage;  // per row: slot_words words of token bits (LSB-first)
@@ -116,39 +112,9 @@ __device__ void write_chunk(uint8_t *p, const char *type, uint32_t n, const uint
     put_be32(p + 8 + n, ~crc_bytes(0xffffffffu, p + 4, 4 + n, table));
 }
 
-// ---- fixed Huffman codes (RFC 1951 3.2.6), bit-reversed for the LSB-first stream --------------------------------
-__device__ __forceinline__ uint32_t lit_bits(uint32_t v) { return v < 144u ? 8u : 9u; }
-
-__device__ __forceinline__ uint32_t lit_code(uint32_t v) {
-    return v < 144u ? __brev(0x30u + v) >> 24 : __brev(0x190u + v - 144u) >> 23;
-}
-
-// length L (3..258) + distance 3 (code 2, 5 bits): one token of at most 8 + 5 + 5 = 18 bits
-__device__ uint32_t match_code(uint32_t L, uint32_t *bits) {
-    int k = 28;
-    while (c_len_base[k] > L) k--;
-    const uint32_t sym = 257u + (uint32_t)k;
-    uint32_t c, n;
-    if (sym < 280u) c = __brev(sym - 256u) >> 25, n = 7;
-    else c = __brev(0xC0u + sym - 280u) >> 24, n = 8;
-    c |= (L - c_len_base[k]) << n;
-    n += c_len_extra[k];
-    c |= (__brev(2u) >> 27) << n;
-    *bits = n + 5;
-    return c;
-}
-
 __device__ __forceinline__ uint32_t raw_byte(const uint8_t *row, uint32_t p) {  // raw-row byte p >= 1
     const uint32_t q = p - 1u, x = q / 3u;
     return row[4u * x + (q - 3u * x)];
-}
-
-// Bytes of a row's piece: the staged token bits, zeros (end-of-block, the stored block's header, padding), then
-// the stored block's LEN / NLEN 00 00 FF FF.
-__device__ __forceinline__ uint32_t piece_bytes(uint32_t bits) { return (bits + 10u + 7u) / 8u + 4u; }
-
-__device__ __forceinline__ uint32_t piece_byte(const uint8_t *staged, uint32_t bits, uint32_t len, uint32_t q) {
-    return q < (bits + 7u) / 8u ? staged[q] : (q + 2u >= len ? 0xffu : 0u);
 }
 
 // One CTA per band of 16 rows, one warp per row.
@@ -210,7 +176,7 @@ __global__ void __launch_bounds__(WARPS * 32) png_encode_rows(const uint8_t *__r
                 cost = 13u * q;
                 if (rr >= 3u) {
                     uint32_t nb;
-                    match_code(rr, &nb);
+                    match_code(rr, DIST3, 5, &nb);
                     cost += nb;
                 } else {
                     for (uint32_t i = t - rr; i < t; i++) cost += lit_bits(raw_byte(row, i));
@@ -241,7 +207,7 @@ __global__ void __launch_bounds__(WARPS * 32) png_encode_rows(const uint8_t *__r
                 if (j < tail) {
                     if (j % 258u == 0) code = code258, nb = 13, o = ro + 13u * (j / 258u);
                 } else if (rr >= 3u) {
-                    if (j == tail) code = match_code(rr, &nb), o = ro + 13u * q;
+                    if (j == tail) code = match_code(rr, DIST3, 5, &nb), o = ro + 13u * q;
                 } else {
                     code = lit_code(v), nb = lit_bits(v), o = ro + 13u * q + (j > tail ? lit_bits(vprev) : 0u);
                 }

@@ -16,7 +16,10 @@
 // encoded on the GPU: the output is then named *.png and sweep frames <stem>.f.png, or all frames in ONE animated PNG
 // named *.png), --fps=F (frame rate of --format apng), --format=pfm (the pixels before quantisation as a colour PFM
 // of 32-bit floats, named *.pfm; sweep frames <stem>.f.pfm), --aov (with --format pfm: the geometry behind each
-// pixel beside it, as <stem>.normal.pfm, <stem>.coverage.pfm, <stem>.distance.pfm and <stem>.position.pfm).
+// pixel beside it, as <stem>.normal.pfm, <stem>.coverage.pfm, <stem>.distance.pfm and <stem>.position.pfm),
+// --format=exr (the unquantised pixels as an OpenEXR file of 32-bit floats with alpha, ZIP-compressed and encoded on
+// the GPU, named *.exr; sweep frames <stem>.f.exr; with --aov the geometry is in the same file as the channels Z,
+// coverage.Y, normal.* and position.*, so it may go to the output -).
 #include <cerrno>
 #include <chrono>
 #include <cmath>
@@ -61,9 +64,12 @@ const char *USAGE =
     "                                           on the GPU (the output is then named *.png) [default: ppm]\n"
     "        --format apng                      All frames in one animated PNG encoded on the GPU (named *.png)\n"
     "        --format pfm                       The unquantised pixels as a colour PFM of 32-bit floats (named *.pfm)\n"
+    "        --format exr                       The unquantised pixels with alpha as an OpenEXR file of 32-bit floats,\n"
+    "                                           ZIP-compressed on the GPU (named *.exr)\n"
     "        --aov                              With --format pfm: also write <stem>.normal.pfm, <stem>.coverage.pfm,\n"
     "                                           <stem>.distance.pfm and <stem>.position.pfm (the geometry behind each\n"
-    "                                           pixel; not with the output -)\n"
+    "                                           pixel; not with the output -).  With --format exr: the same geometry\n"
+    "                                           as the channels Z, coverage.Y, normal.XYZ and position.XYZ of the file\n"
     "        --fps <F>                          Frames per second of --format apng, 1..65535 [default: 24]\n"
     "        --preview <N>                      Undersampled preview: trace one pixel per NxN block (1 sample) [default: off]\n"
     "        --stats                            Print a timing summary to stderr\n"
@@ -71,8 +77,8 @@ const char *USAGE =
     "                                           be multiples of 64, as in the reference); default is whole frames\n"
     "\n"
     "ARGS:\n"
-    "    <output>    Either a file with .tga extension (.png with --format png or apng, .pfm with --format pfm), or - to\n"
-    "                write file to stdout\n";
+    "    <output>    Either a file with .tga extension (.png with --format png or apng, .pfm with --format pfm, .exr with\n"
+    "                --format exr), or - to write file to stdout\n";
 
 [[noreturn]] void usage_error(const std::string &msg) {
     // clap 2: message + usage hint on stderr, exit status 1
@@ -235,13 +241,13 @@ int main(int argc, char **argv) {
     const std::string &output_file = args.output;
     FileOrAnyWriter output;
     FILE *fp = nullptr;
-    const bool png = args.format == "png", apng = args.format == "apng", pfm = args.format == "pfm";
-    const std::string ext = png || apng ? "png" : pfm ? "pfm" : "tga";
+    const bool png = args.format == "png", apng = args.format == "apng", pfm = args.format == "pfm", exr = args.format == "exr";
+    const std::string ext = png || apng ? "png" : pfm ? "pfm" : exr ? "exr" : "tga";
     // before the output's name is checked: a misused --fps is a usage error whatever the name
     if (!args.fps.empty() && !apng) usage_error("The argument '--fps' can only be used with '--format apng'");
-    if (args.aov && !pfm) usage_error("The argument '--aov' can only be used with '--format pfm'");
-    // the AOV images are files named after the output's stem
-    if (args.aov && output_file == "-") usage_error("The argument '--aov' cannot be used with the output '-'");
+    if (args.aov && !pfm && !exr) usage_error("The argument '--aov' can only be used with '--format pfm' or '--format exr'");
+    // the AOV images of a PFM are files named after the output's stem (an EXR holds them itself)
+    if (args.aov && pfm && output_file == "-") usage_error("The argument '--aov' cannot be used with the output '-'");
     unsigned long long fps = 24;
     if (!args.fps.empty() && (!parse_unsigned(args.fps, 65535, &fps) || fps == 0))
         usage_error("Invalid value for '--fps <F>': '" + args.fps + "' is not a whole number in 1..65535");
@@ -263,12 +269,12 @@ int main(int argc, char **argv) {
     unsigned frames = (unsigned)parse_or_panic(args.frames.empty() ? "1" : args.frames, 100000, "frames");
     if (gpus < 1) gpus = 1;
     if (frames < 1) frames = 1;
-    if (!args.format.empty() && args.format != "ppm" && args.format != "tga" && !png && !apng && !pfm)
-        usage_error("'" + args.format + "' isn't a valid value for '--format <ppm|tga|png|apng|pfm>'");
+    if (!args.format.empty() && args.format != "ppm" && args.format != "tga" && !png && !apng && !pfm && !exr)
+        usage_error("'" + args.format + "' isn't a valid value for '--format <ppm|tga|png|apng|pfm|exr>'");
     // the bucket schedule exists to drive the host writer seam; a PNG is encoded on the GPU from a whole frame,
-    // and a PFM is the float frame of the whole-frame path
-    if ((png || apng || pfm) && args.buckets) usage_error("The argument '--buckets' cannot be used with '--format " + args.format + "'");
-    if (pfm && !args.preview.empty()) usage_error("The argument '--preview' cannot be used with '--format pfm'");
+    // and a PFM or an EXR is the float frame of the whole-frame path
+    if ((png || apng || pfm || exr) && args.buckets) usage_error("The argument '--buckets' cannot be used with '--format " + args.format + "'");
+    if ((pfm || exr) && !args.preview.empty()) usage_error("The argument '--preview' cannot be used with '--format " + args.format + "'");
     const bool real_tga = args.format == "tga";
     const unsigned preview = args.preview.empty() ? 0u : (unsigned)parse_or_panic(args.preview, 1024, "preview");
     if (options.width == 0 || options.height == 0) {
@@ -294,7 +300,7 @@ int main(int argc, char **argv) {
             if (!fp) throw Panic(std::string("called `Result::unwrap()` on an `Err` value: ") + strerror(errno));
             return FileOrAnyWriter::file_writer(fp);
         };
-        if (frames > 1 && !preview && !args.buckets && !pfm) {
+        if (frames > 1 && !preview && !args.buckets && !pfm && !exr) {
             // orbit sweep: the GPUs draw frames from one queue, copy-out of a frame overlapping the render of the next ones;
             // the frames come back in order (rt_render_sweep_multi)
             std::vector<rt_camera> cams;
@@ -357,6 +363,11 @@ int main(int argc, char **argv) {
                         kernel_ms += st.kernel_ms;
                     }
                     render_ms += std::chrono::duration<double, std::milli>(clk::now() - r0).count();
+                } else if (exr) {  // <stem>.f.exr per frame, or the files back to back on stdout
+                    auto r0 = clk::now();
+                    Renderer::render_exr(options, scene, output.f, frames > 1 ? &cam : nullptr, args.aov, &st);
+                    render_ms += std::chrono::duration<double, std::milli>(clk::now() - r0).count();
+                    kernel_ms += st.kernel_ms;
                 } else if (png || apng) {
                     const Renderer::ApngFrame af{f, frames, 1, (uint16_t)fps};
                     auto r0 = clk::now();

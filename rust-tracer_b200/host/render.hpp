@@ -487,6 +487,42 @@ struct Renderer {
                       AOV_IMAGES[k].channels);
     }
 
+    // One frame before quantisation as an OpenEXR file on `f` (extension): the float frame and, with `aov`, the AOV
+    // frame rendered on the scene's GPUs into device memory of the first GPU (rt_render_frame_multi_f32 / _aov) and
+    // encoded there (rt_encode_exr), so only the file crosses the host link.  stats->kernel_ms is both renders'.
+    static void render_exr(const RenderOptions &o, const Scene &scene, FILE *f, const rt_camera *camera = nullptr,
+                           bool aov = false, rt_stats *stats = nullptr) {
+        struct Buffers {
+            void *rgba = nullptr, *aov = nullptr, *file = nullptr;
+            ~Buffers() {
+                rt_device_free(rgba);
+                rt_device_free(aov);
+                rt_host_free(file);
+            }
+        } b;
+        const size_t px = (size_t)o.width * o.height;
+        size_t bound = 0, len = 0;
+        rt_check(rt_exr_bound(o.width, o.height, aov ? 1 : 0, &bound), "Renderer::render_exr");
+        rt_check(rt_device_alloc(px * 16, &b.rgba), "Renderer::render_exr");
+        rt_check(rt_host_alloc(bound, &b.file), "Renderer::render_exr");
+        rt_check(rt_render_frame_multi_f32(scene.replicas(), scene.gpus(), camera, o.width, o.height, o.samples_per_pixel,
+                                           static_cast<float *>(b.rgba), px * 16, stats),
+                 "Renderer::render_exr");
+        if (aov) {
+            rt_stats st;
+            rt_check(rt_device_alloc(px * 32, &b.aov), "Renderer::render_exr");
+            rt_check(rt_render_frame_multi_aov(scene.replicas(), scene.gpus(), camera, o.width, o.height,
+                                               o.samples_per_pixel, static_cast<float *>(b.aov), px * 32, &st),
+                     "Renderer::render_exr");
+            if (stats) stats->kernel_ms += st.kernel_ms;
+        }
+        rt_check(rt_encode_exr(static_cast<const float *>(b.rgba), 0, static_cast<const float *>(b.aov), 0, o.width,
+                               o.height, static_cast<uint8_t *>(b.file), bound, &len, nullptr),
+                 "Renderer::render_exr");
+        if (fwrite(b.file, 1, len, f) != len) throw Panic("write_all failed");
+        fflush(f);
+    }
+
   private:
     // `call(cb, user)` runs a sweep that hands each frame to `sink`.  An exception thrown by the sink does not cross
     // the C boundary: it is caught in the trampoline, the remaining frames are skipped, and it is rethrown here once

@@ -29,6 +29,7 @@ ABI_SYMBOLS = [
     "rt_apng_bound", "rt_encode_apng_frame", "rt_render_sweep_apng",
     "rt_render_rows_f32", "rt_render_frame_multi_f32",
     "rt_render_rows_aov", "rt_render_frame_multi_aov",
+    "rt_exr_bound", "rt_encode_exr",
 ]
 
 
@@ -136,6 +137,8 @@ def lib():
                                        C.POINTER(C.c_size_t), vp]
     L.rt_render_sweep_apng.argtypes = [C.POINTER(vp), C.c_int, C.POINTER(Camera), u32, u32, u32, u32, u16, u16,
                                        FRAME_CALLBACK, vp, C.POINTER(Stats)]
+    L.rt_exr_bound.argtypes = [u32, u32, C.c_int, C.POINTER(C.c_size_t)]
+    L.rt_encode_exr.argtypes = [vp, C.c_size_t, vp, C.c_size_t, u32, u32, vp, C.c_size_t, C.POINTER(C.c_size_t), vp]
     L.rt_render_rows_f32.argtypes = [vp, C.POINTER(Camera), u32, u32, u32, u32, u32, u32, vp, C.c_size_t, vp,
                                      C.POINTER(Stats)]
     L.rt_render_frame_multi_f32.argtypes = [C.POINTER(vp), C.c_int, C.POINTER(Camera), u32, u32, u32, vp, C.c_size_t,
@@ -667,6 +670,25 @@ def encode_apng_frame(device_ptr, width, height, frame, n_frames, fps=24, pitch=
     n = C.c_size_t()
     _check(lib().rt_encode_apng_frame(C.c_void_p(device_ptr), width, height, pitch, frame, n_frames, 1, fps, out, cap,
                                       C.byref(n), stream))
+    return out.raw[:n.value]
+
+
+def exr_bound(width, height, aov=False):
+    """Worst-case size of encode_exr's file (pure arithmetic, no device needed)."""
+    n = C.c_size_t()
+    _check(lib().rt_exr_bound(width, height, 1 if aov else 0, C.byref(n)))
+    return n.value
+
+
+def encode_exr(rgba_ptr, width, height, aov_ptr=None, pitch=0, aov_pitch=0, stream=None):
+    """OpenEXR file (bytes) of a width x height float frame (the layout of render_rows_f32) and, with `aov_ptr`, the
+    AOV frame (the layout of render_rows_aov) beside it, both in device memory of the current device, encoded on the
+    GPU (rt_encode_exr); waits for `stream`."""
+    cap = exr_bound(width, height, aov_ptr is not None)
+    out = C.create_string_buffer(cap)
+    n = C.c_size_t()
+    _check(lib().rt_encode_exr(C.c_void_p(rgba_ptr), pitch, None if aov_ptr is None else C.c_void_p(aov_ptr), aov_pitch,
+                               width, height, out, cap, C.byref(n), stream))
     return out.raw[:n.value]
 
 
