@@ -13,7 +13,7 @@ import zlib
 
 import numpy as np
 
-from _png_ref import FC, LB, LE, rev
+from _png_ref import FC, LB, LE, Bits, rev
 
 LINES = 16
 PIECE = 16384
@@ -104,8 +104,9 @@ def _cover(starts, ends, n):
     return np.cumsum(acc[:n]) > 0
 
 
-def zlib_stream(d, d2):
-    """The chunk's zlib stream by the parse rule (d2 = 0: no far distance)."""
+def zlib_stream(d, d2, pieces=False):
+    """The chunk's zlib stream by the parse rule (d2 = 0: no far distance); with `pieces`, also the offset of each
+    piece in it."""
     n = len(d)
     far = np.zeros(n, bool)
     if d2:
@@ -159,7 +160,57 @@ def zlib_stream(d, d2):
     out[piece_off + piece_len - 1] = 0xFF
     out[0], out[1] = 0x78, 0x01
     out[-6:] = np.frombuffer(b"\x03\x00" + struct.pack(">I", zlib.adler32(d.tobytes())), np.uint8)
-    return out.tobytes()
+    return (out.tobytes(), piece_off) if pieces else out.tobytes()
+
+
+def slow_stream(d, d2):
+    """The zlib stream of one chunk by the parse rule, byte by byte (for small inputs)."""
+    d = [int(v) for v in d]
+    n = len(d)
+    out = bytearray(b"\x78\x01")
+    for p0 in range(0, n, PIECE):
+        p1 = min(n, p0 + PIECE)
+        far = [bool(d2) and i >= d2 and d[i] == d[i - d2] for i in range(p0, p1)]
+        in_far = [False] * (p1 - p0)
+        i = 0
+        while i < len(far):
+            j = i
+            while j < len(far) and far[j]:
+                j += 1
+            if j - i >= 3:
+                in_far[i:j] = [True] * (j - i)
+            i = max(j, i + 1)
+        near = [(p0 + k) >= 1 and d[p0 + k] == d[p0 + k - 1] and not in_far[k] for k in range(p1 - p0)]
+        bw = Bits()
+        bw.put(0b010, 3)
+        k = 0
+        while k < p1 - p0:
+            mask = in_far if in_far[k] else near if near[k] else None
+            if mask is None:
+                bw.put(*FC[d[p0 + k]])
+                k += 1
+                continue
+            dc = dist_code(d2 if mask is in_far else 1)
+            j = k
+            while j < p1 - p0 and mask[j]:
+                j += 1
+            R = j - k
+            for _ in range(R // 258):
+                bw.put(int(_LEN_CODE[258]), int(_LEN_BITS[258]))
+                bw.put(*dc)
+            rr = R % 258
+            if rr >= 3:
+                bw.put(int(_LEN_CODE[rr]), int(_LEN_BITS[rr]))
+                bw.put(*dc)
+            else:
+                for q in range(j - rr, j):
+                    bw.put(*FC[d[p0 + q]])
+            k = j
+        bw.put(*FC[256])
+        bw.put(0, 3)
+        bw.align()
+        out += bw.out + b"\x00\x00\xff\xff"
+    return bytes(out) + b"\x03\x00" + struct.pack(">I", zlib.adler32(bytes(d)))
 
 
 def chunk_raw(planes, y0, y1):

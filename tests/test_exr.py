@@ -9,7 +9,6 @@ import os
 
 os.environ["OPENCV_IO_ENABLE_OPENEXR"] = "1"   # before OpenCV is imported anywhere
 
-import struct
 import subprocess
 import sys
 import zlib
@@ -20,7 +19,6 @@ import pytest
 import _exr_ref as X
 import _oracle_aov
 import _oracle_f32
-from _png_ref import FC, Bits
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
@@ -71,56 +69,6 @@ def check_file(data, rgba, aov, tmp_path=None):
             assert bits_equal(img.reshape(h, w, 4), rgba[..., [2, 1, 0, 3]])
 
 
-def slow_stream(d, d2):
-    """The zlib stream of one chunk by the parse rule, byte by byte (for small inputs)."""
-    d = [int(v) for v in d]
-    n = len(d)
-    out = bytearray(b"\x78\x01")
-    for p0 in range(0, n, X.PIECE):
-        p1 = min(n, p0 + X.PIECE)
-        far = [bool(d2) and i >= d2 and d[i] == d[i - d2] for i in range(p0, p1)]
-        in_far = [False] * (p1 - p0)
-        i = 0
-        while i < len(far):
-            j = i
-            while j < len(far) and far[j]:
-                j += 1
-            if j - i >= 3:
-                in_far[i:j] = [True] * (j - i)
-            i = max(j, i + 1)
-        near = [(p0 + k) >= 1 and d[p0 + k] == d[p0 + k - 1] and not in_far[k] for k in range(p1 - p0)]
-        bw = Bits()
-        bw.put(0b010, 3)
-        k = 0
-        while k < p1 - p0:
-            mask = in_far if in_far[k] else near if near[k] else None
-            if mask is None:
-                bw.put(*FC[d[p0 + k]])
-                k += 1
-                continue
-            dc = X.dist_code(d2 if mask is in_far else 1)
-            j = k
-            while j < p1 - p0 and mask[j]:
-                j += 1
-            R = j - k
-            for _ in range(R // 258):
-                bw.put(int(X._LEN_CODE[258]), int(X._LEN_BITS[258]))
-                bw.put(*dc)
-            rr = R % 258
-            if rr >= 3:
-                bw.put(int(X._LEN_CODE[rr]), int(X._LEN_BITS[rr]))
-                bw.put(*dc)
-            else:
-                for q in range(j - rr, j):
-                    bw.put(*FC[d[p0 + q]])
-            k = j
-        bw.put(*FC[256])
-        bw.put(0, 3)
-        bw.align()
-        out += bw.out + b"\x00\x00\xff\xff"
-    return bytes(out) + b"\x03\x00" + struct.pack(">I", zlib.adler32(bytes(d)))
-
-
 # ---- CPU ----------------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("w,h,spp", [(1, 1, 1), (37, 21, 2), (64, 48, 3), (100, 17, 4), (24, 16, 5), (20, 31, 6),
                                      (17, 9, 7), (16, 8, 8), (12, 40, 9), (160, 90, 2)])
@@ -164,7 +112,7 @@ def test_parse_rule_matches_the_byte_by_byte_statement():
     cases += [(runs, 6), (runs, 0), (np.full(20000, 7, np.uint8), 2), (rng.integers(0, 256, 300).astype(np.uint8), 8)]
     for d, d2 in cases:
         z = X.zlib_stream(d, d2)
-        assert z == slow_stream(d, d2)
+        assert z == X.slow_stream(d, d2)
         assert zlib.decompress(z) == d.tobytes()
 
 

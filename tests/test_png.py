@@ -242,6 +242,50 @@ def test_encode_pitched_input_and_synthetic_frames(rt, gpu_scene8):
             rt.device_free(ptr)
 
 
+def lane_rows():
+    """32 rows, row L with one run of 258 repeated bytes (87 pixels of one colour) starting at raw-row byte p with
+    p = L mod 32: the lane of the 32-byte step where the run starts.  The other pixels repeat no byte 3 back."""
+    rows = []
+    for lane in range(32):
+        x0 = (lane - 4) * 11 % 32                      # the run starts at byte 1 + 3 * (x0 + 1); 3 * 11 = 1 mod 32
+        px = [[(7 * k + c) % 97 for c in range(3)] for k in range(120)]
+        px[x0:x0 + 87] = [[200, 201, 202]] * 87
+        rows.append(px)
+    return np.array(rows, np.uint8)
+
+
+DEVICE_CASES = dict(REFERENCE_CASES, run258_lanes=lane_rows())
+
+
+def test_lane_rows_start_a_258_run_at_every_lane():
+    starts = set()
+    for row in lane_rows():
+        a = np.frombuffer(b"\x00" + row.tobytes(), np.uint8)
+        eq = np.flatnonzero(a[4:] == a[1:-3]) + 4
+        assert len(eq) == 258 and eq[-1] - eq[0] == 257
+        starts.add(int(eq[0]) % 32)
+    assert starts == set(range(32))
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("name", sorted(DEVICE_CASES))
+def test_encode_reference_cases_on_the_device(rt, name):
+    """The crafted cases (runs of every remainder mod 258, band heights 15/16/17, runs starting at every lane)
+    encoded on the device from RGBA with random alpha, which must be dropped."""
+    rgb = DEVICE_CASES[name]
+    h, w, _ = rgb.shape
+    alpha = np.random.default_rng(len(name) * 131 + h).integers(0, 256, (h, w, 1)).astype(np.uint8)
+    rgba = np.ascontiguousarray(np.concatenate([rgb, alpha], axis=2))
+    ptr = rt.device_alloc(rgba.nbytes)
+    try:
+        rt.memcpy(ptr, rgba.ctypes.data, rgba.nbytes)
+        png = rt.encode_png(ptr, w, h)
+    finally:
+        rt.device_free(ptr)
+    assert png == P.encode(rgb)
+    check_file(png, rgb)
+
+
 @pytest.mark.gpu
 def test_encode_errors(rt, gpu_scene8):
     L = rt.lib()
