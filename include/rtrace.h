@@ -314,6 +314,27 @@ int rt_render_sweep_apng(rt_scene *const *scenes, int ngpu, const rt_camera *cam
                          uint32_t width, uint32_t height, uint32_t spp, uint16_t delay_num, uint16_t delay_den,
                          rt_frame_callback cb, void *user, rt_stats *stats);
 
+/* ---- JPEG output, encoded on the GPU --------------------------------------------------------------------------
+ * One fixed layout, so there is exactly one file per image and quality (DESIGN.md "JPEG output"): baseline
+ * sequential JPEG (JFIF), 4:2:0, the standard Huffman tables of ITU T.81 Annex K, the quality's scaled Annex K
+ * quantisation tables, and one restart interval per MCU row of 16 image rows.  Alpha is dropped, as the P6 sink does.
+ * The bytes are those libjpeg-turbo writes for the same pixels, quality and settings, without optimised tables. */
+/* Worst-case size of rt_encode_jpeg's output for a width x height frame (1..65535 each) at any quality.  Pure
+ * arithmetic, no device. */
+int rt_jpeg_bound(uint32_t width, uint32_t height, size_t *bytes);
+/* JPEG file (layout above) at `quality` (1..100) of a width x height RGBA8 frame in device memory of the current
+ * device (pitch 0 = width*4).  out: host or device memory.  Waits for `stream` and returns the file length in
+ * *len_out; RT_ERR_BUFFER (with *len_out = the needed size) if cap is short; RT_ERR_INVALID for a host rgba pointer,
+ * a zero size or a quality outside 1..100.  Device scratch is kept per (device, stream). */
+int rt_encode_jpeg(const uint8_t *rgba, uint32_t width, uint32_t height, size_t pitch_bytes, int quality,
+                   uint8_t *out, size_t cap, size_t *len_out, void *stream);
+/* rt_render_sweep_png delivering each frame as a complete JPEG file at `quality` (len = file size), in frame order,
+ * on the calling thread; ngpu == 1 is the single-GPU pipelined sweep.  Each frame is encoded on the GPU that rendered
+ * it, behind its render launches, and only the file's bytes cross the host link. */
+int rt_render_sweep_jpeg(rt_scene *const *scenes, int ngpu, const rt_camera *cameras, uint32_t n_frames,
+                         uint32_t width, uint32_t height, uint32_t spp, int quality,
+                         rt_frame_callback cb, void *user, rt_stats *stats);
+
 /* ---- OpenEXR output, encoded on the GPU ----------------------------------------------------------------------
  * One fixed layout, so there is exactly one file per image (DESIGN.md "OpenEXR output"): a single-part scanline
  * OpenEXR 2 file, ZIP compression (16 scanlines per chunk), increasing Y (image row 0 first), every channel 32-bit

@@ -24,6 +24,7 @@
 #include "rt_device.cuh"
 #include "rt_kernels.h"
 #include "rt_exr.h"
+#include "rt_jpeg.h"
 #include "rt_png.h"
 #include "rt_scene.h"
 
@@ -40,9 +41,9 @@ struct RowLayout {
     bool out_abs = false;
 };
 
-// What a sweep hands to its frame callback: the RGBA8 frame, its RGB8 bytes (the P6 body), or a PNG file (with an
-// Animation: the frame's payload of an animated PNG).
-enum class OutKind { RGBA, RGB, PNG };
+// What a sweep hands to its frame callback: the RGBA8 frame, its RGB8 bytes (the P6 body), a PNG file (with an
+// Animation: the frame's payload of an animated PNG), or a JPEG file.
+enum class OutKind { RGBA, RGB, PNG, JPEG };
 
 int fail(int code, const char *fmt, ...) {
     va_list ap;
@@ -128,9 +129,9 @@ struct Stream : NonCopyable {
 };
 
 // Scratch of the launches on one stream (launches on different streams may overlap): the PHASED variant's buffers
-// and the PNG encoder's.
+// and the PNG and JPEG encoders'.
 struct StreamScratch {
-    DeviceBuffer winner, hdr, pool, pool_count, png;
+    DeviceBuffer winner, hdr, pool, pool_count, png, jpeg;
     uint32_t pool_units = 0;  // pool entries the kernels may use: a forced RTRACE_POOL_UNITS may leave it below pool.cap
 };
 
@@ -138,9 +139,9 @@ struct StreamScratch {
 struct SweepSlot {
     DeviceBuffer frame;  // RGBA8
     DeviceBuffer rgb;    // its RGB8 pack (RGB sweeps)
-    DeviceBuffer png;    // its PNG file, then the file's length word (PNG sweeps)
+    DeviceBuffer png;    // its PNG or JPEG file, then the file's length word (PNG and JPEG sweeps)
     HostBuffer host;     // what the frame callback receives
-    HostBuffer len;      // the PNG length word read back
+    HostBuffer len;      // the length word read back
     Event rendered, copied, len_ready;
 };
 
@@ -459,6 +460,18 @@ int queue_encode(const uint8_t *rgba, size_t pitch, uint32_t width, uint32_t hei
     return RT_OK;
 }
 
+// queue_encode for a JPEG file at `quality`; `bound` is rt_jpeg_bound_bytes.
+int queue_encode_jpeg(const uint8_t *rgba, size_t pitch, uint32_t width, uint32_t height, int quality, size_t bound,
+                      DeviceBuffer &scratch, DeviceBuffer &out, unsigned long long *len_host, cudaStream_t stream) {
+    const size_t len_at = (bound + 7) / 8 * 8;
+    RT_TRY(scratch.ensure(rt_jpeg_scratch_bytes(width, height)));
+    RT_TRY(out.ensure(len_at + sizeof(unsigned long long)));
+    unsigned long long *len_word = reinterpret_cast<unsigned long long *>(out.ptr + len_at);
+    CUDA_TRY(rt_launch_jpeg_encode(rgba, pitch, width, height, quality, scratch.ptr, out.ptr, len_word, stream));
+    CUDA_TRY(cudaMemcpyAsync(len_host, len_word, sizeof(unsigned long long), cudaMemcpyDeviceToHost, stream));
+    return RT_OK;
+}
+
 // Peer access from device `from` (the current device) to the memory of device `to`: *can = false when there is none.
 int enable_peer(int from, int to, bool *can) {
     int c = 0;
@@ -488,6 +501,12 @@ struct PngEncodeScratch {
 
 // rt_encode_exr's device buffers for one (device, stream), as PngEncodeScratch.
 struct ExrEncodeScratch {
+    std::mutex mu;
+    DeviceBuffer scratch, out;  // out: the file, then its length word
+};
+
+// rt_encode_jpeg's device buffers for one (device, stream), as PngEncodeScratch.
+struct JpegEncodeScratch {
     std::mutex mu;
     DeviceBuffer scratch, out;  // out: the file, then its length word
 };
@@ -866,10 +885,11 @@ struct CallbackSource : FrameSource {
 };
 
 static int sweep_locked(rt_scene *s, FrameSource &src, uint32_t width, uint32_t height, uint32_t spp, rt_frame_callback cb,
-                        void *user, rt_stats *stats, OutKind kind, const Animation *anim);
+                        void *user, rt_stats *stats, OutKind kind, const Animation *anim, int quality);
 
 static int sweep_impl(const rt_scene *cs, FrameSource &src, uint32_t width, uint32_t height, uint32_t spp,
-                      rt_frame_callback cb, void *user, rt_stats *stats, OutKind kind, const Animation *anim = nullptr) {
+                      rt_frame_callback cb, void *user, rt_stats *stats, OutKind kind, const Animation *anim = nullptr,
+                      int quality = 0) {
     rt_scene *s = const_cast<rt_scene *>(cs);
     int rc = check_frame_args(s, width, height, spp, 0, 1, height);
     if (rc != RT_OK) return rc;
@@ -877,7 +897,7 @@ static int sweep_impl(const rt_scene *cs, FrameSource &src, uint32_t width, uint
     DeviceGuard guard(s->device);
     if (!guard.ok) return fail(RT_ERR_CUDA, "cannot select device %d", s->device);
     std::lock_guard<std::mutex> lock(s->mu);
-    rc = sweep_locked(s, src, width, height, spp, cb, user, stats, kind, anim);
+    rc = sweep_locked(s, src, width, height, spp, cb, user, stats, kind, anim, quality);
     if (rc != RT_OK) {  // leave no render or copy in flight on the ring buffers (keeps the first error text)
         if (s->own_stream) cudaStreamSynchronize(s->own_stream);
         if (s->render2) cudaStreamSynchronize(s->render2);
@@ -887,14 +907,15 @@ static int sweep_impl(const rt_scene *cs, FrameSource &src, uint32_t width, uint
     return rc;
 }
 
-// anim != nullptr (PNG only): every frame is its payload of that animated PNG
+// anim != nullptr (PNG only): every frame is its payload of that animated PNG; quality: of the JPEG files
 static int sweep_locked(rt_scene *s, FrameSource &src, uint32_t width, uint32_t height, uint32_t spp, rt_frame_callback cb,
-                        void *user, rt_stats *stats, OutKind kind, const Animation *anim) {
+                        void *user, rt_stats *stats, OutKind kind, const Animation *anim, int quality) {
     const double t0 = now_ms();
-    const bool rgb = kind == OutKind::RGB, png = kind == OutKind::PNG;
+    const bool rgb = kind == OutKind::RGB, jpeg = kind == OutKind::JPEG, png = kind == OutKind::PNG || jpeg;
     const size_t row_bytes = (size_t)width * 4, frame_bytes = row_bytes * height;
     const size_t out_bytes = rgb ? (size_t)width * height * 3 : frame_bytes;
-    const size_t png_bytes = png ? rt_png_bound_bytes(width, height, anim) : 0;
+    // png_bytes: the bound of the encoded file, PNG or JPEG
+    const size_t png_bytes = jpeg ? rt_jpeg_bound_bytes(width, height) : png ? rt_png_bound_bytes(width, height, anim) : 0;
     const size_t host_bytes = std::max(frame_bytes, png_bytes);
     // `depth` frames render at a time, each on its own stream (depth 2: the launch tails of frame f are filled
     // by the first launches of frame f+1), while an earlier frame is copied out: depth + 1 device frames and
@@ -947,11 +968,15 @@ static int sweep_locked(rt_scene *s, FrameSource &src, uint32_t width, uint32_t 
                     // stream, so that the copy stream never waits for a later frame); the file is copied at hand-over
                     {
                         std::lock_guard<std::mutex> lock(s->mu_scratch);
-                        RT_TRY(queue_encode(sl.frame.ptr, row_bytes, width, height, anim, (uint32_t)id, png_bytes,
-                                            s->scratch[rs].png, sl.png, sl.len.as<unsigned long long>(), rs));
+                        if (jpeg)
+                            RT_TRY(queue_encode_jpeg(sl.frame.ptr, row_bytes, width, height, quality, png_bytes,
+                                                     s->scratch[rs].jpeg, sl.png, sl.len.as<unsigned long long>(), rs));
+                        else
+                            RT_TRY(queue_encode(sl.frame.ptr, row_bytes, width, height, anim, (uint32_t)id, png_bytes,
+                                                s->scratch[rs].png, sl.png, sl.len.as<unsigned long long>(), rs));
                     }
                     CUDA_TRY(cudaEventRecord(sl.len_ready, rs));
-                    launches += 2;
+                    launches += jpeg ? 3 : 2;
                 } else {
                     CUDA_TRY(cudaEventRecord(sl.rendered, rs));
                     CUDA_TRY(cudaStreamWaitEvent(s->copy_stream, sl.rendered, 0));
@@ -969,7 +994,8 @@ static int sweep_locked(rt_scene *s, FrameSource &src, uint32_t width, uint32_t 
             if (png) {  // the file's length first, then just that many bytes
                 CUDA_TRY(cudaEventSynchronize(sl.len_ready));
                 len = (size_t)*sl.len.as<unsigned long long>();
-                if (len > png_bytes) return fail(RT_ERR_CUDA, "PNG encoder returned %zu bytes, more than the bound %zu", len, png_bytes);
+                if (len > png_bytes)
+                    return fail(RT_ERR_CUDA, "%s encoder returned %zu bytes, more than the bound %zu", jpeg ? "JPEG" : "PNG", len, png_bytes);
                 CUDA_TRY(cudaMemcpyAsync(sl.host.ptr, sl.png.ptr, len, cudaMemcpyDeviceToHost, s->copy_stream));
                 CUDA_TRY(cudaEventRecord(sl.copied, s->copy_stream));
             }
@@ -1225,7 +1251,7 @@ void board_offer(void *user, uint32_t frame, const uint8_t *data, size_t len) {
 
 static int sweep_multi_impl(rt_scene *const *scenes, int ngpu, const rt_camera *cameras, uint32_t n_frames, uint32_t width,
                             uint32_t height, uint32_t spp, OutKind kind, rt_frame_callback cb, void *user, rt_stats *stats,
-                            const Animation *anim = nullptr) {
+                            const Animation *anim = nullptr, int quality = 0) {
     if (!scenes || ngpu < 1) return fail(RT_ERR_INVALID, "need at least one scene");
     for (int g = 0; g < ngpu; g++) {
         int rc = check_frame_args(scenes[g], width, height, spp, 0, 1, height);
@@ -1235,7 +1261,7 @@ static int sweep_multi_impl(rt_scene *const *scenes, int ngpu, const rt_camera *
     if (n_frames == 0) return RT_OK;
     if (ngpu == 1) {
         ListSource src(cameras, n_frames);
-        return sweep_impl(scenes[0], src, width, height, spp, cb, user, stats, kind, anim);
+        return sweep_impl(scenes[0], src, width, height, spp, cb, user, stats, kind, anim, quality);
     }
     RT_TRY(check_distinct_scenes(scenes, ngpu));  // each worker locks its own
     const double t0 = now_ms();
@@ -1251,7 +1277,8 @@ static int sweep_multi_impl(rt_scene *const *scenes, int ngpu, const rt_camera *
         workers.emplace_back([&, g, variant]() {
             g_variant = variant;
             BoardSource src(board);
-            const int rc = sweep_impl(scenes[g], src, width, height, spp, board_offer, &board, &wstats[(size_t)g], kind, anim);
+            const int rc = sweep_impl(scenes[g], src, width, height, spp, board_offer, &board, &wstats[(size_t)g], kind, anim,
+                                      quality);
             std::lock_guard<std::mutex> lock(board.mu);
             if (rc != RT_OK && board.rc == RT_OK) {
                 board.rc = rc;
@@ -1321,6 +1348,16 @@ int rt_render_sweep_apng(rt_scene *const *scenes, int ngpu, const rt_camera *cam
     Animation anim;
     anim.n_frames = n_frames, anim.delay_num = delay_num, anim.delay_den = delay_den;
     return sweep_multi_impl(scenes, ngpu, cameras, n_frames, width, height, spp, OutKind::PNG, cb, user, stats, &anim);
+}
+
+int rt_render_sweep_jpeg(rt_scene *const *scenes, int ngpu, const rt_camera *cameras, uint32_t n_frames, uint32_t width,
+                         uint32_t height, uint32_t spp, int quality, rt_frame_callback cb, void *user, rt_stats *stats) {
+    size_t bound = 0;
+    const int rc = rt_jpeg_bound(width, height, &bound);
+    if (rc != RT_OK) return rc;
+    if (quality < 1 || quality > 100) return fail(RT_ERR_INVALID, "quality must be in 1..100 (got %d)", quality);
+    return sweep_multi_impl(scenes, ngpu, cameras, n_frames, width, height, spp, OutKind::JPEG, cb, user, stats, nullptr,
+                            quality);
 }
 
 uint64_t rt_atomic_fetch_add_u64(void *addr, uint64_t value) {
@@ -1635,6 +1672,50 @@ int rt_encode_exr(const float *rgba, size_t rgba_pitch, const float *aov, size_t
     CUDA_TRY(cudaMemcpyAsync(&len, len_word, sizeof(len), cudaMemcpyDeviceToHost, stream));
     CUDA_TRY(cudaStreamSynchronize(stream));
     if (len == 0 || len > bound) return fail(RT_ERR_CUDA, "EXR encoder returned %llu bytes (bound %zu)", len, bound);
+    *len_out = (size_t)len;
+    if (len > cap) return fail(RT_ERR_BUFFER, "out holds %zu bytes, the file needs %llu", cap, len);
+    CUDA_TRY(cudaMemcpyAsync(out, sc->out.ptr, (size_t)len, cudaMemcpyDefault, stream));
+    CUDA_TRY(cudaStreamSynchronize(stream));
+    return RT_OK;
+}
+
+int rt_jpeg_bound(uint32_t width, uint32_t height, size_t *bytes) {
+    if (!bytes) return fail(RT_ERR_INVALID, "NULL argument");
+    if (width == 0 || height == 0 || width > 65535u || height > 65535u)
+        return fail(RT_ERR_INVALID, "width/height must be in 1..65535 (got %u x %u)", width, height);
+    *bytes = rt_jpeg_bound_bytes(width, height);
+    return RT_OK;
+}
+
+int rt_encode_jpeg(const uint8_t *rgba, uint32_t width, uint32_t height, size_t pitch_bytes, int quality, uint8_t *out,
+                   size_t cap, size_t *len_out, void *stream_) {
+    if (!rgba || !len_out || (!out && cap)) return fail(RT_ERR_INVALID, "NULL argument");
+    *len_out = 0;
+    size_t bound = 0;
+    const int rc = rt_jpeg_bound(width, height, &bound);
+    if (rc != RT_OK) return rc;
+    if (quality < 1 || quality > 100) return fail(RT_ERR_INVALID, "quality must be in 1..100 (got %d)", quality);
+    const size_t row_bytes = (size_t)width * 4;
+    if (pitch_bytes == 0) pitch_bytes = row_bytes;
+    if (pitch_bytes < row_bytes) return fail(RT_ERR_INVALID, "pitch %zu is smaller than a row (%zu bytes)", pitch_bytes, row_bytes);
+    int dev = -1, cur = -1;
+    if (!is_device_ptr(rgba, &dev)) return fail(RT_ERR_INVALID, "rgba must be device memory");
+    CUDA_TRY(cudaGetDevice(&cur));
+    if (dev != cur) return fail(RT_ERR_INVALID, "rgba lives on device %d, the current device is %d", dev, cur);
+    cudaStream_t stream = (cudaStream_t)stream_;
+    // scratch per (device, stream), kept for the life of the process, as rt_encode_png's
+    static std::mutex g_mu;
+    static auto *g_scratch = new std::map<std::pair<int, cudaStream_t>, JpegEncodeScratch>();
+    JpegEncodeScratch *sc;
+    {
+        std::lock_guard<std::mutex> lock(g_mu);
+        sc = &(*g_scratch)[std::make_pair(cur, stream)];
+    }
+    std::lock_guard<std::mutex> lock(sc->mu);
+    unsigned long long len = 0;
+    RT_TRY(queue_encode_jpeg(rgba, pitch_bytes, width, height, quality, bound, sc->scratch, sc->out, &len, stream));
+    CUDA_TRY(cudaStreamSynchronize(stream));
+    if (len == 0 || len > bound) return fail(RT_ERR_CUDA, "JPEG encoder returned %llu bytes (bound %zu)", len, bound);
     *len_out = (size_t)len;
     if (len > cap) return fail(RT_ERR_BUFFER, "out holds %zu bytes, the file needs %llu", cap, len);
     CUDA_TRY(cudaMemcpyAsync(out, sc->out.ptr, (size_t)len, cudaMemcpyDefault, stream));

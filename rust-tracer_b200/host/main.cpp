@@ -19,7 +19,8 @@
 // pixel beside it, as <stem>.normal.pfm, <stem>.coverage.pfm, <stem>.distance.pfm and <stem>.position.pfm),
 // --format=exr (the unquantised pixels as an OpenEXR file of 32-bit floats with alpha, ZIP-compressed and encoded on
 // the GPU, named *.exr; sweep frames <stem>.f.exr; with --aov the geometry is in the same file as the channels Z,
-// coverage.Y, normal.* and position.*, so it may go to the output -).
+// coverage.Y, normal.* and position.*, so it may go to the output -), --format=jpg (a JPEG encoded on the GPU, named
+// *.jpg; sweep frames <stem>.f.jpg), --quality=Q (of --format jpg, 1..100, default 90).
 #include <cerrno>
 #include <chrono>
 #include <cmath>
@@ -70,6 +71,8 @@ const char *USAGE =
     "                                           <stem>.distance.pfm and <stem>.position.pfm (the geometry behind each\n"
     "                                           pixel; not with the output -).  With --format exr: the same geometry\n"
     "                                           as the channels Z, coverage.Y, normal.XYZ and position.XYZ of the file\n"
+    "        --format jpg                       A JPEG (baseline, 4:2:0) encoded on the GPU (named *.jpg)\n"
+    "        --quality <Q>                      JPEG quality of --format jpg, 1..100 [default: 90]\n"
     "        --fps <F>                          Frames per second of --format apng, 1..65535 [default: 24]\n"
     "        --preview <N>                      Undersampled preview: trace one pixel per NxN block (1 sample) [default: off]\n"
     "        --stats                            Print a timing summary to stderr\n"
@@ -78,7 +81,8 @@ const char *USAGE =
     "\n"
     "ARGS:\n"
     "    <output>    Either a file with .tga extension (.png with --format png or apng, .pfm with --format pfm, .exr with\n"
-    "                --format exr), or - to write file to stdout\n";
+    "                --format exr), or - to write file to stdout\n"
+    "                (.jpg with --format jpg, which also writes to stdout)\n";
 
 [[noreturn]] void usage_error(const std::string &msg) {
     // clap 2: message + usage hint on stderr, exit status 1
@@ -112,7 +116,7 @@ unsigned long long parse_or_panic(const std::string &s, unsigned long long max, 
 }
 
 struct Args {
-    std::string width, height, ssp, numcores, output, level, gpus, frames, format, preview, fps;
+    std::string width, height, ssp, numcores, output, level, gpus, frames, format, preview, fps, quality;
     bool has_output = false, stats = false, buckets = false, aov = false;
 };
 
@@ -125,7 +129,7 @@ Args parse_args(int argc, char **argv) {
     const Opt opts[] = {{"--width", &Args::width},   {"--height", &Args::height}, {"--samples-per-pixel", &Args::ssp},
                         {"--num-cores", &Args::numcores}, {"--level", &Args::level},   {"--gpus", &Args::gpus},
                         {"--frames", &Args::frames}, {"--format", &Args::format},
-                        {"--preview", &Args::preview}, {"--fps", &Args::fps}};
+                        {"--preview", &Args::preview}, {"--fps", &Args::fps}, {"--quality", &Args::quality}};
     bool only_positional = false;
     for (int i = 1; i < argc; i++) {
         std::string arg = argv[i];
@@ -242,15 +246,20 @@ int main(int argc, char **argv) {
     FileOrAnyWriter output;
     FILE *fp = nullptr;
     const bool png = args.format == "png", apng = args.format == "apng", pfm = args.format == "pfm", exr = args.format == "exr";
-    const std::string ext = png || apng ? "png" : pfm ? "pfm" : exr ? "exr" : "tga";
+    const bool jpg = args.format == "jpg";
+    const std::string ext = png || apng ? "png" : pfm ? "pfm" : exr ? "exr" : jpg ? "jpg" : "tga";
     // before the output's name is checked: a misused --fps is a usage error whatever the name
     if (!args.fps.empty() && !apng) usage_error("The argument '--fps' can only be used with '--format apng'");
+    if (!args.quality.empty() && !jpg) usage_error("The argument '--quality' can only be used with '--format jpg'");
     if (args.aov && !pfm && !exr) usage_error("The argument '--aov' can only be used with '--format pfm' or '--format exr'");
     // the AOV images of a PFM are files named after the output's stem (an EXR holds them itself)
     if (args.aov && pfm && output_file == "-") usage_error("The argument '--aov' cannot be used with the output '-'");
     unsigned long long fps = 24;
     if (!args.fps.empty() && (!parse_unsigned(args.fps, 65535, &fps) || fps == 0))
         usage_error("Invalid value for '--fps <F>': '" + args.fps + "' is not a whole number in 1..65535");
+    unsigned long long quality = 90;
+    if (!args.quality.empty() && (!parse_unsigned(args.quality, 100, &quality) || quality == 0))
+        usage_error("Invalid value for '--quality <Q>': '" + args.quality + "' is not a whole number in 1..100");
     if (output_file != "-") {
         if (extension_of(output_file) != ext) {
             printf("Output file '%s' must have the %s extension, e.g. %s\n", output_file.c_str(), ext.c_str(), with_extension(output_file, ext).c_str());
@@ -269,11 +278,11 @@ int main(int argc, char **argv) {
     unsigned frames = (unsigned)parse_or_panic(args.frames.empty() ? "1" : args.frames, 100000, "frames");
     if (gpus < 1) gpus = 1;
     if (frames < 1) frames = 1;
-    if (!args.format.empty() && args.format != "ppm" && args.format != "tga" && !png && !apng && !pfm && !exr)
-        usage_error("'" + args.format + "' isn't a valid value for '--format <ppm|tga|png|apng|pfm|exr>'");
-    // the bucket schedule exists to drive the host writer seam; a PNG is encoded on the GPU from a whole frame,
-    // and a PFM or an EXR is the float frame of the whole-frame path
-    if ((png || apng || pfm || exr) && args.buckets) usage_error("The argument '--buckets' cannot be used with '--format " + args.format + "'");
+    if (!args.format.empty() && args.format != "ppm" && args.format != "tga" && !png && !apng && !pfm && !exr && !jpg)
+        usage_error("'" + args.format + "' isn't a valid value for '--format <ppm|tga|png|apng|pfm|exr|jpg>'");
+    // the bucket schedule exists to drive the host writer seam; a PNG or a JPEG is encoded on the GPU from a whole
+    // frame, and a PFM or an EXR is the float frame of the whole-frame path
+    if ((png || apng || pfm || exr || jpg) && args.buckets) usage_error("The argument '--buckets' cannot be used with '--format " + args.format + "'");
     if ((pfm || exr) && !args.preview.empty()) usage_error("The argument '--preview' cannot be used with '--format " + args.format + "'");
     const bool real_tga = args.format == "tga";
     const unsigned preview = args.preview.empty() ? 0u : (unsigned)parse_or_panic(args.preview, 1024, "preview");
@@ -316,6 +325,13 @@ int main(int argc, char **argv) {
                 if (fp) fclose(fp), fp = nullptr;
             } else if (png) {  // frames arrive as complete PNG files
                 Renderer::render_sweep_png(options, scene, cams, [&](uint32_t f, const uint8_t *file, size_t len) {
+                    output = open_output(f);
+                    if (fwrite(file, 1, len, output.f) != len) throw Panic("write_all failed");
+                    fflush(output.f);
+                    if (fp) fclose(fp), fp = nullptr;
+                }, &st);
+            } else if (jpg) {  // frames arrive as complete JPEG files
+                Renderer::render_sweep_jpeg(options, scene, cams, (int)quality, [&](uint32_t f, const uint8_t *file, size_t len) {
                     output = open_output(f);
                     if (fwrite(file, 1, len, output.f) != len) throw Panic("write_all failed");
                     fflush(output.f);
@@ -372,6 +388,11 @@ int main(int argc, char **argv) {
                     const Renderer::ApngFrame af{f, frames, 1, (uint16_t)fps};
                     auto r0 = clk::now();
                     Renderer::render_png(options, scene, output.f, frames > 1 ? &cam : nullptr, preview, &st, apng ? &af : nullptr);
+                    render_ms += std::chrono::duration<double, std::milli>(clk::now() - r0).count();
+                    kernel_ms += preview ? 0.0 : st.kernel_ms;
+                } else if (jpg) {
+                    auto r0 = clk::now();
+                    Renderer::render_jpeg(options, scene, output.f, (int)quality, frames > 1 ? &cam : nullptr, preview, &st);
                     render_ms += std::chrono::duration<double, std::milli>(clk::now() - r0).count();
                     kernel_ms += preview ? 0.0 : st.kernel_ms;
                 } else {

@@ -410,6 +410,17 @@ struct Renderer {
         });
     }
 
+    // The same sweep delivering every frame as a JPEG file at `quality` encoded on its GPU (extension):
+    // `sink(f, file, len)`.
+    template <class Sink>
+    static void render_sweep_jpeg(const RenderOptions &o, const Scene &scene, const std::vector<rt_camera> &cameras,
+                                  int quality, Sink &&sink, rt_stats *stats = nullptr) {
+        sweep_through(sink, "Renderer::render_sweep_jpeg", [&](rt_frame_callback cb, void *user) {
+            return rt_render_sweep_jpeg(scene.replicas(), scene.gpus(), cameras.data(), (uint32_t)cameras.size(), o.width,
+                                        o.height, o.samples_per_pixel, quality, cb, user, stats);
+        });
+    }
+
     // Which frame of an animated PNG render_png writes, and the animation's frame count and frame delay.
     struct ApngFrame {
         uint32_t frame, n_frames;
@@ -448,6 +459,33 @@ struct Renderer {
                       : rt_encode_png(frame, o.width, o.height, 0, file, bound, &len, nullptr),
                  "Renderer::render_png");
         if (fwrite(b.file, 1, len, f) != len) throw Panic("write_all failed");
+        fflush(f);
+    }
+
+    // One frame (or an undersampled preview when preview_step > 0) as a JPEG file at `quality` on `f` (extension),
+    // rendered and encoded as render_png does.  The file lands in ordinary host memory: the bound covers the worst
+    // case of every block, about 13 times the frame's RGBA bytes, and only the file's length is ever written.
+    static void render_jpeg(const RenderOptions &o, const Scene &scene, FILE *f, int quality, const rt_camera *camera = nullptr,
+                            uint32_t preview_step = 0, rt_stats *stats = nullptr) {
+        struct Frame {
+            void *p = nullptr;
+            ~Frame() { rt_device_free(p); }
+        } b;
+        const size_t frame_bytes = (size_t)o.width * o.height * 4;
+        size_t bound = 0, len = 0;
+        rt_check(rt_jpeg_bound(o.width, o.height, &bound), "Renderer::render_jpeg");
+        rt_check(rt_device_alloc(frame_bytes, &b.p), "Renderer::render_jpeg");
+        uint8_t *frame = static_cast<uint8_t *>(b.p);
+        if (preview_step)
+            rt_check(rt_render_preview(scene.replicas()[0], camera, o.width, o.height, preview_step, frame, frame_bytes, nullptr),
+                     "Renderer::render_preview");
+        else
+            rt_check(rt_render_frame_multi(scene.replicas(), scene.gpus(), camera, o.width, o.height, o.samples_per_pixel,
+                                           frame, frame_bytes, stats),
+                     "Renderer::render");
+        std::unique_ptr<uint8_t[]> file(new uint8_t[bound]);
+        rt_check(rt_encode_jpeg(frame, o.width, o.height, 0, quality, file.get(), bound, &len, nullptr), "Renderer::render_jpeg");
+        if (fwrite(file.get(), 1, len, f) != len) throw Panic("write_all failed");
         fflush(f);
     }
 

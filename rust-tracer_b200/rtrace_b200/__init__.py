@@ -27,6 +27,7 @@ ABI_SYMBOLS = [
     "rt_count_rays", "rt_trace_rays", "rt_measure_fp32_peak", "rt_microbench_fp32", "rt_selftest_math", "rt_debug_phased_tiles", "rt_host_alloc", "rt_host_free", "rt_host_register", "rt_host_unregister", "rt_microbench_d2h", "rt_device_alloc", "rt_device_free", "rt_ipc_export", "rt_ipc_open", "rt_ipc_close", "rt_memcpy", "rt_memcpy2d_async", "rt_pack_rgb_rows",
     "rt_png_bound", "rt_encode_png", "rt_render_sweep_png",
     "rt_apng_bound", "rt_encode_apng_frame", "rt_render_sweep_apng",
+    "rt_jpeg_bound", "rt_encode_jpeg", "rt_render_sweep_jpeg",
     "rt_render_rows_f32", "rt_render_frame_multi_f32",
     "rt_render_rows_aov", "rt_render_frame_multi_aov",
     "rt_exr_bound", "rt_encode_exr",
@@ -136,6 +137,10 @@ def lib():
     L.rt_encode_apng_frame.argtypes = [vp, u32, u32, C.c_size_t, u32, u32, u16, u16, vp, C.c_size_t,
                                        C.POINTER(C.c_size_t), vp]
     L.rt_render_sweep_apng.argtypes = [C.POINTER(vp), C.c_int, C.POINTER(Camera), u32, u32, u32, u32, u16, u16,
+                                       FRAME_CALLBACK, vp, C.POINTER(Stats)]
+    L.rt_jpeg_bound.argtypes = [u32, u32, C.POINTER(C.c_size_t)]
+    L.rt_encode_jpeg.argtypes = [vp, u32, u32, C.c_size_t, C.c_int, vp, C.c_size_t, C.POINTER(C.c_size_t), vp]
+    L.rt_render_sweep_jpeg.argtypes = [C.POINTER(vp), C.c_int, C.POINTER(Camera), u32, u32, u32, u32, C.c_int,
                                        FRAME_CALLBACK, vp, C.POINTER(Stats)]
     L.rt_exr_bound.argtypes = [u32, u32, C.c_int, C.POINTER(C.c_size_t)]
     L.rt_encode_exr.argtypes = [vp, C.c_size_t, vp, C.c_size_t, u32, u32, vp, C.c_size_t, C.POINTER(C.c_size_t), vp]
@@ -540,6 +545,23 @@ class Renderer:
         return st
 
     @staticmethod
+    def render_sweep_jpeg(options, scenes, n_frames, cameras=None, quality=90, on_frame=None):
+        """The frame-sharded sweep (render_sweep_multi) delivering every frame as a JPEG file at `quality` encoded on
+        its GPU: on_frame(f, bytes) in frame order on the calling thread; one scene is the single-GPU sweep."""
+        w, h, spp = options.width, options.height, options.samples_per_pixel
+        cams = (Camera * n_frames)(*cameras) if cameras is not None else None
+
+        def _cb(user, frame, ptr, nbytes):
+            if on_frame is not None:
+                on_frame(int(frame), C.string_at(ptr, nbytes))
+
+        cb = FRAME_CALLBACK(_cb)
+        st = Stats()
+        arr = (C.c_void_p * len(scenes))(*[s.handle for s in scenes])
+        _check(lib().rt_render_sweep_jpeg(arr, len(scenes), cams, n_frames, w, h, spp, quality, cb, None, C.byref(st)))
+        return st
+
+    @staticmethod
     def render_multi(options, scenes, camera=None, want_stats=False):
         """Whole frame on len(scenes) GPUs of this process, rows interleaved, gathered on GPU 0."""
         w, h, spp = options.width, options.height, options.samples_per_pixel
@@ -671,6 +693,24 @@ def encode_apng_frame(device_ptr, width, height, frame, n_frames, fps=24, pitch=
     _check(lib().rt_encode_apng_frame(C.c_void_p(device_ptr), width, height, pitch, frame, n_frames, 1, fps, out, cap,
                                       C.byref(n), stream))
     return out.raw[:n.value]
+
+
+def jpeg_bound(width, height):
+    """Worst-case size of encode_jpeg's file for a width x height frame at any quality (pure arithmetic, no device
+    needed)."""
+    n = C.c_size_t()
+    _check(lib().rt_jpeg_bound(width, height, C.byref(n)))
+    return n.value
+
+
+def encode_jpeg(device_ptr, width, height, quality=90, pitch=0, stream=None):
+    """JPEG file (bytes) at `quality` (1..100) of a width x height RGBA8 frame in device memory of the current device
+    (alpha dropped), encoded on the GPU (rt_encode_jpeg); waits for `stream`."""
+    cap = jpeg_bound(width, height)
+    out = C.create_string_buffer(cap)
+    n = C.c_size_t()
+    _check(lib().rt_encode_jpeg(C.c_void_p(device_ptr), width, height, pitch, quality, out, cap, C.byref(n), stream))
+    return C.string_at(out, n.value)
 
 
 def exr_bound(width, height, aov=False):

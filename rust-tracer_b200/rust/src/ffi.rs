@@ -92,6 +92,12 @@ extern "C" {
     pub fn rt_render_sweep_apng(scenes: *const *mut RtScene, ngpu: c_int, cameras: *const RtCamera, n_frames: u32,
                                 width: u32, height: u32, spp: u32, delay_num: u16, delay_den: u16,
                                 cb: RtFrameCallback, user: *mut c_void, stats: *mut RtStats) -> c_int;
+    pub fn rt_jpeg_bound(width: u32, height: u32, bytes: *mut usize) -> c_int;
+    pub fn rt_encode_jpeg(rgba: *const u8, width: u32, height: u32, pitch_bytes: usize, quality: c_int, out: *mut u8,
+                          cap: usize, len_out: *mut usize, stream: *mut c_void) -> c_int;
+    pub fn rt_render_sweep_jpeg(scenes: *const *mut RtScene, ngpu: c_int, cameras: *const RtCamera, n_frames: u32,
+                                width: u32, height: u32, spp: u32, quality: c_int, cb: RtFrameCallback,
+                                user: *mut c_void, stats: *mut RtStats) -> c_int;
     pub fn rt_exr_bound(width: u32, height: u32, aov: c_int, bytes: *mut usize) -> c_int;
     pub fn rt_encode_exr(rgba: *const f32, rgba_pitch: usize, aov: *const f32, aov_pitch: usize, width: u32,
                          height: u32, out: *mut u8, cap: usize, len_out: *mut usize, stream: *mut c_void) -> c_int;
